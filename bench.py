@@ -15,6 +15,12 @@ select configs[1] / configs[0] / configs[4] (8-bit W/A + 16-bit G) and its 8-bit
 two microbenchmark halves of the metric (configs[2]): ``quantize`` (lbt_quantize over 2^28 elements, GB/s and fraction of the
 measured HBM peak) and ``gemm`` (lbt_gemm_i8 at 8192^3, TOPS, fraction of the int8 nominal and of torch._int_mm timed in the
 same run).  Rank 0 prints ONE JSON line.
+
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+also writes what the last step of the first timed region computed as DIR/<name>.npy (see dump_outputs): the loss, and the
+weights, momentum slots, gradients and ranges the step left behind.  Inputs, initial weights and noise are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -71,10 +77,17 @@ def emit(line):
         os.write(_REAL_STDOUT, data)
 
 
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError('must be at least 1, got %d' % v)
+    return v
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=20)
+    ap.add_argument('--steps', type=positive_int, default=20, help='timed steps of each timed region')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='native', choices=['native', 'reference'])
     ap.add_argument('--workload', default='resnet18', choices=sorted(WORKLOADS))
@@ -87,7 +100,29 @@ def parse():
     ap.add_argument('--no-overlap', action='store_true', help='A/B: weight-gradient kernels on the main stream (no side branch)')
     ap.add_argument('--breakdown', action='store_true', help='also print the per-kernel time table to stderr')
     ap.add_argument('--dump-launches', default='', help='write the per-launch device times of one step (CSV) to this file')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='write the outputs of the last timed step as DIR/<name>.npy (native path, rank 0)')
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != 'native':
+        ap.error('--dump-outputs writes the outputs of the native path')
+    return a
+
+
+DUMP_CAP = 1 << 22      # elements per dumped array: 16 MiB each, so the three model-sized arrays + the small ones stay under 64 MiB
+
+
+def dump_outputs(path, arrays):
+    """Write every array of ``arrays`` (name -> numpy array) flattened as ``path/<name>.npy``: float32 stays float32,
+    everything else (integer ranges, counters) becomes float64, which holds it exactly.  An array of more than DUMP_CAP
+    elements is written as a fixed sample: the elements at DUMP_CAP sorted indices drawn by numpy's default_rng(0), the
+    same indices for the same size, so two runs of the same workload compare element for element."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        v = np.ascontiguousarray(v).reshape(-1)
+        if v.size > DUMP_CAP:
+            v = v[np.sort(np.random.default_rng(0).choice(v.size, DUMP_CAP, replace=False))]
+        np.save(os.path.join(path, name + '.npy'), v.astype(np.float32 if v.dtype == np.float32 else np.float64))
 
 
 def describe(a, batch):
@@ -419,6 +454,12 @@ def run_native(a):
     ms_step = ms_total / a.steps
     value = batch * world / (ms_step * 1e-3)
     final_loss = float(loss)
+    outputs = None
+    if a.dump_outputs and rank == 0:     # copied now: the steps of the second timed region train on from here
+        rt = model.runtime
+        outputs = {'loss': loss.detach().float().reshape(1).cpu().numpy(), 'weights': trainer.flat_w.cpu().numpy(),
+                   'momentum': trainer.flat_a.cpu().numpy(), 'gradients': trainer.flat_g.cpu().numpy(),
+                   'ranges': rt.flat['ranges'].cpu().numpy(), 'step_counter': rt.dev_step.reshape(1).cpu().numpy()}
 
     # ---- timed region 2: end to end through the public API with HOST buffers ----------------------
     # every step: H2D copy of ITS inputs from pinned host memory (prefetched on a copy stream while the previous step runs,
@@ -618,6 +659,8 @@ def run_native(a):
     if a.breakdown:
         for k, d in breakdown.items():
             print('[breakdown] %-28s %s' % (k, d), file=sys.stderr)
+    if outputs is not None:
+        dump_outputs(a.dump_outputs, outputs)
     emit(line)
     _finish(world)
 

@@ -4,7 +4,7 @@ LDGSTS; legacy tensor paths (HMMA/IMMA = mma.sync) listed so their absence is vi
 
     python benchmarks/sass_summary.py [lbt_b200/liblbt_b200.so] > profiles/r2_sass_summary.txt
 
-__graft_entry__.build() regenerates profiles/r2_sass_summary.txt after every build.
+__graft_entry__.build() compares profiles/r2_sass_summary.txt with every build and says when it needs regenerating.
 """
 import collections
 import os
