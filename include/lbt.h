@@ -440,6 +440,29 @@ int lbt_bn_fwd_apply_pooled(const int8_t* k1, size_t n_outer, int H, int W, int 
                             int POH, int POW, float* pooled, uint8_t* pidx, const lbt_qsite* q_next, void* next_mant,
                             int next_kind, void* stream);
 /*
+ * fwd 2 in eval mode (dfxp:616 with the running statistics): lbt_bn_fwd_apply / lbt_bn_fwd_apply2 with mean = run_mean[c] and
+ * var = run_var[c] in place of the batch moments of `sums` — y1 = (xq - run_mean) / (run_var + eps) ** 0.5, then the same
+ * Rescale_q quantiser, affine, add, ReLU and consumer quantisers, bit-identical to the training kernel's arithmetic.  Nothing
+ * is written but the outputs: no batch moments, no running-average update.  k2 may be NULL (nothing is saved for a backward
+ * pass).  q_next2 may be NULL (one consumer quantiser) or set together with q_next.  NULL k1 / run_mean / run_var / gamma_q /
+ * beta_q, or C % 4 != 0: LBT_EINVAL before any CUDA call.
+ */
+int lbt_bn_fwd_apply_running(const int8_t* k1, size_t n_outer, size_t n_inner, int C, int bits1, const int32_t* ib1,
+                             const float* run_mean, const float* run_var, float eps, int bits2, const int32_t* ib2,
+                             const float* noise2, uint64_t seed, uint64_t offset2, const uint64_t* dev_step,
+                             uint64_t* counters2, const float* gamma_q, const float* beta_q, const float* add, int relu,
+                             int8_t* k2, float* out, int stats_minmax, const lbt_qsite* q_next, void* next_mant,
+                             int next_kind, const lbt_qsite* q_next2, void* next_mant2, int next_kind2, void* stream);
+/* lbt_bn_fwd_apply_pooled in eval mode: the running statistics as in lbt_bn_fwd_apply_running, the max-pool as in
+ * lbt_bn_fwd_apply_pooled (same shape limits, else LBT_EUNSUPPORTED); k2 may be NULL. */
+int lbt_bn_fwd_apply_running_pooled(const int8_t* k1, size_t n_outer, int H, int W, int C, int bits1, const int32_t* ib1,
+                                    const float* run_mean, const float* run_var, float eps, int bits2, const int32_t* ib2,
+                                    const float* noise2, uint64_t seed, uint64_t offset2, const uint64_t* dev_step,
+                                    uint64_t* counters2, const float* gamma_q, const float* beta_q, int relu, int8_t* k2,
+                                    int stats_minmax, int k, int s, int pad_top, int pad_left, int POH, int POW,
+                                    float* pooled, uint8_t* pidx, const lbt_qsite* q_next, void* next_mant, int next_kind,
+                                    void* stream);
+/*
  * bwd 1: g (w.r.t. the module output) -> ReLU mask (relu: 0 none, 1 recomputed from k2, 2 from `out`)
  * [-> d_add = masked g] -> kg2 = Q(g) (dfxp:687) -> sums[0..C) = sum kg2 (dbeta, :690),
  * sums[C..2C) = sum kg2*k2 (dgamma, :689) -> dx2 = gq2 * gamma_q (:691) -> kg1 = Q(dx2) (dfxp:621)

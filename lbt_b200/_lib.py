@@ -80,6 +80,17 @@ SIGNATURES = {
                                         c_void_p, c_void_p, c_u64, c_u64, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
                                         c_void_p, c_void_p, c_void_p, ctypes.c_double, c_int, c_int, c_int, c_int, c_int,
                                         c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
+    # k1, n_outer, n_inner, C, bits1, ib1, run_mean, run_var, eps, bits2, ib2, noise2, seed, offset2, dev_step, counters2, gamma_q,
+    # beta_q, add, relu, k2, out, stats_minmax, q_next, next_mant, next_kind, q_next2, next_mant2, next_kind2, stream
+    'lbt_bn_fwd_apply_running': (c_int, [c_void_p, c_size_t, c_size_t, c_int, c_int, c_void_p, c_void_p, c_void_p, c_float, c_int,
+                                         c_void_p, c_void_p, c_u64, c_u64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+                                         c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_int, c_void_p]),
+    # k1, n_outer, H, W, C, bits1, ib1, run_mean, run_var, eps, bits2, ib2, noise2, seed, offset2, dev_step, counters2, gamma_q,
+    # beta_q, relu, k2, stats_minmax, k, s, pad_top, pad_left, POH, POW, pooled, pidx, q_next, next_mant, next_kind, stream
+    'lbt_bn_fwd_apply_running_pooled': (c_int, [c_void_p, c_size_t, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
+                                                c_float, c_int, c_void_p, c_void_p, c_u64, c_u64, c_void_p, c_void_p, c_void_p,
+                                                c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                                c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     'lbt_bn_bwd_quant_stats': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_size_t, c_int, c_int,
                                        c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_u64, c_void_p, c_int,
                                        c_void_p, c_void_p, c_u64, c_void_p, c_u64, c_void_p, c_void_p, c_void_p,

@@ -333,18 +333,18 @@ struct Fwd2Params {
   const int8_t* k1;
   int bits1;
   const int32_t* ib1;
-  const long long* sums;  // [2*C] from fwd 1
+  const long long* sums;  // [2*C] from fwd 1 (RUN: unused)
   float eps;
   QSite q2;               // Rescale_q's X quantiser
   const float* gq;        // quantised gamma [C]
   const float* bq;        // quantised beta  [C]
   const float* add;       // optional shortcut tensor, same shape
   int relu;
-  int8_t* k2;
+  int8_t* k2;             // RUN: optional
   float* out;
   float* batch_mean;      // [C] optional
   float* batch_var;       // [C] optional
-  float* run_mean;        // [C] optional, updated in place with `momentum` (dfxp:602-612)
+  float* run_mean;        // [C] optional, updated in place with `momentum` (dfxp:602-612); RUN: the (read-only) mean / var
   float* run_var;
   float momentum, one_minus_momentum;   // the reference's Python constants `momentum` and `(1-momentum)`, each rounded to fp32
   QSite q3;               // optional: the consuming layer's input quantiser (bits == 0: off)
@@ -358,7 +358,9 @@ struct Fwd2Params {
 // per-channel constants where that commutes with the roundings exactly (x * 2^f scalings commute with RN):
 //   y1 * m2 = RN((xq - mean) / den) * m2 = RN((xq - mean) / (den / m2));   RN(xq2 * g) = RN(k2 * (g / m2)).
 // Q4: the second-consumer instantiation (its own registers: only the HBM-bound add + out launches in front of a strided block use it)
-template <bool MM, bool Q4 = false>
+// RUN: eval mode (dfxp:616 with the running statistics): mean / var are read from run_mean / run_var instead of being formed
+// from the batch sums; no batch moments, no running-average update, k2 optional.  Only the per-channel prologue differs.
+template <bool MM, bool Q4 = false, bool RUN = false>
 __global__ void __launch_bounds__(kThreads, Q4 ? 2 : LBT_BN_FWD2_CTAS) bn_fwd2_kernel(const Fwd2Params p) {
   extern __shared__ float s_par[];  // [4*C]: mean, den / m2, gq / m2, bq
   __shared__ uint32_t s_red[16];
@@ -384,12 +386,17 @@ __global__ void __launch_bounds__(kThreads, Q4 ? 2 : LBT_BN_FWD2_CTAS) bn_fwd2_k
   const DivN n = make_divn((unsigned long long)(p.t.n_outer * (p.t.n_inner / C)));
   for (int ch = threadIdx.x; ch < C; ch += kThreads) {
     float mean, var;
-    moments(p.sums, C, ch, n, c1.inv_m, mean, var);
+    if (RUN) {
+      mean = p.run_mean[ch];
+      var = p.run_var[ch];
+    } else {
+      moments(p.sums, C, ch, n, c1.inv_m, mean, var);
+    }
     s_par[ch] = mean;
     s_par[C + ch] = __fsqrt_rn(__fadd_rn(var, p.eps)) * c2.inv_m;  // (var + eps) ** 0.5 (dfxp:616), pre-divided by m2 (exact)
     s_par[2 * C + ch] = p.gq[ch] * c2.inv_m;                         // gq / m2 (exact)
     s_par[3 * C + ch] = p.bq[ch];
-    if (blockIdx.x == 0) {
+    if (!RUN && blockIdx.x == 0) {
       if (p.batch_mean) p.batch_mean[ch] = mean;
       if (p.batch_var) p.batch_var[ch] = var;
       if (p.run_mean) {  // momentum * average + (1 - momentum) * variable
@@ -482,7 +489,7 @@ __global__ void __launch_bounds__(kThreads, Q4 ? 2 : LBT_BN_FWD2_CTAS) bn_fwd2_k
             if (relu) y2 = fmaxf(0.0f, y2);                                             // tf.maximum(0.0, X), dfxp:986
             o[j] = y2;
           }
-          *reinterpret_cast<uint32_t*>(p.k2 + idx) = tm_pack4(t2);
+          if (!RUN || p.k2) *reinterpret_cast<uint32_t*>(p.k2 + idx) = tm_pack4(t2);
           if (has_out) *reinterpret_cast<float4*>(p.out + idx) = make_float4(o[0], o[1], o[2], o[3]);
           if (nxt) {                                                                    // the consumer's Xq, dfxp:287
             float t3[4];
@@ -548,7 +555,8 @@ struct Fwd2PoolParams {
   uint32_t tiles_x, tiles_img, rows_per_group, total_tiles;
 };
 
-template <bool MM>
+// RUN: eval mode, as in bn_fwd2_kernel (run_mean / run_var are the read-only source of mean / var, k2 optional)
+template <bool MM, bool RUN = false>
 __global__ void __launch_bounds__(kPoolThreads, 1) bn_fwd2_pool_kernel(const Fwd2PoolParams p) {
   extern __shared__ float4 s_y[];   // [2][kPoolTH + 1][kPoolTW + 1][kPoolCG]
   __shared__ float s_par[4 * 64];   // mean, den / m2, gq / m2, bq
@@ -561,12 +569,17 @@ __global__ void __launch_bounds__(kPoolThreads, 1) bn_fwd2_pool_kernel(const Fwd
   if (threadIdx.x < C) {
     const int ch = threadIdx.x;
     float mean, var;
-    moments(p.sums, C, ch, n, c1.inv_m, mean, var);
+    if (RUN) {
+      mean = p.run_mean[ch];
+      var = p.run_var[ch];
+    } else {
+      moments(p.sums, C, ch, n, c1.inv_m, mean, var);
+    }
     s_par[ch] = mean;
     s_par[C + ch] = __fsqrt_rn(__fadd_rn(var, p.eps)) * c2.inv_m;
     s_par[2 * C + ch] = p.gq[ch] * c2.inv_m;
     s_par[3 * C + ch] = p.bq[ch];
-    if (blockIdx.x == 0 && p.run_mean) {
+    if (!RUN && blockIdx.x == 0 && p.run_mean) {
       p.run_mean[ch] = __fadd_rn(__fmul_rn(p.momentum, p.run_mean[ch]), __fmul_rn(p.one_minus_momentum, mean));
       p.run_var[ch] = __fadd_rn(__fmul_rn(p.momentum, p.run_var[ch]), __fmul_rn(p.one_minus_momentum, var));
     }
@@ -672,7 +685,7 @@ __global__ void __launch_bounds__(kPoolThreads, 1) bn_fwd2_pool_kernel(const Fwd
       for (int q = 0; q < 4; ++q)
         if (pv[q]) {
           const uint32_t k2p = apply4(w[q], un[q], mx, mn, n1, n2, own[q]);
-          k2w[ibase + pw[q]] = k2p;
+          if (!RUN || k2w) k2w[ibase + pw[q]] = k2p;
           sy[((2 * by + (q >> 1)) * (kPoolTW + 1) + 2 * bx + (q & 1)) * kPoolCG + cg] = make_float4(own[q][0], own[q][1], own[q][2], own[q][3]);
         }
       if (hv) {
@@ -1433,14 +1446,23 @@ extern "C" int lbt_bn_fwd_quant_stats(const float* x, size_t n_outer, size_t n_i
   return check_launch("lbt_bn_fwd_quant_stats");
 }
 
+using Fwd2Kernel = void (*)(const Fwd2Params);
+template <bool RUN>
+Fwd2Kernel fwd2_kernel(bool mm, bool q4) {
+  return q4 ? (mm ? bn_fwd2_kernel<true, true, RUN> : bn_fwd2_kernel<false, true, RUN>)
+            : (mm ? bn_fwd2_kernel<true, false, RUN> : bn_fwd2_kernel<false, false, RUN>);
+}
+
+// running: eval mode — run_mean / run_var are the statistics (read only), `sums` and k2 are not used / optional
 static int bn_fwd_apply_run(const int8_t* k1, size_t n_outer, size_t n_inner, int C, int bits1, const int32_t* ib1,
                             const int64_t* sums, float eps, int bits2, const int32_t* ib2, const float* noise2,
                             uint64_t seed, uint64_t offset2, const uint64_t* dev_step, uint64_t* counters2,
                             const float* gamma_q, const float* beta_q, const float* add, int relu, int8_t* k2,
                             float* out, float* batch_mean, float* batch_var, float* run_mean, float* run_var,
                             double momentum, int stats_minmax, const lbt_qsite* q_next, void* next_mant, int next_kind,
-                            const lbt_qsite* q_next2, void* next_mant2, int next_kind2, void* stream) {
-  if (!k1 || !ib1 || !sums || !ib2 || !gamma_q || !beta_q || !k2) return LBT_EINVAL;
+                            const lbt_qsite* q_next2, void* next_mant2, int next_kind2, void* stream, bool running = false) {
+  if (!k1 || !ib1 || !ib2 || !gamma_q || !beta_q) return LBT_EINVAL;
+  if (running ? (!run_mean || !run_var || C <= 0 || (C & 3)) : (!sums || !k2)) return LBT_EINVAL;
   if (q_next2) {
     if (!q_next || !next_mant2 || !q_next2->ib || !al4(next_mant2) || (q_next2->noise && !al16(q_next2->noise))) return LBT_EINVAL;
     if (next_kind2 == LBT_MANT_U8 ? (q_next2->bits < 2 || q_next2->bits > 9 || !relu)
@@ -1458,14 +1480,13 @@ static int bn_fwd_apply_run(const int8_t* k1, size_t n_outer, size_t n_inner, in
   }
   if ((run_mean == nullptr) != (run_var == nullptr)) return LBT_EINVAL;
   if (n_outer == 0 || n_inner == 0) return LBT_OK;
-  if (!al4(k1) || !al4(k2) || (out && !al16(out)) || (add && !al16(add)) || (noise2 && !al16(noise2))) return LBT_EUNSUPPORTED;
+  if (!al4(k1) || (k2 && !al4(k2)) || (out && !al16(out)) || (add && !al16(add)) || (noise2 && !al16(noise2))) return LBT_EUNSUPPORTED;
   LBT_REQUIRE_ARCH();
   Fwd2Params p{};
   unsigned grid;
   // one statistics flavour per launch: min/max only when EVERY site of the launch asked for it (exact counts are always valid)
   const bool mm = stats_minmax && (!q_next || q_next->stats_minmax) && (!q_next2 || q_next2->stats_minmax);
-  void (*kern)(const Fwd2Params) = q_next2 ? (mm ? bn_fwd2_kernel<true, true> : bn_fwd2_kernel<false, true>)
-                                           : (mm ? bn_fwd2_kernel<true, false> : bn_fwd2_kernel<false, false>);
+  const Fwd2Kernel kern = running ? fwd2_kernel<true>(mm, q_next2 != nullptr) : fwd2_kernel<false>(mm, q_next2 != nullptr);
   int rc = make_tiling(p.t, n_outer, n_inner, C, grid, ctas_per_sm(kern, (size_t)4 * C * 4));
   if (rc) return rc;
   p.k1 = k1;
@@ -1493,7 +1514,7 @@ static int bn_fwd_apply_run(const int8_t* k1, size_t n_outer, size_t n_inner, in
   const size_t smem = (size_t)4 * C * 4;
   if ((rc = set_smem(kern, smem))) return rc;
   launch_pdl(kern, grid, kThreads, smem, reinterpret_cast<cudaStream_t>(stream), p);
-  return check_launch("lbt_bn_fwd_apply");
+  return check_launch(running ? "lbt_bn_fwd_apply_running" : "lbt_bn_fwd_apply");
 }
 
 extern "C" int lbt_bn_fwd_apply(const int8_t* k1, size_t n_outer, size_t n_inner, int C, int bits1, const int32_t* ib1,
@@ -1521,14 +1542,29 @@ extern "C" int lbt_bn_fwd_apply2(const int8_t* k1, size_t n_outer, size_t n_inne
                           q_next, next_mant, next_kind, q_next2, next_mant2, next_kind2, stream);
 }
 
-extern "C" int lbt_bn_fwd_apply_pooled(const int8_t* k1, size_t n_outer, int H, int W, int C, int bits1, const int32_t* ib1,
-                                       const int64_t* sums, float eps, int bits2, const int32_t* ib2, const float* noise2,
-                                       uint64_t seed, uint64_t offset2, const uint64_t* dev_step, uint64_t* counters2,
-                                       const float* gamma_q, const float* beta_q, int relu, int8_t* k2, float* run_mean,
-                                       float* run_var, double momentum, int stats_minmax, int k, int s, int pad_top, int pad_left,
-                                       int POH, int POW, float* pooled, uint8_t* pidx, const lbt_qsite* q_next, void* next_mant,
-                                       int next_kind, void* stream) {
-  if (!k1 || !ib1 || !sums || !ib2 || !gamma_q || !beta_q || !k2 || !pooled || !pidx) return LBT_EINVAL;
+extern "C" int lbt_bn_fwd_apply_running(const int8_t* k1, size_t n_outer, size_t n_inner, int C, int bits1, const int32_t* ib1,
+                                        const float* run_mean, const float* run_var, float eps, int bits2, const int32_t* ib2,
+                                        const float* noise2, uint64_t seed, uint64_t offset2, const uint64_t* dev_step,
+                                        uint64_t* counters2, const float* gamma_q, const float* beta_q, const float* add, int relu,
+                                        int8_t* k2, float* out, int stats_minmax, const lbt_qsite* q_next, void* next_mant,
+                                        int next_kind, const lbt_qsite* q_next2, void* next_mant2, int next_kind2, void* stream) {
+  // the kernel only reads the running statistics (the Fwd2Params slots are shared with the training update)
+  return bn_fwd_apply_run(k1, n_outer, n_inner, C, bits1, ib1, nullptr, eps, bits2, ib2, noise2, seed, offset2, dev_step, counters2,
+                          gamma_q, beta_q, add, relu, k2, out, nullptr, nullptr, const_cast<float*>(run_mean),
+                          const_cast<float*>(run_var), 0.0, stats_minmax, q_next, next_mant, next_kind, q_next2, next_mant2,
+                          next_kind2, stream, true);
+}
+
+// running: eval mode, as in bn_fwd_apply_run
+static int bn_fwd_apply_pooled_run(const int8_t* k1, size_t n_outer, int H, int W, int C, int bits1, const int32_t* ib1,
+                                   const int64_t* sums, float eps, int bits2, const int32_t* ib2, const float* noise2,
+                                   uint64_t seed, uint64_t offset2, const uint64_t* dev_step, uint64_t* counters2,
+                                   const float* gamma_q, const float* beta_q, int relu, int8_t* k2, float* run_mean,
+                                   float* run_var, double momentum, int stats_minmax, int k, int s, int pad_top, int pad_left,
+                                   int POH, int POW, float* pooled, uint8_t* pidx, const lbt_qsite* q_next, void* next_mant,
+                                   int next_kind, void* stream, bool running = false) {
+  if (!k1 || !ib1 || !ib2 || !gamma_q || !beta_q || !pooled || !pidx) return LBT_EINVAL;
+  if (running ? (!run_mean || !run_var || C <= 0 || (C & 3)) : (!sums || !k2)) return LBT_EINVAL;
   if (q_next) {
     if (!next_mant || !q_next->ib || !al4(next_mant) || (q_next->noise && !al16(q_next->noise))) return LBT_EINVAL;
     // u8 holds a 9-bit mantissa only when the tensor is non-negative, i.e. the ReLU is fused here
@@ -1543,7 +1579,7 @@ extern "C" int lbt_bn_fwd_apply_pooled(const int8_t* k1, size_t n_outer, int H, 
   if (C != 64 || k != 3 || s != 2 || pad_top != 0 || pad_left != 0 || POH != (H + 1) / 2 || POW != (W + 1) / 2) return LBT_EUNSUPPORTED;
   if (n_outer == 0) return LBT_OK;
   if ((uint64_t)n_outer * H * W * 16 >= (1ull << 31)) return LBT_EUNSUPPORTED;   // 32-bit word indices
-  if (!al4(k1) || !al4(k2) || !al16(pooled) || !al4(pidx) || (noise2 && !al16(noise2))) return LBT_EUNSUPPORTED;
+  if (!al4(k1) || (k2 && !al4(k2)) || !al16(pooled) || !al4(pidx) || (noise2 && !al16(noise2))) return LBT_EUNSUPPORTED;
   LBT_REQUIRE_ARCH();
   const DeviceInfo& di = device_info();
   Fwd2PoolParams p{};
@@ -1582,15 +1618,40 @@ extern "C" int lbt_bn_fwd_apply_pooled(const int8_t* k1, size_t n_outer, int H, 
   p.total_tiles = (uint32_t)total;
   const size_t smem = (size_t)2 * (kPoolTH + 1) * (kPoolTW + 1) * kPoolCG * sizeof(float4);
   const unsigned grid = (unsigned)total;
+  // one statistics flavour per launch (exact counts are always valid)
+  const bool mm = stats_minmax && (!q_next || q_next->stats_minmax);
+  void (*kern)(const Fwd2PoolParams) = running ? (mm ? bn_fwd2_pool_kernel<true, true> : bn_fwd2_pool_kernel<false, true>)
+                                               : (mm ? bn_fwd2_pool_kernel<true, false> : bn_fwd2_pool_kernel<false, false>);
   int rc;
-  if (stats_minmax && (!q_next || q_next->stats_minmax)) {   // one statistics flavour per launch (exact counts are always valid)
-    if ((rc = set_smem(bn_fwd2_pool_kernel<true>, smem))) return rc;
-    launch_pdl(bn_fwd2_pool_kernel<true>, grid, kPoolThreads, smem, reinterpret_cast<cudaStream_t>(stream), p);
-  } else {
-    if ((rc = set_smem(bn_fwd2_pool_kernel<false>, smem))) return rc;
-    launch_pdl(bn_fwd2_pool_kernel<false>, grid, kPoolThreads, smem, reinterpret_cast<cudaStream_t>(stream), p);
-  }
-  return check_launch("lbt_bn_fwd_apply_pooled");
+  if ((rc = set_smem(kern, smem))) return rc;
+  launch_pdl(kern, grid, kPoolThreads, smem, reinterpret_cast<cudaStream_t>(stream), p);
+  return check_launch(running ? "lbt_bn_fwd_apply_running_pooled" : "lbt_bn_fwd_apply_pooled");
+}
+
+extern "C" int lbt_bn_fwd_apply_pooled(const int8_t* k1, size_t n_outer, int H, int W, int C, int bits1, const int32_t* ib1,
+                                       const int64_t* sums, float eps, int bits2, const int32_t* ib2, const float* noise2,
+                                       uint64_t seed, uint64_t offset2, const uint64_t* dev_step, uint64_t* counters2,
+                                       const float* gamma_q, const float* beta_q, int relu, int8_t* k2, float* run_mean,
+                                       float* run_var, double momentum, int stats_minmax, int k, int s, int pad_top, int pad_left,
+                                       int POH, int POW, float* pooled, uint8_t* pidx, const lbt_qsite* q_next, void* next_mant,
+                                       int next_kind, void* stream) {
+  return bn_fwd_apply_pooled_run(k1, n_outer, H, W, C, bits1, ib1, sums, eps, bits2, ib2, noise2, seed, offset2, dev_step,
+                                 counters2, gamma_q, beta_q, relu, k2, run_mean, run_var, momentum, stats_minmax, k, s, pad_top,
+                                 pad_left, POH, POW, pooled, pidx, q_next, next_mant, next_kind, stream);
+}
+
+extern "C" int lbt_bn_fwd_apply_running_pooled(const int8_t* k1, size_t n_outer, int H, int W, int C, int bits1, const int32_t* ib1,
+                                               const float* run_mean, const float* run_var, float eps, int bits2, const int32_t* ib2,
+                                               const float* noise2, uint64_t seed, uint64_t offset2, const uint64_t* dev_step,
+                                               uint64_t* counters2, const float* gamma_q, const float* beta_q, int relu, int8_t* k2,
+                                               int stats_minmax, int k, int s, int pad_top, int pad_left, int POH, int POW,
+                                               float* pooled, uint8_t* pidx, const lbt_qsite* q_next, void* next_mant, int next_kind,
+                                               void* stream) {
+  // the kernel only reads the running statistics (the Fwd2PoolParams slots are shared with the training update)
+  return bn_fwd_apply_pooled_run(k1, n_outer, H, W, C, bits1, ib1, nullptr, eps, bits2, ib2, noise2, seed, offset2, dev_step,
+                                 counters2, gamma_q, beta_q, relu, k2, const_cast<float*>(run_mean), const_cast<float*>(run_var),
+                                 0.0, stats_minmax, k, s, pad_top, pad_left, POH, POW, pooled, pidx, q_next, next_mant, next_kind,
+                                 stream, true);
 }
 
 static int bn_bwd1_run(const float* g, const float* out, int relu, const int8_t* k2, const int8_t* k1,

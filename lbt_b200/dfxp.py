@@ -1291,16 +1291,18 @@ def _bn_fwd1(bn, xm_):
     return k1, sums
 
 
-def _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, next_site=None, next_kind=Q.MANT_NONE, want_fp32=True, next2=None):
+def _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, next_site=None, next_kind=Q.MANT_NONE, want_fp32=True, next2=None,
+             running=False):
     """BN forward pass 2 (+ residual add, ReLU, the consumer's input quantiser): (k2, out or None, next mantissas or None,
     relu_mode).  next2 = (site, kind): a second consumer's input quantiser; its mantissas come back as ``next2[2]`` (a list
-    cell the caller passes in)."""
+    cell the caller passes in).  running: eval mode — normalise with the running statistics (``sums`` is not read, the
+    running averages stay, k2 is None)."""
     norm, resc = bn[0], bn[1]
     rt = norm.qX.runtime
     N, C = k1.shape[0], k1.shape[-1]
     n_inner = k1.numel() // N
     dev = k1.device
-    k2 = torch.empty_like(k1)
+    k2 = None if running else torch.empty_like(k1)
     out = torch.empty(k1.shape, dtype=torch.float32, device=dev) if want_fp32 else None
     nz2, off2 = _site_args(resc.qX, k1)
     relu_mode = 0 if not relu else (2 if add_ is not None else 1)
@@ -1308,20 +1310,28 @@ def _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, next_site=None, next_kind=Q.MANT_
     if next_site is not None:
         qn = next_site.abi(n_inner, dev)
         nm = torch.empty(k1.shape, dtype=torch.uint8 if next_kind == Q.MANT_U8 else torch.int8, device=dev)
-    args = (_lib.ptr(k1), N, n_inner, C, norm.qX.bits, _lib.ptr(norm.qX.range), _lib.ptr(sums),
-            float(norm.eps), resc.qX.bits, _lib.ptr(resc.qX.range), _lib.ptr(nz2), rt.seed, off2,
-            _lib.ptr(rt.dev_step), _lib.ptr(resc.qX.counters), _lib.ptr(gq), _lib.ptr(bq), _lib.ptr(add_),
-            1 if relu else 0, _lib.ptr(k2), _lib.ptr(out), None, None, _lib.ptr(norm.X_mean_running),
-            _lib.ptr(norm.X_var_running), float(norm.momentum), int(resc.qX.target == 0),
-            ctypes.addressof(qn) if qn is not None else None, _lib.ptr(nm), int(next_kind))
-    nbytes = k1.numel() * (2 + (4 if want_fp32 else 0) + (4 if add_ is not None else 0) + (1 if nm is not None else 0))
+    qn2 = nm2 = None
     if next2 is not None and qn is not None:
         site2, kind2 = next2[0], next2[1]
         qn2 = site2.abi(n_inner, dev)
         nm2 = torch.empty(k1.shape, dtype=torch.uint8 if kind2 == Q.MANT_U8 else torch.int8, device=dev)
-        _lib.call('lbt_bn_fwd_apply2', *args, ctypes.addressof(qn2), _lib.ptr(nm2), int(kind2), _lib.stream(),
-                  meta=dict(bytes=nbytes + k1.numel()))
         next2[2] = nm2
+    nbytes = k1.numel() * ((1 if running else 2) + (4 if want_fp32 else 0) + (4 if add_ is not None else 0) +
+                           (1 if nm is not None else 0) + (1 if nm2 is not None else 0))
+    head = (_lib.ptr(k1), N, n_inner, C, norm.qX.bits, _lib.ptr(norm.qX.range))
+    site = (float(norm.eps), resc.qX.bits, _lib.ptr(resc.qX.range), _lib.ptr(nz2), rt.seed, off2,
+            _lib.ptr(rt.dev_step), _lib.ptr(resc.qX.counters), _lib.ptr(gq), _lib.ptr(bq), _lib.ptr(add_),
+            1 if relu else 0, _lib.ptr(k2), _lib.ptr(out))
+    nxt = (ctypes.addressof(qn) if qn is not None else None, _lib.ptr(nm), int(next_kind))
+    nxt2 = (ctypes.addressof(qn2), _lib.ptr(nm2), int(next2[1])) if qn2 is not None else ()
+    if running:
+        _lib.call('lbt_bn_fwd_apply_running', *head, _lib.ptr(norm.X_mean_running), _lib.ptr(norm.X_var_running), *site,
+                  int(resc.qX.target == 0), *nxt, *(nxt2 or (None, None, 0)), _lib.stream(), meta=dict(bytes=nbytes))
+        return k2, out, nm, relu_mode
+    args = head + (_lib.ptr(sums),) + site + (None, None, _lib.ptr(norm.X_mean_running), _lib.ptr(norm.X_var_running),
+                                               float(norm.momentum), int(resc.qX.target == 0)) + nxt
+    if nxt2:
+        _lib.call('lbt_bn_fwd_apply2', *args, *nxt2, _lib.stream(), meta=dict(bytes=nbytes))
     else:
         _lib.call('lbt_bn_fwd_apply', *args, _lib.stream(), meta=dict(bytes=nbytes))
     return k2, out, nm, relu_mode
@@ -1411,21 +1421,23 @@ class _FusedBNFn(torch.autograd.Function):
     activation (csrc/bn.cu), saving only the two s8 mantissa tensors for backward."""
 
     @staticmethod
-    def forward(ctx, x, gamma, beta, add, bn, relu):
+    def forward(ctx, x, gamma, beta, add, bn, relu, running=False):
+        # running: eval mode without an autograd graph (BatchNorm2d_q._running); nothing is saved
         x_ = _to_mem(x)
         k1, sums = _bn_fwd1(bn, x_)
         gq, bq = _bn_params(bn[1], gamma, beta)
         add_ = _to_mem(add) if add is not None else None
-        k2, out, _, relu_mode = _bn_fwd2(bn, k1, sums, gq, bq, add_, relu)
-        ctx.bn, ctx.relu_mode, ctx.has_add = bn, relu_mode, add is not None
-        ctx.save_for_backward(k1, k2, sums, gq, bq, out if relu_mode == 2 else None)
+        k2, out, _, relu_mode = _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, running=running)
+        if not running:
+            ctx.bn, ctx.relu_mode, ctx.has_add = bn, relu_mode, add is not None
+            ctx.save_for_backward(k1, k2, sums, gq, bq, out if relu_mode == 2 else None)
         return _from_mem(out)
 
     @staticmethod
     def backward(ctx, g):
         k1, k2, sums, gq, bq, out = ctx.saved_tensors
         dx, _, dgamma, dbeta, d_add = _bn_backward(ctx.bn, _to_mem(g), k1, k2, sums, gq, bq, out, ctx.relu_mode, ctx.has_add)
-        return _from_mem(dx), dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None), None, None
+        return _from_mem(dx), dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None), None, None, None
 
 
 _link_count = 0        # fused backward links taken (tests)
@@ -1474,7 +1486,9 @@ class _ConvBNFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight, gamma, beta, add, conv, bn, relu, next_site, next_kind, want_fp32, alias, link_in, link_out, pool=None,
-                next2=None):
+                next2=None, running=False):
+        # running: eval mode without an autograd graph (BatchNorm2d_q._running): the BN kernels normalise with the running
+        # statistics, nothing is saved for backward
         geom = _conv_geom(conv, x, weight)
         N, H, W, Cin, Cout, kh, kw, sh, sw, pt, pl, OH, OW = geom
         norm, resc = bn[0], bn[1]
@@ -1495,7 +1509,7 @@ class _ConvBNFn(torch.autograd.Function):
         if pool is not None and FUSE_POOL_FWD and add is None and Cout == 64 and pool[:4] == (3, 2, 0, 0):
             # the ImageNet stem: BN apply + ReLU + 3x3/2 max-pool in ONE kernel, the fp32 module output never exists
             pk, ps, ppt, ppl, POH, POW = pool
-            k2 = torch.empty_like(k1)
+            k2 = None if running else torch.empty_like(k1)
             pooled = torch.empty(N, POH, POW, Cout, dtype=torch.float32, device=dev)
             pidx = torch.empty(N, POH, POW, Cout, dtype=torch.uint8, device=dev)
             nz2, off2 = _site_args(resc.qX, k1)
@@ -1503,24 +1517,31 @@ class _ConvBNFn(torch.autograd.Function):
             if next_site is not None:
                 qn = next_site.abi(POH * POW * Cout, dev)
                 nmp = torch.empty(N, POH, POW, Cout, dtype=torch.uint8 if next_kind == Q.MANT_U8 else torch.int8, device=dev)
-            if _lib.try_call('lbt_bn_fwd_apply_pooled', _lib.ptr(k1), N, OH, OW, Cout, norm.qX.bits, _lib.ptr(norm.qX.range),
-                             _lib.ptr(sums), float(norm.eps), resc.qX.bits, _lib.ptr(resc.qX.range), _lib.ptr(nz2), rt.seed, off2,
-                             _lib.ptr(rt.dev_step), _lib.ptr(resc.qX.counters), _lib.ptr(gq), _lib.ptr(bq), 1 if relu else 0,
-                             _lib.ptr(k2), _lib.ptr(norm.X_mean_running), _lib.ptr(norm.X_var_running), float(norm.momentum),
-                             int(resc.qX.target == 0), pk, ps, ppt, ppl, POH, POW, _lib.ptr(pooled), _lib.ptr(pidx),
-                             ctypes.addressof(qn) if qn is not None else None, _lib.ptr(nmp), int(next_kind), _lib.stream(),
-                             meta=dict(bytes=k1.numel() * 2 + pooled.numel() * (5 + (1 if nmp is not None else 0)))):
+            head = (_lib.ptr(k1), N, OH, OW, Cout, norm.qX.bits, _lib.ptr(norm.qX.range))
+            site = (float(norm.eps), resc.qX.bits, _lib.ptr(resc.qX.range), _lib.ptr(nz2), rt.seed, off2,
+                    _lib.ptr(rt.dev_step), _lib.ptr(resc.qX.counters), _lib.ptr(gq), _lib.ptr(bq), 1 if relu else 0, _lib.ptr(k2))
+            tail = (pk, ps, ppt, ppl, POH, POW, _lib.ptr(pooled), _lib.ptr(pidx),
+                    ctypes.addressof(qn) if qn is not None else None, _lib.ptr(nmp), int(next_kind), _lib.stream())
+            meta = dict(bytes=k1.numel() * (1 if running else 2) + pooled.numel() * (5 + (1 if nmp is not None else 0)))
+            if running:
+                done = _lib.try_call('lbt_bn_fwd_apply_running_pooled', *head, _lib.ptr(norm.X_mean_running),
+                                     _lib.ptr(norm.X_var_running), *site, int(resc.qX.target == 0), *tail, meta=meta)
+            else:
+                done = _lib.try_call('lbt_bn_fwd_apply_pooled', *head, _lib.ptr(sums), *site, _lib.ptr(norm.X_mean_running),
+                                     _lib.ptr(norm.X_var_running), float(norm.momentum), int(resc.qX.target == 0), *tail,
+                                     meta=meta)
+            if done:
                 out, nm, relu_mode = None, nmp, (1 if relu else 0)
             else:
                 pooled = pidx = None
                 next_site, next_kind = None, Q.MANT_NONE
         if pooled is None:
             k2, out, nm, relu_mode = _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, next_site, next_kind, True if pool is not None else want_fp32,
-                                              next2=next2 if pool is None else None)
+                                              next2=next2 if pool is None else None, running=running)
         ctx.conv, ctx.bn, ctx.geom, ctx.xkind, ctx.prep = conv, bn, geom, xkind, prep
         ctx.relu_mode, ctx.has_add = relu_mode, add is not None
         ctx.link_in, ctx.link_out = link_in, link_out
-        if link_out is not None and out is None:     # the next unit may run this BN's backward pass 1 in its dgrad epilogue
+        if link_out is not None and out is None and not running:     # the next unit may run this BN's backward pass 1 in its dgrad epilogue
             link_out.offer(bn, k1, k2, gq, bq, relu_mode, add is not None)
         ctx.pool = None
         if pooled is not None:    # lbt_bn_fwd_apply_pooled did both
@@ -1534,7 +1555,8 @@ class _ConvBNFn(torch.autograd.Function):
                       _lib.stream(), meta=dict(bytes=out.numel() * 4 + pooled.numel() * 5))
             ctx.pool = (pk, ps, ppt, ppl, POH, POW)
             out = pooled
-        ctx.save_for_backward(xm, wm, k1, k2, sums, gq, bq, out if relu_mode == 2 else None, pidx)
+        if not running:
+            ctx.save_for_backward(xm, wm, k1, k2, sums, gq, bq, out if relu_mode == 2 else None, pidx)
         if out is None:       # mantissa-only activation: the fp32 tensor is never materialised (shape carrier only)
             out = torch.empty(1, dtype=torch.float32, device=dev).expand(N, OH, OW, Cout)
         if nm is None:
@@ -1574,7 +1596,8 @@ class _ConvBNFn(torch.autograd.Function):
         else:
             dx, dW, _ = _conv_backward(conv, ctx.geom, xm, ctx.xkind, wm, ctx.prep, gm, need_dx, need_dw, False, addend=addend, link=li)
         return ((_from_mem(dx) if dx is not None else None), dW, dgamma, dbeta,
-                (_from_mem(d_add) if d_add is not None else None), None, None, None, None, None, None, None, None, None, None, None)
+                (_from_mem(d_add) if d_add is not None else None), None, None, None, None, None, None, None, None, None, None, None,
+                None)
 
 
 FUSE_POOL = os.environ.get('LBT_FUSE_POOL', '0') == '1'   # module switch: a MaxPool_q right behind a fused unit runs its backward inside the
@@ -1584,16 +1607,17 @@ FUSE_POOL = os.environ.get('LBT_FUSE_POOL', '0') == '1'   # module switch: a Max
 FUSE_BN_BWD = False   # module switch: both BN backward passes in ONE launch (lbt_bn_bwd_fused, grid barrier) where the
                       # tensor is one wave of CTAs.  Bit-identical; measured no faster on B200 (1.77 vs 1.75 ms ResNet-20
                       # step: the barrier + second fp64 prologue cost what the saved launch gains), so off by default
-FUSE_UNITS = True     # module switch for the Conv2d_q + BatchNorm2d_q fused units (tests compare both settings)
+FUSE_UNITS = True     # module switch for the Conv2d_q + BatchNorm2d_q fused units (tests compare both settings); in eval mode it
+                      # also selects the running-statistics kernels of a stand-alone BatchNorm2d_q (off: the eager reference path)
 DUAL_WGRAD = os.environ.get('LBT_DUAL_WGRAD', '1') != '0'   # 16-bit gradients: weight gradient of both byte planes in one launch
 DUAL_HALO = os.environ.get('LBT_DUAL_HALO', '1') != '0'     # 16-bit gradients: stride-1 3x3 input gradients through lbt_conv_i8_fprop_dual
 FUSE_NEXT2 = os.environ.get('LBT_FUSE_NEXT2', '1') != '0'   # a strided block's shortcut convolution gets its input mantissas from the
                       # kernel that produced the block input too (lbt_bn_fwd_apply2) instead of a separate lbt_quantize
 
 
-def _unit_fusable(conv, bn, x):
+def _unit_fusable(conv, bn, x, running=False):
     return (FUSE_UNITS and isinstance(conv, Conv2d_q) and isinstance(bn, BatchNorm2d_q) and conv.bias is None and conv.fuse_bn and
-            bn._can_fuse_c(conv.weight.shape[3], 4) and conv.qG.bits <= 16 and conv.qW.bits <= 8 and conv.qX.bits <= 9 and
+            bn._can_fuse_c(conv.weight.shape[3], 4, running) and conv.qG.bits <= 16 and conv.qW.bits <= 8 and conv.qX.bits <= 9 and
             x.is_cuda)
 
 
@@ -1605,7 +1629,8 @@ def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=Tr
     and the mantissas travel with the returned tensor (``_lbt_q``); want_fp32=False (only legal when next_conv is the
     ONLY consumer) skips the fp32 tensor altogether."""
     relu = relu or getattr(bn, 'relu', False)
-    if not _unit_fusable(conv, bn, x):
+    running = isinstance(bn, BatchNorm2d_q) and bn._running(x, add, conv.weight)
+    if not _unit_fusable(conv, bn, x, running):
         y = bn(conv(x), add=add, relu=relu) if isinstance(bn, BatchNorm2d_q) else bn(conv(x))
         if pool is not None:
             y = pool(y)
@@ -1645,7 +1670,7 @@ def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=Tr
     use_alias = bool(alias and x.requires_grad and not getattr(x, '_lbt_hollow', False) and conv.weight.shape[2] <= 128)
     out, nm, xa = _ConvBNFn.apply(x, conv.weight, bn[1].gamma, bn[1].beta, add, conv, bn, relu, next_site, next_kind,
                                   want_fp32, use_alias, link_in if FUSE_BWD_LINK else None, link_out if FUSE_BWD_LINK else None,
-                                  pgeom, next2)
+                                  pgeom, next2, running)
     if next_site is not None and nm.numel():       # (empty: the pooled one-kernel path declined, the consumer quantises itself)
         out._lbt_q = {id(next_site): (nm, next_kind)}
         if next2 is not None and next2[2] is not None:
@@ -1701,7 +1726,8 @@ class BatchNorm2d_q(nn.Sequential):
 
     In training mode with <= 8-bit activation quantisers, <= 16-bit gradient quantisers and C % 4 == 0 the pair runs as the fused kernels of
     csrc/bn.cu; ``forward(x, add=None, relu=False)`` can additionally fold the residual sum and the ReLU
-    that follow it in the reference's blocks (dfxp:862, 986).  Otherwise the two sub-modules run one
+    that follow it in the reference's blocks (dfxp:862, 986).  In eval mode the same kernels normalise with the running
+    statistics (dfxp:616) when no autograd graph is recorded (see ``_running``).  Otherwise the two sub-modules run one
     after the other."""
 
     def __init__(self, bits, num_features, momentum=0.999, eps=1e-5, *, weight_decay=0.0, target_overflow_rate=0.0,
@@ -1717,19 +1743,29 @@ class BatchNorm2d_q(nn.Sequential):
         self.fused = fused
         self.relu = relu            # apply the ReLU that follows this BN in the reference's layer lists
 
-    def _can_fuse_c(self, C, dim):
+    def _can_fuse_c(self, C, dim, running=False):
         norm, resc = self[0], self[1]
-        return (self.fused and self.training and dim in (2, 4) and C % 4 == 0 and
+        return (self.fused and (self.training or running) and dim in (2, 4) and C % 4 == 0 and
                 max(norm.qX.bits, resc.qX.bits) <= 8 and max(norm.qG.bits, resc.qG.bits) <= 16 and
                 min(norm.qX.bits, resc.qX.bits, norm.qG.bits, resc.qG.bits) >= 2)
 
-    def _can_fuse(self, x):
-        return self._can_fuse_c(x.shape[1], x.dim())
+    def _can_fuse(self, x, running=False):
+        return self._can_fuse_c(x.shape[1], x.dim(), running)
+
+    def _running(self, *inputs):
+        """Eval mode on the fused kernels: normalise with the running statistics.  Only where no autograd graph is recorded
+        (a backward pass through running-statistics batch-norm is not built: eval mode with gradients keeps the eager path),
+        and only with FUSE_UNITS on (off, eval mode runs the eager reference arithmetic)."""
+        if self.training or not FUSE_UNITS:
+            return False
+        return not torch.is_grad_enabled() or not any(t is not None and t.requires_grad
+                                                      for t in inputs + (self[1].gamma, self[1].beta))
 
     def forward(self, x, add=None, relu=False):
         relu = relu or self.relu
-        if self._can_fuse(x):
-            return _FusedBNFn.apply(x, self[1].gamma, self[1].beta, add, self, relu)
+        running = self._running(x, add)
+        if self._can_fuse(x, running):
+            return _FusedBNFn.apply(x, self[1].gamma, self[1].beta, add, self, relu, running)
         y = self[1](self[0](x))
         if add is not None:
             y = y + add

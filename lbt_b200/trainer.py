@@ -246,17 +246,21 @@ class Trainer:
 
     # ---- evaluation (trainer.py:164-187) ---------------------------------------------------------------------------
     @torch.no_grad()
-    def evaluate(self, X, y, batch_size=1000):
+    def evaluate(self, X, y, batch_size=1000, running_stats=False):
         """Mean loss and accuracy over (X, y) in batches of ``batch_size`` — the reference's test loop.  Like the
         reference (its ``set_testing`` call is commented out, trainer.py:164-165, "TODO BatchNorm bug") the forward pass
-        runs in TRAINING mode: batch statistics, stochastic quantisers; nothing is updated — no range controller
-        (``update_range_op`` is not fetched), no running statistics, no step counter."""
+        runs in TRAINING mode by default: batch statistics, stochastic quantisers; nothing is updated — no range controller
+        (``update_range_op`` is not fetched), no running statistics, no step counter.
+        ``running_stats=True``: the batches run in eval mode instead (``model.eval()``: batch-norm with the running
+        statistics, no dropout) on the fused kernels; the module's previous mode is restored afterwards.  Quantisers stay
+        stochastic, with the same per-batch noise positions, and nothing is updated either."""
         from .dfxp import Normalization_q
         rt = self.model.runtime
-        norms = [m for m in self.model.modules() if isinstance(m, Normalization_q)]
+        norms = [] if running_stats else [m for m in self.model.modules() if isinstance(m, Normalization_q)]
         saved = [m.momentum for m in norms]
         for m in norms:
             m.momentum = 1.0                       # running <- 1.0 * running + 0.0 * batch: unchanged
+        modes = [(m, m.training) for m in self.model.modules()]
         counters = rt.flat['counters'].clone()
         # the reference draws fresh quantiser / dropout noise at every sess.run (dfxp:36): every test batch gets its own
         # position of the Philox stream, disjoint from the training steps' (bit 31 of the step word), and the training
@@ -265,6 +269,8 @@ class Trainer:
         base = (int(step_saved.item()) & 0x7FFFF) << 12
         loss_sum, acc_sum, n_batches = 0.0, 0.0, 0
         try:
+            if running_stats:
+                self.model.eval()
             for i in range(0, X.shape[0], batch_size):
                 xb, yb = X[i:i + batch_size], y[i:i + batch_size]
                 rt.dev_step.fill_(0x80000000 | ((base + n_batches) & 0x7FFFFFFF))
@@ -275,17 +281,19 @@ class Trainer:
         finally:
             for m, mom in zip(norms, saved):
                 m.momentum = mom
+            for m, mode in modes:
+                m.training = mode
             rt.flat['counters'].copy_(counters)    # the overflow statistics of a test batch never reach the controller
             rt.dev_step.copy_(step_saved)
         return loss_sum / max(1, n_batches), acc_sum / max(1, n_batches)          # mean of per-batch means, as trainer.py:185-186
 
     # ---- the epoch loop (trainer.py:109-187) ---------------------------------------------------------------------------
     def fit(self, pipeline, n_epoch, batch_size, *, lr_decay_factor=0.1, decay_epochs=(80, 120, 140), test=None, log=None,
-            max_batches=None, graph=False):
+            max_batches=None, graph=False, eval_running_stats=False):
         """``pipeline``: lbt_b200.data.Pipeline over the device-resident training set (shuffle + flip / pad-4 / crop on
         the GPU).  The learning rate is multiplied by ``lr_decay_factor`` at epochs 80, 120 and 140 and the optimizer is
         re-created (momentum slots zeroed) exactly there (trainer.py:117-132).  ``test`` = (X, y) evaluated after each
-        epoch.  ``graph=True``: full batches run as replays of the captured step (capture() on first use; the pipeline
+        epoch (``eval_running_stats``: see ``evaluate(running_stats=...)``).  ``graph=True``: full batches run as replays of the captured step (capture() on first use; the pipeline
         writes each batch straight into the static inputs), a short last batch runs eagerly.  With several replicas the
         pipeline must be rank-aware (lbt_b200.data.Pipeline shards every global batch by rank).
         Returns [(epoch, last_train_loss, test_loss, test_acc)]."""
@@ -312,7 +320,7 @@ class Trainer:
                 if log is not None and (b + 1) % 100 == 0:
                     log('Batch %d loss %f' % (b + 1, float(loss)))
             self.check()
-            tl, ta = self.evaluate(*test) if test is not None else (None, None)
+            tl, ta = self.evaluate(*test, running_stats=eval_running_stats) if test is not None else (None, None)
             history.append((epoch, float(loss) if loss is not None else None, tl, ta))
             if log is not None and ta is not None:
                 log('Epoch %d test accuracy %f' % (epoch + 1, ta))
