@@ -684,6 +684,26 @@ int lbt_conv_i8_dgrad_strided(const void* g, int g_kind, int N, int OH, int OW, 
                               int Cin, int kh, int kw, int sh, int sw, int pad_top, int pad_left, int H, int W,
                               const int32_t* ib_g, const int32_t* ib_w, int exp_const, float* dx, size_t ldc,
                               const float* addend, void* stream);
+/*
+ * The whole input gradient of a downsampling residual block in ONE launch:
+ *   dX = dgrad_{kh x kw / (sh, sw)}(g, w2) [+ dgrad_{1x1 / (sh, sw)}(g_short, w_short)] [+ addend]
+ * The main term is lbt_conv_i8_dgrad_strided's parity-class decomposition (same operands: g[N,OH,OW,Cout], w2 in parity-class
+ * order, e = exp_const + *ib_g + *ib_w), all classes in one tile list.  g_short[N, OHs, OWs, Cout_s] (or NULL) is the output
+ * gradient of a 1x1 shortcut convolution of stride (sh, sw) without padding over the same input, w_short[Cin, Cout_s] (row
+ * pitch ldws) its filter, e_s = exp_short + *ib_gs + *ib_ws; it samples parity class (0, 0), so OHs x OWs must be
+ * ceil(H / sh) x ceil(W / sw).  Where the shortcut lands dX = RN(RN(main * 2^e) + RN(short * 2^e_s)), elsewhere RN(main * 2^e):
+ * bit-identical to lbt_conv_i8_dgrad_strided on the shortcut followed by lbt_conv_i8_dgrad_strided on the main convolution
+ * with that result as addend.  addend (the layout of dX) only without a shortcut.  Null pointers, bad kinds or shapes:
+ * LBT_EINVAL; Cin % 4 != 0, strides > 2, Cin neither 64 nor a multiple of 128, Cout (Cout_s) not 32, 64 or a multiple of 128
+ * (with the same channel chunk), misalignment, a shortcut lattice that does not match or a shortcut together with addend:
+ * LBT_EUNSUPPORTED — all before any CUDA call.  Run the two lbt_conv_i8_dgrad_strided calls then.
+ */
+int lbt_conv_i8_dgrad_block(const void* g, int g_kind, int N, int OH, int OW, int Cout, const void* w2, int w_kind, size_t ldw,
+                            int Cin, int kh, int kw, int sh, int sw, int pad_top, int pad_left, int H, int W,
+                            const int32_t* ib_g, const int32_t* ib_w, int exp_const, const void* g_short, int gs_kind,
+                            int OHs, int OWs, int Cout_s, const void* w_short, int ws_kind, size_t ldws,
+                            const int32_t* ib_gs, const int32_t* ib_ws, int exp_short, float* dx, size_t ldc,
+                            const float* addend, void* stream);
 /* The same for a 9..16-bit gradient given as its byte planes k = 256 * hi + lo (g_hi s8, g_lo u8; BASELINE config 5): every class is
  * a dual-accumulator convolution (lbt_conv_i8_fprop_dual's kernels), one rounding.  Cin >= 64, Cout == 64 or a multiple of 128. */
 int lbt_conv_i8_dgrad_strided_dual(const int8_t* g_hi, const uint8_t* g_lo, int N, int OH, int OW, int Cout, const void* w2,

@@ -106,6 +106,9 @@ SIGNATURES = {
     'lbt_conv_i8_dgrad_strided': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_size_t, c_int, c_int, c_int,
                                           c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p, c_size_t,
                                           c_void_p, c_void_p]),
+    'lbt_conv_i8_dgrad_block': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_size_t] + [c_int] * 9 +
+                                [c_void_p, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_size_t,
+                                 c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p, c_void_p]),
     'lbt_dp_step': (c_int, [c_void_p, c_void_p, c_size_t, c_float, c_void_p, c_float, c_int, c_void_p, c_void_p, c_void_p,
                             c_size_t, c_void_p, c_void_p]),
     'lbt_dp_export': (c_int, [c_void_p, c_void_p, c_void_p]),

@@ -99,6 +99,52 @@ extern "C" int lbt_conv_i8_dgrad_strided(const void* g, int g_kind, int N, int O
                            exp_const, dx, ldc, addend, stream);
 }
 
+// The whole input gradient of a downsampling block in one launch (conv_i8.cu, conv_dgrad_block_kernel): every parity class
+// of the main convolution's dgrad and, in a second accumulator of the class it samples, the 1x1/s shortcut's dgrad.
+extern "C" int lbt_conv_i8_dgrad_block(const void* g, int g_kind, int N, int OH, int OW, int Cout, const void* w2, int w_kind, size_t ldw,
+                                       int Cin, int kh, int kw, int sh, int sw, int pad_top, int pad_left, int H, int W,
+                                       const int32_t* ib_g, const int32_t* ib_w, int exp_const, const void* g_short, int gs_kind,
+                                       int OHs, int OWs, int Cout_s, const void* w_short, int ws_kind, size_t ldws,
+                                       const int32_t* ib_gs, const int32_t* ib_ws, int exp_short, float* dx, size_t ldc,
+                                       const float* addend, void* stream) {
+  w_kind &= ~LBT_MANT_PREPARED;
+  ws_kind &= ~LBT_MANT_PREPARED;
+  if (!g || !w2 || !dx || !ib_g || !ib_w) return LBT_EINVAL;
+  if ((g_kind != LBT_MANT_S8 && g_kind != LBT_MANT_U8) || (w_kind != LBT_MANT_S8 && w_kind != LBT_MANT_U8)) return LBT_EINVAL;
+  if (N <= 0 || H <= 0 || W <= 0 || Cin <= 0 || Cout <= 0 || kh <= 0 || kw <= 0 || sh <= 0 || sw <= 0 || OH <= 0 || OW <= 0)
+    return LBT_EINVAL;
+  if (pad_top < 0 || pad_left < 0 || ldc < (size_t)Cin || ldw < (size_t)kh * kw * Cout) return LBT_EINVAL;
+  if (g_short) {
+    if (!w_short || !ib_gs || !ib_ws) return LBT_EINVAL;
+    if ((gs_kind != LBT_MANT_S8 && gs_kind != LBT_MANT_U8) || (ws_kind != LBT_MANT_S8 && ws_kind != LBT_MANT_U8)) return LBT_EINVAL;
+    if (OHs <= 0 || OWs <= 0 || Cout_s <= 0 || ldws < (size_t)Cout_s) return LBT_EINVAL;
+    // the 1x1 / (sh, sw) shortcut without padding samples exactly parity class (0, 0), in g_short's row order
+    if (OHs != (H + sh - 1) / sh || OWs != (W + sw - 1) / sw) return LBT_EUNSUPPORTED;
+    if (addend) return LBT_EUNSUPPORTED;   // one sum per element: the shortcut term or an external addend
+  }
+  const int cb = Cout >= 128 ? 128 : Cout;
+  if (Cin % 4) return LBT_EUNSUPPORTED;
+  if (sh > 2 || sw > 2 || (cb != 32 && cb != 64 && cb != 128) || Cout % cb || (Cin != 64 && Cin % 128)) return LBT_EUNSUPPORTED;
+  if (g_short && (Cout_s % cb || Cout_s > 65536 || (Cout_s >= 128 ? 128 : Cout_s) != cb)) return LBT_EUNSUPPORTED;
+  if ((size_t)kh * kw * Cout > 65536 || kh > 255 || kw > 255) return LBT_EUNSUPPORTED;   // exactness bound of one s32 accumulator
+  if ((size_t)N * H * W >= (1ull << 31)) return LBT_EUNSUPPORTED;
+  if ((reinterpret_cast<uintptr_t>(g) & 15) || (reinterpret_cast<uintptr_t>(w2) & 15) || (ldw & 15) || (ldc & 3) ||
+      (reinterpret_cast<uintptr_t>(dx) & 15) || (addend && (reinterpret_cast<uintptr_t>(addend) & 15)) ||
+      (g_short && ((reinterpret_cast<uintptr_t>(g_short) & 15) || (reinterpret_cast<uintptr_t>(w_short) & 15) || (ldws & 15))))
+    return LBT_EUNSUPPORTED;
+  for (int a = 0; a < sh; ++a) {
+    const int r0 = (a + pad_top) % sh, nr = class_count(r0, kh, sh);
+    if (nr && nr - 1 - (a + pad_top) / sh < 0) return LBT_EUNSUPPORTED;
+  }
+  for (int b = 0; b < sw; ++b) {
+    const int s0 = (b + pad_left) % sw, nc = class_count(s0, kw, sw);
+    if (nc && nc - 1 - (b + pad_left) / sw < 0) return LBT_EUNSUPPORTED;
+  }
+  return conv_dgrad_block_run(g, g_kind, N, OH, OW, Cout, w2, w_kind, ldw, Cin, kh, kw, sh, sw, pad_top, pad_left, H, W, ib_g, ib_w,
+                              exp_const, g_short, gs_kind, Cout_s, w_short, ws_kind, ldws, ib_gs, ib_ws, exp_short, dx, ldc, addend,
+                              stream);
+}
+
 extern "C" int lbt_conv_i8_dgrad_strided_dual(const int8_t* g_hi, const uint8_t* g_lo, int N, int OH, int OW, int Cout, const void* w2,
                                               int w_kind, size_t ldw, int Cin, int kh, int kw, int sh, int sw, int pad_top, int pad_left,
                                               int H, int W, const int32_t* ib_g, const int32_t* ib_w, int exp_const, float* dx, size_t ldc,

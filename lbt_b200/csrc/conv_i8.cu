@@ -14,6 +14,7 @@
 // Channel chunk Cb = min(C, 128) in {16, 32, 64, 128} selects the shared-memory layout: 16-byte rows of
 // interleaved 8x16B core matrices, or 32/64/128-byte swizzled rows; a pipeline stage always carries 128 bytes
 // of K per row (128/Cb tap-blocks), i.e. four K=32 MMAs.  Same warp roles and mbarrier protocol as gemm_i8.cu.
+#include "conv_classes.h"
 #include "conv_internal.h"
 #include "qsite.cuh"
 #include "tcgen05.cuh"
@@ -978,6 +979,440 @@ extern "C" int lbt_conv_i8_wgrad_dual(const void* src, int src_kind, int N, int 
   if (!g_lo) return LBT_EINVAL;
   return conv_wgrad_run(src, src_kind, N, H, W, C, g_hi, LBT_MANT_S8, g_lo, Cout, kh, kw, sh, sw, pad_top, pad_left, OH, OW, acc64,
                         alpha, k_splits, stream);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Input gradient of a downsampling block in ONE persistent launch (lbt_conv_i8_dgrad_block):
+//
+//   dX = dgrad_{kh x kw / s}(g, W2)  [+ dgrad_{1x1 / s}(g_short, W_short)]  [+ addend]
+//
+// The tile list runs over (parity class, M tile, N tile) of every class of lbt_conv_i8_dgrad_strided's decomposition, classes
+// with the most K-steps first and each class's tiles together (its slice of g stays in L2).  Per class: its own im2col map of
+// g (sub-filter extents and padding differ), the K column of its sub-filter in the class-ordered W2 and the (a::sh, b::sw)
+// sub-lattice of dX it writes.  The 1x1/s shortcut samples exactly class (0, 0): its rows are g_short's rows in order, so its
+// K-steps (plain 2-D tiles of g_short and W_short) go into a second accumulator at +BN columns of the same tile, and the
+// epilogue writes RN(f_main + f_short) there — the rounding of the shortcut dgrad followed by the main dgrad with it as
+// addend.  Classes no tap reaches (a 1x1/s main convolution) are tiles without K-steps: the epilogue writes the addend or 0.
+// ------------------------------------------------------------------------------------------------
+namespace lbt {
+namespace {
+
+constexpr int kBlkMaxClasses = 4;   // strides <= 2
+
+struct BlkClass {
+  uint32_t M, OW, OHW;       // pixels of the class, its grid width, Hc * Wc
+  FastDiv d_OW, d_OHW;
+  int lower_w, lower_h;      // -pad_left, -pad_top of the class's stride-1 sub-convolution
+  uint32_t kw;               // sub-filter width
+  uint32_t ksteps;           // main K-steps (taps * channel chunks; 0: no tap reaches the class)
+  uint32_t kcol;             // first K column of the sub-filter in W2
+  uint32_t shortcut;         // 1: the shortcut's pixels are this class's pixels
+  uint32_t tile0, m_tiles;   // first tile of the class in the tile list, its M tiles
+  long long out_off;         // element offset of the class's first pixel in dX
+};
+
+struct BlkParams {
+  uint32_t nclasses;
+  BlkClass cls[kBlkMaxClasses];
+  uint32_t total_tiles, n_tiles, N;   // N: dX channels
+  uint32_t cb, mode;                  // channel chunk bytes of g and g_short, log2(cb / 16)
+  uint32_t cchunks_g;                 // Cout / cb
+  uint32_t ks_short;                  // shortcut K-steps (0: no shortcut)
+  const int32_t *ib_g, *ib_w, *ib_gs, *ib_ws;
+  int exp_const, exp_short;
+  const float* addend;
+  float* out;
+  long long rs_n, rs_y, rs_x;
+  uint32_t idesc, idesc_s;
+};
+
+struct BlkMaps {
+  CUtensorMap a[kBlkMaxClasses];   // im2col of g per class
+  CUtensorMap b;                   // W2[Cin, kh*kw*Cout]
+  CUtensorMap as, bs;              // g_short rows, W_short[Cin, Cout_s]
+};
+
+// Two accumulators (main, shortcut) per TMEM stage; two CTAs per SM share the 512 columns
+template <int BN>
+struct BCfg {
+  static constexpr int kStageA = Cfg<BN>::kStageA;
+  static constexpr int kStageB = Cfg<BN>::kStageB;
+  static constexpr int kStageBytes = kStageA + kStageB;
+  static constexpr int kCtasPerSm = 2;
+  static constexpr int kStages = BN <= 64 ? 4 : 3;
+  static constexpr int kSmemBytes = kStages * kStageBytes + 1024;
+  static constexpr int kAccW = 2 * BN;
+  static constexpr int kAccStages = (512 / kCtasPerSm) / kAccW;
+  static constexpr int kTmemCols = kAccStages * kAccW;
+  static_assert(kAccStages >= 1, "block dgrad accumulators");
+  static_assert(kCtasPerSm * kSmemBytes <= 227 * 1024, "shared memory budget");
+  static_assert(kCtasPerSm * kTmemCols <= 512, "tensor memory budget");
+};
+
+__device__ __forceinline__ uint32_t blk_class_of(const BlkParams& p, uint32_t tile) {
+  uint32_t c = 0;
+  while (c + 1 < p.nclasses && tile >= p.cls[c + 1].tile0) ++c;
+  return c;
+}
+
+template <int BN>
+__global__ void __launch_bounds__(kThreadsF, BCfg<BN>::kCtasPerSm)
+conv_dgrad_block_kernel(const __grid_constant__ BlkMaps maps, const __grid_constant__ BlkParams p) {
+  using C = BCfg<BN>;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  __shared__ __align__(8) uint64_t full_bar[C::kStages];
+  __shared__ __align__(8) uint64_t empty_bar[C::kStages];
+  __shared__ __align__(8) uint64_t tmem_full_bar[C::kAccStages];
+  __shared__ __align__(8) uint64_t tmem_empty_bar[C::kAccStages];
+  __shared__ uint32_t tmem_slot;
+  __shared__ int s_abort;
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < C::kStages; ++s) {
+      mbar_init(&full_bar[s], 1);
+      mbar_init(&empty_bar[s], 1);
+    }
+    for (int s = 0; s < C::kAccStages; ++s) {
+      mbar_init(&tmem_full_bar[s], 1);
+      mbar_init(&tmem_empty_bar[s], kEpiWarps);
+    }
+    s_abort = 0;
+    fence_barrier_init();
+    for (uint32_t c = 0; c < p.nclasses; ++c)
+      if (p.cls[c].ksteps) tma_prefetch_desc(&maps.a[c]);
+    tma_prefetch_desc(&maps.b);
+    if (p.ks_short) {
+      tma_prefetch_desc(&maps.as);
+      tma_prefetch_desc(&maps.bs);
+    }
+  }
+  if (warp == 1) tmem_alloc(&tmem_slot, C::kTmemCols);
+  pdl_trigger();
+  fence_before();
+  __syncthreads();
+  fence_after();
+  pdl_wait();   // everything above touched only shared / tensor memory and kernel parameters
+  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(&tmem_slot);
+  volatile int* abort_flag = &s_abort;
+
+  const uint32_t spb = kStageK / p.cb;   // tap-blocks per stage
+  const uint32_t a_block = kBlockM * p.cb, b_block = BN * p.cb;
+  const uint32_t ss_short = (p.ks_short + spb - 1) / spb;
+
+  if (warp == 0) {
+    if (lane == 0) {
+      uint32_t stage = 0, phase = 0;
+      bool ok = true;
+      for (uint32_t tile = blockIdx.x; tile < p.total_tiles && ok; tile += gridDim.x) {
+        const uint32_t ci = blk_class_of(p, tile);
+        const BlkClass& k = p.cls[ci];
+        const uint32_t ss_main = (k.ksteps + spb - 1) / spb, ss_sc = k.shortcut ? ss_short : 0u;
+        if (ss_main + ss_sc == 0) continue;
+        const uint32_t local = tile - k.tile0;
+        const uint32_t m_tile = local % k.m_tiles, n_tile = local / k.m_tiles;
+        const uint32_t m0 = m_tile * kBlockM;
+        const uint32_t img = fastdiv(m0, k.d_OHW), rem = m0 - img * k.OHW;
+        const uint32_t ohu = fastdiv(rem, k.d_OW);
+        const int base_w = k.lower_w + (int)(rem - ohu * k.OW), base_h = k.lower_h + (int)ohu;
+        uint32_t cc = 0, r = 0, s = 0;   // running decomposition of the main K-step into (channel chunk, tap)
+        for (uint32_t ks = 0; ks < ss_main + ss_sc && ok; ++ks) {
+          if (!(ok = mbar_wait(&empty_bar[stage], phase ^ 1, abort_flag, &g_conv_error))) break;
+          uint8_t* sa = smem + stage * C::kStageBytes;
+          uint8_t* sb = sa + C::kStageA;
+          if (ks < ss_main) {
+            const uint32_t k0 = ks * spb, nblk = min(spb, k.ksteps - k0);
+            mbar_expect_tx(&full_bar[stage], nblk * (a_block + b_block));
+            for (uint32_t j = 0; j < nblk; ++j) {
+              tma_load_im2col_4d(&maps.a[ci], &full_bar[stage], sa + j * a_block, (int)(cc * p.cb), base_w, base_h, (int)img,
+                                 (uint16_t)s, (uint16_t)r);
+              tma_load_2d(&maps.b, &full_bar[stage], sb + j * b_block, (int)(k.kcol + (k0 + j) * p.cb), (int)(n_tile * BN));
+              if (++cc == p.cchunks_g) {
+                cc = 0;
+                if (++s == k.kw) {
+                  s = 0;
+                  ++r;
+                }
+              }
+            }
+          } else {   // the shortcut: plain tiles of g_short's rows (the class's pixels in order) and of W_short
+            const uint32_t k0 = (ks - ss_main) * spb, nblk = min(spb, p.ks_short - k0);
+            mbar_expect_tx(&full_bar[stage], nblk * (a_block + b_block));
+            for (uint32_t j = 0; j < nblk; ++j) {
+              tma_load_2d(&maps.as, &full_bar[stage], sa + j * a_block, (int)((k0 + j) * p.cb), (int)m0);
+              tma_load_2d(&maps.bs, &full_bar[stage], sb + j * b_block, (int)((k0 + j) * p.cb), (int)(n_tile * BN));
+            }
+          }
+          if (++stage == C::kStages) {
+            stage = 0;
+            phase ^= 1;
+          }
+        }
+      }
+    }
+  } else if (warp == 1) {
+    if (lane == 0) {
+      uint32_t stage = 0, phase = 0, acc = 0, acc_phase = 0;
+      bool ok = true;
+      for (uint32_t tile = blockIdx.x; tile < p.total_tiles && ok; tile += gridDim.x) {
+        const BlkClass& k = p.cls[blk_class_of(p, tile)];
+        const uint32_t ss_main = (k.ksteps + spb - 1) / spb, ss_sc = k.shortcut ? ss_short : 0u;
+        if (ss_main + ss_sc == 0) continue;
+        if (!(ok = mbar_wait(&tmem_empty_bar[acc], acc_phase ^ 1, abort_flag, &g_conv_error))) break;
+        fence_after();
+        const uint32_t d_main = tmem_base + acc * C::kAccW;
+        for (uint32_t ks = 0; ks < ss_main + ss_sc; ++ks) {
+          if (!(ok = mbar_wait(&full_bar[stage], phase, abort_flag, &g_conv_error))) break;
+          fence_after();
+          const uint32_t sa = smem_u32(smem + stage * C::kStageBytes);
+          const uint32_t sb = sa + C::kStageA;
+          const bool sc = ks >= ss_main;
+          const uint32_t k0 = (sc ? ks - ss_main : ks) * spb;
+          const uint32_t nblk = min(spb, (sc ? p.ks_short : k.ksteps) - k0);
+          const uint32_t d = sc ? d_main + BN : d_main;
+          const uint32_t idesc = sc ? p.idesc_s : p.idesc;
+          const uint32_t per_block = p.cb / 32;
+          for (uint32_t j = 0; j < nblk; ++j)
+            for (uint32_t kk = 0; kk < per_block; ++kk) {
+              const uint32_t accumulate = (k0 + j > 0 || kk > 0) ? 1u : 0u;   // each accumulator starts at its first K-step
+              umma_i8(d, make_desc_kmajor(sa + j * a_block + kk * 32, (int)p.mode, 16),
+                      make_desc_kmajor(sb + j * b_block + kk * 32, (int)p.mode, 16), idesc, accumulate);
+            }
+          umma_commit(&empty_bar[stage]);
+          if (++stage == C::kStages) {
+            stage = 0;
+            phase ^= 1;
+          }
+        }
+        if (!ok) break;
+        umma_commit(&tmem_full_bar[acc]);
+        if (++acc == C::kAccStages) {
+          acc = 0;
+          acc_phase ^= 1;
+        }
+      }
+    }
+  } else {
+    const uint32_t quad = warp & 3;
+    const uint32_t half = (uint32_t)(warp - 2) >> 2;   // which of the quadrant's two warps: chunks half, half + 2, ...
+    const float scale = exp2i(p.exp_const + *p.ib_g + *p.ib_w);
+    const float scale_s = p.ks_short ? exp2i(p.exp_short + *p.ib_gs + *p.ib_ws) : 0.f;
+    uint32_t acc = 0, acc_phase = 0;
+    bool ok = true;
+    for (uint32_t tile = blockIdx.x; tile < p.total_tiles && ok; tile += gridDim.x) {
+      const BlkClass& k = p.cls[blk_class_of(p, tile)];
+      const bool has_m = k.ksteps != 0, has_s = k.shortcut && p.ks_short;   // warp-uniform
+      const bool has_acc = has_m || has_s;
+      const uint32_t local = tile - k.tile0;
+      const uint32_t m_tile = local % k.m_tiles, n_tile = local / k.m_tiles;
+      const uint32_t row = m_tile * kBlockM + quad * 32 + lane;
+      const uint32_t col0 = n_tile * BN;
+      if (has_acc) {
+        ok = mbar_wait(&tmem_full_bar[acc], acc_phase, abort_flag, &g_conv_error);
+        ok = __all_sync(0xffffffffu, ok);
+        if (!ok) break;
+        fence_after();
+      }
+      const uint32_t taddr = tmem_base + acc * C::kAccW + ((quad * 32u) << 16);
+      float* orow = nullptr;
+      if (row < k.M) {
+        const uint32_t img = fastdiv(row, k.d_OHW), rem = row - img * k.OHW;
+        const uint32_t oh = fastdiv(rem, k.d_OW), ow = rem - oh * k.OW;
+        orow = p.out + (k.out_off + (long long)img * p.rs_n + (long long)oh * p.rs_y + (long long)ow * p.rs_x) + col0;
+      }
+#pragma unroll 1
+      for (int c = 16 * (int)half; c < BN; c += 32) {
+        uint32_t v[16], w[16];
+        if (has_m) tmem_ld16(taddr + c, v);
+        if (has_s) tmem_ld16(taddr + BN + c, w);
+        if (has_acc) tmem_ld_wait();
+        if (orow && col0 + c < p.N) {   // N is a multiple of BN: whole 16-column chunks
+          float* o = orow + c;
+          float f[16];
+#pragma unroll
+          for (int j = 0; j < 16; ++j) f[j] = has_m ? __int2float_rn((int)v[j]) * scale : 0.f;
+          if (has_s) {
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+              const float fs = __int2float_rn((int)w[j]) * scale_s;
+              f[j] = has_m ? __fadd_rn(f[j], fs) : fs;
+            }
+          } else if (p.addend) {   // + an fp32 tensor of dX's shape (the other branch of a gradient sum)
+            const float4* ad = reinterpret_cast<const float4*>(p.addend + (o - p.out));
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              const float4 a4 = __ldcs(ad + j);
+              f[4 * j + 0] = has_m ? __fadd_rn(f[4 * j + 0], a4.x) : a4.x;
+              f[4 * j + 1] = has_m ? __fadd_rn(f[4 * j + 1], a4.y) : a4.y;
+              f[4 * j + 2] = has_m ? __fadd_rn(f[4 * j + 2], a4.z) : a4.z;
+              f[4 * j + 3] = has_m ? __fadd_rn(f[4 * j + 3], a4.w) : a4.w;
+            }
+          }
+#pragma unroll
+          for (int j = 0; j < 16; j += 4) *reinterpret_cast<float4*>(o + j) = make_float4(f[j], f[j + 1], f[j + 2], f[j + 3]);
+        }
+      }
+      if (has_acc) {
+        fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&tmem_empty_bar[acc]);
+        if (++acc == C::kAccStages) {
+          acc = 0;
+          acc_phase ^= 1;
+        }
+      }
+    }
+  }
+
+  fence_before();
+  __syncthreads();
+  fence_after();
+  if (warp == 1) tmem_dealloc(tmem_base, C::kTmemCols);
+}
+
+template <int BN>
+int launch_block(const BlkMaps& maps, const BlkParams& p, unsigned grid, cudaStream_t st) {
+  static bool attr_done[16] = {};
+  const int dev = device_info().device;
+  if (!attr_done[dev]) {
+    cudaError_t e = cudaFuncSetAttribute(conv_dgrad_block_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, BCfg<BN>::kSmemBytes);
+    if (e != cudaSuccess) {
+      set_cuda_error(e, "cudaFuncSetAttribute(conv_dgrad_block_kernel)");
+      return LBT_ECUDA;
+    }
+    attr_done[dev] = true;
+  }
+  launch_pdl(conv_dgrad_block_kernel<BN>, grid, kThreadsF, BCfg<BN>::kSmemBytes, st, maps, p);
+  return check_launch("lbt_conv_i8_dgrad_block");
+}
+
+}  // namespace
+}  // namespace lbt
+
+// Arguments are validated by lbt_conv_i8_dgrad_block (conv_dgrad.cu); this builds the class table and the tensor maps.
+int lbt::conv_dgrad_block_run(const void* g, int g_kind, int N, int OH, int OW, int Cout, const void* w2, int w_kind, size_t ldw, int Cin,
+                              int kh, int kw, int sh, int sw, int pad_top, int pad_left, int H, int W, const int32_t* ib_g,
+                              const int32_t* ib_w, int exp_const, const void* gs, int gs_kind, int Cout_s, const void* ws, int ws_kind,
+                              size_t ldws, const int32_t* ib_gs, const int32_t* ib_ws, int exp_short, float* dx, size_t ldc,
+                              const float* addend, void* stream) {
+  const uint32_t cb = Cout >= 128 ? 128u : (uint32_t)Cout;
+  uint32_t mode = 0;
+  while ((16u << mode) < cb) ++mode;
+  const int bn = Cin == 64 ? 64 : 128;
+  LBT_REQUIRE_ARCH();
+  const DeviceInfo& di = device_info();
+  static EncodeTiledFn enc_tiled = reinterpret_cast<EncodeTiledFn>(driver_fn("cuTensorMapEncodeTiled"));
+  static EncodeIm2colFn enc_im2col = reinterpret_cast<EncodeIm2colFn>(driver_fn("cuTensorMapEncodeIm2col"));
+  if (!enc_tiled || !enc_im2col) return LBT_ECUDA;
+
+  BlkParams p{};
+  BlkMaps maps;
+  memset(&maps, 0, sizeof(maps));
+  p.n_tiles = (uint32_t)Cin / bn;
+  p.N = (uint32_t)Cin;
+  p.cb = cb;
+  p.mode = mode;
+  p.cchunks_g = (uint32_t)Cout / cb;
+  p.ks_short = gs ? (uint32_t)Cout_s / cb : 0u;
+  p.ib_g = ib_g;
+  p.ib_w = ib_w;
+  p.ib_gs = ib_gs;
+  p.ib_ws = ib_ws;
+  p.exp_const = exp_const;
+  p.exp_short = exp_short;
+  p.addend = addend;
+  p.out = dx;
+  p.rs_n = (long long)H * W * (long long)ldc;
+  p.rs_y = (long long)sh * W * (long long)ldc;
+  p.rs_x = (long long)sw * (long long)ldc;
+  p.idesc = tc::make_idesc_i8(g_kind == LBT_MANT_S8, w_kind == LBT_MANT_S8, false, false, bn, kBlockM);
+  p.idesc_s = tc::make_idesc_i8(gs_kind == LBT_MANT_S8, ws_kind == LBT_MANT_S8, false, false, bn, kBlockM);
+
+  // classes with the most K-steps first (stable), each class's tiles together
+  struct Cls {
+    int a, b, work;
+  } order[kBlkMaxClasses];
+  int nc = 0;
+  for (int a = 0; a < sh && a < H; ++a)
+    for (int b = 0; b < sw && b < W; ++b) {
+      const int r0 = (a + pad_top) % sh, s0 = (b + pad_left) % sw;
+      const int work = class_count(r0, kh, sh) * class_count(s0, kw, sw) * (int)p.cchunks_g + (a == 0 && b == 0 ? (int)p.ks_short : 0);
+      int i = nc++;
+      while (i > 0 && order[i - 1].work < work) {
+        order[i] = order[i - 1];
+        --i;
+      }
+      order[i] = Cls{a, b, work};
+    }
+  p.nclasses = (uint32_t)nc;
+  uint32_t tile0 = 0;
+  for (int i = 0; i < nc; ++i) {
+    const int a = order[i].a, b = order[i].b;
+    const int Hc = (H - a + sh - 1) / sh, Wc = (W - b + sw - 1) / sw;
+    const int r0 = (a + pad_top) % sh, s0 = (b + pad_left) % sw;
+    const int nr = class_count(r0, kh, sh), ncol = class_count(s0, kw, sw);
+    BlkClass& k = p.cls[i];
+    k.M = (uint32_t)N * (uint32_t)(Hc * Wc);
+    k.OW = (uint32_t)Wc;
+    k.OHW = (uint32_t)(Hc * Wc);
+    k.d_OW = make_fastdiv(k.OW);
+    k.d_OHW = make_fastdiv(k.OHW);
+    k.shortcut = (a == 0 && b == 0 && gs) ? 1u : 0u;
+    k.m_tiles = (k.M + kBlockM - 1) / kBlockM;
+    k.tile0 = tile0;
+    tile0 += k.m_tiles * p.n_tiles;
+    k.out_off = ((long long)a * W + b) * (long long)ldc;
+    k.ksteps = (uint32_t)(nr * ncol) * p.cchunks_g;
+    if (!k.ksteps) continue;
+    const int pt2 = nr - 1 - (a + pad_top) / sh, pl2 = ncol - 1 - (b + pad_left) / sw;
+    k.lower_w = -pl2;
+    k.lower_h = -pt2;
+    k.kw = (uint32_t)ncol;
+    k.kcol = class_group_offset(r0, s0, kh, kw, sh, sw) * (uint32_t)Cout;
+    // the class's stride-1 sub-convolution of g: box of base pixels [lower, OW + upper) with exactly Wc (Hc) positions
+    cuuint64_t gdim[4] = {(cuuint64_t)Cout, (cuuint64_t)OW, (cuuint64_t)OH, (cuuint64_t)N};
+    cuuint64_t gstr[3] = {(cuuint64_t)Cout, (cuuint64_t)OW * Cout, (cuuint64_t)OH * OW * Cout};
+    int lower[2] = {-pl2, -pt2};
+    int upper[2] = {Wc - OW - pl2, Hc - OH - pt2};
+    cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = enc_im2col(&maps.a[i], CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, const_cast<void*>(g), gdim, gstr, lower, upper, cb, kBlockM,
+                            estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_of(mode), CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+      set_cuda_error(cudaErrorInvalidValue, "cuTensorMapEncodeIm2col(block dgrad)");
+      return LBT_ECUDA;
+    }
+  }
+  p.total_tiles = tile0;
+  auto tiled = [&](CUtensorMap* m, const void* base, uint64_t inner, uint64_t outer, uint64_t pitch, uint32_t rows,
+                   CUtensorMapL2promotion l2, const char* what) {
+    cuuint64_t gdim[2] = {(cuuint64_t)inner, (cuuint64_t)outer};
+    cuuint64_t gstr[1] = {(cuuint64_t)pitch};
+    cuuint32_t box[2] = {cb, rows};
+    cuuint32_t estr[2] = {1, 1};
+    if (enc_tiled(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  swizzle_of(mode), l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) {
+      set_cuda_error(cudaErrorInvalidValue, what);
+      return false;
+    }
+    return true;
+  };
+  if (!tiled(&maps.b, w2, (uint64_t)kh * kw * Cout, (uint64_t)Cin, ldw, (uint32_t)bn, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+             "cuTensorMapEncodeTiled(block dgrad weights)"))
+    return LBT_ECUDA;
+  if (gs) {
+    const uint64_t rows_s = (uint64_t)N * ((H + sh - 1) / sh) * ((W + sw - 1) / sw);
+    if (!tiled(&maps.as, gs, (uint64_t)Cout_s, rows_s, (uint64_t)Cout_s, (uint32_t)kBlockM, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+               "cuTensorMapEncodeTiled(block dgrad shortcut gradient)") ||
+        !tiled(&maps.bs, ws, (uint64_t)Cout_s, (uint64_t)Cin, ldws, (uint32_t)bn, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+               "cuTensorMapEncodeTiled(block dgrad shortcut weights)"))
+      return LBT_ECUDA;
+  }
+  const uint64_t cap = (uint64_t)di.sm_count * BCfg<64>::kCtasPerSm;
+  const unsigned grid = (unsigned)(p.total_tiles < cap ? p.total_tiles : cap);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  return bn == 64 ? launch_block<64>(maps, p, grid, st) : launch_block<128>(maps, p, grid, st);
 }
 
 extern "C" int lbt_conv_debug_error(void) {

@@ -41,6 +41,13 @@ int conv_fprop_run(const void* src, int src_kind, int N, int H, int W, int C, co
                    int exp_const, const float* bias, float* out, size_t ldc, const lbt_qsite* q_out, int8_t* k_out, int64_t* sums,
                    const float* addend, void* stream, const OutRemap* remap, const void* src_lo = nullptr);   // src_lo: see conv_halo_run
 
+// conv_i8.cu: lbt_conv_i8_dgrad_block's launch (arguments already validated by the entry point in conv_dgrad.cu)
+int conv_dgrad_block_run(const void* g, int g_kind, int N, int OH, int OW, int Cout, const void* w2, int w_kind, size_t ldw, int Cin,
+                         int kh, int kw, int sh, int sw, int pad_top, int pad_left, int H, int W, const int32_t* ib_g,
+                         const int32_t* ib_w, int exp_const, const void* gs, int gs_kind, int Cout_s, const void* ws, int ws_kind,
+                         size_t ldws, const int32_t* ib_gs, const int32_t* ib_ws, int exp_short, float* dx, size_t ldc,
+                         const float* addend, void* stream);
+
 bool conv_wgrad_ldg_ok(int C, int Cout, int kh, int kw);
 int conv_wgrad_ldg_run(const void* src, int src_kind, int N, int H, int W, int C, const void* g, int g_kind, int Cout, int kh, int kw,
                        int sh, int sw, int pt, int pl, int OH, int OW, int64_t* acc64, int alpha, void* stream);

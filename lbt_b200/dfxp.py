@@ -709,10 +709,12 @@ def _conv_fprop(layer, geom, xm, xkind, prep, wm, bq, out2d, bnq=None):
         G.gemm_i8(A, wt, ibA=ibx, ibB=ibw, exp_const=e, bias=bq, out=out2d, bnq=gbnq)
 
 
-def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_db, addend=None, link=None):
+def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_db, addend=None, link=None, shortcut=None):
     """dfxp:302-305 from the quantised gradient mantissas gm [N, OH, OW, Cout] (s8): (dX NHWC fp32, dW, db).
     ``addend`` (NHWC fp32, the shape of dX): the gradient reaching the same input along another branch (residual
-    shortcut), added in the dgrad epilogue instead of by a separate pass over the tensor."""
+    shortcut), added in the dgrad epilogue instead of by a separate pass over the tensor.  ``shortcut``: a strided block's
+    1x1 shortcut parked by _BlockDgrad (only with the parity-class path, see _block_dgrad_ok): its input gradient is computed
+    in the same launch as this one (lbt_conv_i8_dgrad_block), or first on its own and then added as ``addend``."""
     N, H, W, Cin, Cout, kh, kw, sh, sw, pt, pl, OH, OW = geom
     xb, wb, gb = layer.qX.bits, layer.qW.bits, layer.qG.bits
     dev = gm.device
@@ -830,11 +832,16 @@ def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_
             else:
                 perm = torch.tensor(_class_perm(kh, kw, sh, sw), device=dev)
                 w2 = _as_operand(wm.view(kh * kw, Cin, Cout).index_select(0, perm).permute(1, 0, 2).reshape(Cin, K2))
-            _lib.call('lbt_conv_i8_dgrad_strided', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2),
-                      Q.MANT_S8 | (_W_PREPARED if pw2 is not None else 0), w2.stride(0),
-                      Cin, kh, kw, sh, sw, pt, pl, H, W, _lib.ptr(layer.qG.range), _lib.ptr(layer.qW.range), int(e),
-                      _lib.ptr(dx), Cin, _lib.ptr(ad2), _lib.stream(),
-                      meta=dict(ops=2 * N * OH * OW * Cin * K2, bytes=N * OH * OW * Cout * min(sh * sw, kh * kw) + Cin * K2 + N * H * W * Cin * 4))
+            done = shortcut is not None and addend is None and _dgrad_block(layer, geom, gm, w2, pw2 is not None, e, dx, shortcut)
+            if not done:
+                if shortcut is not None:      # the kernel declined the shapes: the shortcut's dgrad first, then this one adds it
+                    ad2 = _shortcut_dgrad(shortcut).reshape(N * H * W, Cin)
+                _lib.call('lbt_conv_i8_dgrad_strided', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2),
+                          Q.MANT_S8 | (_W_PREPARED if pw2 is not None else 0), w2.stride(0),
+                          Cin, kh, kw, sh, sw, pt, pl, H, W, _lib.ptr(layer.qG.range), _lib.ptr(layer.qW.range), int(e),
+                          _lib.ptr(dx), Cin, _lib.ptr(ad2), _lib.stream(),
+                          meta=dict(ops=2 * N * OH * OW * Cin * K2,
+                                    bytes=N * OH * OW * Cout * min(sh * sw, kh * kw) + Cin * K2 + N * H * W * Cin * 4))
         else:
             w2 = pw2 if pw2 is not None else _as_operand(wm.view(kh * kw, Cin, Cout).permute(1, 0, 2).reshape(Cin, K2))
             A2 = _im2col(gm, Q.MANT_S8, H, W, kh, kw, sh, sw, pt, pl, True)
@@ -847,6 +854,69 @@ def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_
             t.record_stream(side)
         rt._side_pending = True
     return dx, dW, db
+
+
+FUSE_BLOCK_DGRAD = os.environ.get('LBT_FUSE_BLOCK_DGRAD', '1') != '0'   # module switch: a downsampling block's input gradient (every
+                      # parity class of its strided convolution and its 1x1 shortcut) in one launch, lbt_conv_i8_dgrad_block
+_block_dgrad_count = 0   # lbt_conv_i8_dgrad_block launches (tests)
+
+
+class _BlockDgrad:
+    """Backward hand-off between the two units of a downsampling block that read the same input: the first unit of the residual
+    branch (a strided convolution, which hands its input to the shortcut as an alias) and the 1x1 shortcut unit.  The shortcut
+    unit runs its batch-norm backward and weight gradient as usual, then parks its gradient mantissas here and returns a shape
+    carrier for dX; the alias returns it to the first unit, whose input-gradient launch then writes the sum of both branches
+    (lbt_conv_i8_dgrad_block).  The fp32 shortcut gradient is never written."""
+
+    def __init__(self):
+        self.armed = False     # the first unit hands its input to the shortcut through the alias (set in its forward)
+        self.parked = None     # (layer, geom, xkind, wm, prep, gm) of the shortcut
+
+    def take(self):
+        p, self.parked = self.parked, None
+        return p
+
+
+def _block_dgrad_ok(layer, geom, prep):
+    """The first unit's input gradient takes the parity-class path, where lbt_conv_i8_dgrad_block applies."""
+    N, H, W, Cin, Cout, kh, kw, sh, sw, pt, pl, OH, OW = geom
+    if (sh, sw) == (1, 1) or layer.qG.bits > 8:
+        return False
+    if layer.implicit and _gather_ok(Cout, Cin, kh, kw) and sh <= 4 and sw <= 4:
+        return False
+    return bool(prep['classes'] if prep is not None else _dgrad_classes_ok(layer, Cin, Cout, kh, kw, sh, sw))
+
+
+def _shortcut_dgrad(parked):
+    """The parked shortcut's input gradient on its own (NHWC fp32), as its unit would have computed it."""
+    layer, geom, xkind, wm, prep, gm = parked
+    dx, _, _ = _conv_backward(layer, geom, None, xkind, wm, prep, gm, True, False, False)
+    return dx
+
+
+def _dgrad_block(layer, geom, gm, w2, w_prepared, e, dx, shortcut):
+    """lbt_conv_i8_dgrad_block: dx = this strided convolution's input gradient + the parked shortcut's, in one launch.
+    False when the kernel does not take the shapes (the caller then runs the two launches)."""
+    global _block_dgrad_count
+    N, H, W, Cin, Cout, kh, kw, sh, sw, pt, pl, OH, OW = geom
+    sl, sgeom, _, swm, sprep, sgm = shortcut
+    sN, sH, sW, sCin, sCout, skh, skw, ssh, ssw, spt, spl, sOH, sOW = sgeom
+    if (sN, sH, sW, sCin) != (N, H, W, Cin) or (skh, skw, ssh, ssw, spt, spl) != (1, 1, sh, sw, 0, 0):
+        return False
+    spw2 = sprep['w2'] if sprep is not None else None
+    sw2 = spw2 if spw2 is not None else _as_operand(swm.view(Cin, sCout))
+    se = -(sl.qG.bits - 1) - (sl.qW.bits - 1)
+    K2 = kh * kw * Cout
+    done = _lib.try_call('lbt_conv_i8_dgrad_block', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2),
+                         Q.MANT_S8 | (_W_PREPARED if w_prepared else 0), w2.stride(0), Cin, kh, kw, sh, sw, pt, pl, H, W,
+                         _lib.ptr(layer.qG.range), _lib.ptr(layer.qW.range), int(e), _lib.ptr(sgm), Q.MANT_S8, sOH, sOW, sCout,
+                         _lib.ptr(sw2), Q.MANT_S8 | (_W_PREPARED if spw2 is not None else 0), sw2.stride(0),
+                         _lib.ptr(sl.qG.range), _lib.ptr(sl.qW.range), int(se), _lib.ptr(dx), Cin, None, _lib.stream(),
+                         meta=dict(ops=2 * N * OH * OW * Cin * K2 + 2 * N * sOH * sOW * Cin * sCout,
+                                   bytes=N * OH * OW * Cout + N * sOH * sOW * sCout + Cin * (K2 + sCout) + N * H * W * Cin * 4))
+    if done:
+        _block_dgrad_count += 1
+    return done
 
 
 def _check_layer_bits(who, bits, grad_bits):
@@ -1486,7 +1556,7 @@ class _ConvBNFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight, gamma, beta, add, conv, bn, relu, next_site, next_kind, want_fp32, alias, link_in, link_out, pool=None,
-                next2=None, running=False):
+                next2=None, running=False, block=None):
         # running: eval mode without an autograd graph (BatchNorm2d_q._running): the BN kernels normalise with the running
         # statistics, nothing is saved for backward
         geom = _conv_geom(conv, x, weight)
@@ -1541,6 +1611,15 @@ class _ConvBNFn(torch.autograd.Function):
         ctx.conv, ctx.bn, ctx.geom, ctx.xkind, ctx.prep = conv, bn, geom, xkind, prep
         ctx.relu_mode, ctx.has_add = relu_mode, add is not None
         ctx.link_in, ctx.link_out = link_in, link_out
+        # block: the downsampling block's _BlockDgrad; the unit with the alias is the first unit, the other one the shortcut
+        ctx.block = None
+        if block is not None and not running:
+            if alias:       # only where the first unit's input gradient takes the parity-class path the kernel runs on
+                block.armed = conv.qG.bits <= 8 and _block_dgrad_ok(conv, geom, prep)
+                ctx.block = block if block.armed else None
+            elif block.armed:
+                ctx.block = block
+        ctx.block_first = bool(alias)
         if link_out is not None and out is None and not running:     # the next unit may run this BN's backward pass 1 in its dgrad epilogue
             link_out.offer(bn, k1, k2, gq, bq, relu_mode, add is not None)
         ctx.pool = None
@@ -1589,15 +1668,36 @@ class _ConvBNFn(torch.autograd.Function):
         _, gm, dgamma, dbeta, d_add = _bn_backward(ctx.bn, _to_mem(g) if pre is None else None, k1, k2, sums, gq, bq, out,
                                                    ctx.relu_mode, ctx.has_add, grad_site=conv.qG, want_dx=False, pre=pre,
                                                    pool=pool)   # ... dfxp:300
-        addend = _to_mem(g_alias) if (g_alias is not None and need_dx) else None
-        li = ctx.link_in if (addend is None and FUSE_BWD_LINK) else None
+        bd = ctx.block
+        if bd is not None and not ctx.block_first:
+            ctx.block = None
+            if need_dx and not isinstance(gm, tuple):
+                # the shortcut of a downsampling block: weight gradient only; the first unit's dgrad launch adds this branch
+                _, dW, _ = _conv_backward(conv, ctx.geom, xm, ctx.xkind, wm, ctx.prep, gm, False, need_dw, False)
+                bd.parked = (conv, ctx.geom, ctx.xkind, wm, ctx.prep, gm)
+                N, H, W, Cin = ctx.geom[:4]
+                dx = torch.empty(1, dtype=torch.float32, device=gm.device).expand(N, H, W, Cin)     # shape carrier only
+                return ((_from_mem(dx),) + (dW, dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None)) + (None,) * 13)
+        parked = bd.take() if (bd is not None and need_dx) else None
+        shortcut = None
+        if parked is not None:     # g_alias is the shortcut unit's shape carrier
+            if not isinstance(gm, tuple) and _block_dgrad_ok(conv, ctx.geom, ctx.prep):
+                shortcut = parked
+                addend = None
+            else:
+                addend = _shortcut_dgrad(parked)
+        else:
+            addend = _to_mem(g_alias) if (g_alias is not None and need_dx) else None
+        ctx.block = None
+        li = ctx.link_in if (addend is None and shortcut is None and FUSE_BWD_LINK) else None
         if isinstance(gm, tuple):        # 9..16-bit gradient: (hi, lo) byte planes
             dx, dW, _ = _conv_backward16(conv, ctx.geom, xm, ctx.xkind, wm, ctx.prep, gm[0], gm[1], need_dx, need_dw, False, addend=addend)
         else:
-            dx, dW, _ = _conv_backward(conv, ctx.geom, xm, ctx.xkind, wm, ctx.prep, gm, need_dx, need_dw, False, addend=addend, link=li)
+            dx, dW, _ = _conv_backward(conv, ctx.geom, xm, ctx.xkind, wm, ctx.prep, gm, need_dx, need_dw, False, addend=addend, link=li,
+                                       shortcut=shortcut)
         return ((_from_mem(dx) if dx is not None else None), dW, dgamma, dbeta,
                 (_from_mem(d_add) if d_add is not None else None), None, None, None, None, None, None, None, None, None, None, None,
-                None)
+                None, None)
 
 
 FUSE_POOL = os.environ.get('LBT_FUSE_POOL', '0') == '1'   # module switch: a MaxPool_q right behind a fused unit runs its backward inside the
@@ -1622,7 +1722,7 @@ def _unit_fusable(conv, bn, x, running=False):
 
 
 def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=True, alias=False, link_in=None, link_out=None,
-                 pool=None):
+                 pool=None, block=None):
     """``bn(conv(x), add=add, relu=relu)`` as ONE fused unit when the shapes allow (else exactly that expression).
 
     next_conv: the Conv2d_q that consumes the result — its input quantiser then runs inside this unit's last kernel
@@ -1667,10 +1767,14 @@ def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=Tr
         want_fp32 = True
     # measured: folding pays while the dgrad output is narrow (ResNet-18/20 blocks: -1.6 % step time); for the 256..2048-
     # channel block inputs of ResNet-50 the epilogue-bound 1x1 dgrad GEMMs lose more than the coalesced add costs (+3 %)
-    use_alias = bool(alias and x.requires_grad and not getattr(x, '_lbt_hollow', False) and conv.weight.shape[2] <= 128)
+    # block (a downsampling block's _BlockDgrad): the shortcut's gradient joins inside the first unit's input-gradient launch,
+    # so the alias pays at every width
+    block = block if (FUSE_BLOCK_DGRAD and not running) else None
+    use_alias = bool(alias and x.requires_grad and not getattr(x, '_lbt_hollow', False) and
+                     (conv.weight.shape[2] <= 128 or (block is not None and tuple(conv.stride) != (1, 1) and conv.qG.bits <= 8)))
     out, nm, xa = _ConvBNFn.apply(x, conv.weight, bn[1].gamma, bn[1].beta, add, conv, bn, relu, next_site, next_kind,
                                   want_fp32, use_alias, link_in if FUSE_BWD_LINK else None, link_out if FUSE_BWD_LINK else None,
-                                  pgeom, next2, running)
+                                  pgeom, next2, running, block)
     if next_site is not None and nm.numel():       # (empty: the pooled one-kernel path declined, the consumer quantises itself)
         out._lbt_q = {id(next_site): (nm, next_kind)}
         if next2 is not None and next2[2] is not None:
@@ -2100,14 +2204,16 @@ class ResidualBlock_q(nn.Module):
             # consecutive units of the residual branch are linked: the later unit's input-gradient kernel runs the earlier
             # unit's BN backward pass 1 in its epilogue (_BwdLink)
             link = _BwdLink()
-            r, xs = conv_bn_unit(res[0], res[1], x, next_conv=res[2], want_fp32=False, alias=True, link_out=link)
+            # a strided first unit and a 1x1 shortcut unit: one launch for the block's input gradient (_BlockDgrad)
+            bd = _BlockDgrad() if len(sc_layers) == 2 and tuple(res[0].stride) != (1, 1) else None
+            r, xs = conv_bn_unit(res[0], res[1], x, next_conv=res[2], want_fp32=False, alias=True, link_out=link, block=bd)
             if xs is not x and getattr(x, '_lbt_q', None) is not None:
                 xs._lbt_q = x._lbt_q       # mantissas made for the shortcut convolution's quantiser travel with the alias
             for i in range(2, len(res) - 2, 2):
                 nxt = _BwdLink()
                 r = conv_bn_unit(res[i], res[i + 1], r, next_conv=res[i + 2], want_fp32=False, link_in=link, link_out=nxt)
                 link = nxt
-            sc = conv_bn_unit(sc_layers[0], sc_layers[1], xs) if len(sc_layers) == 2 else self.shortcut(xs)
+            sc = conv_bn_unit(sc_layers[0], sc_layers[1], xs, block=bd) if len(sc_layers) == 2 else self.shortcut(xs)
             return conv_bn_unit(res[-2], res[-1], r, add=sc, relu=True, next_conv=next_conv, link_in=link)
         r = x
         for m in res[:-1]:
