@@ -161,8 +161,10 @@ enum lbt_gemm_epilogue {
  *         a_kind/b_kind = LBT_MANT_S8 or LBT_MANT_U8.
  *   LBT_EPI_F32: the value of a mantissa with `bits` total bits is k * 2^-(bits-1-ib), so pass
  *         exp_const = -(bitsA-1) - (bitsB-1) and the two device range pointers (either may be NULL = 0).
- *         Result == RN_fp32(exact_dot * 2^e) bit for bit.  K <= 65536.
- *   LBT_EPI_ACC64: K is cut into k_splits chunks (each <= 65536) spread over the SMs; partial sums are
+ *         Result == RN_fp32(exact_dot * 2^e) bit for bit.  K <= 65536, or 32768 when both operands are unsigned
+ *         (LBT_EUNSUPPORTED above).
+ *   LBT_EPI_ACC64: K is cut into k_splits chunks (each <= 65536, or 32768 when both operands are unsigned; more
+ *         chunks than k_splits if needed) spread over the SMs; partial sums are
  *         added to acc64 (caller zeroes it) scaled by the integer alpha.  Finish with lbt_acc64_finalize.
  *   q_out != NULL (LBT_EPI_F32 only, N % 4 == 0): the fused re-quantising epilogue.  Instead of storing the
  *         fp32 result v, the kernel stores k_out[m*N + n] = Q_site(v) (s8, stochastic) and adds the exact
@@ -185,7 +187,8 @@ int lbt_gemm_i8(const void* A, int a_kind, size_t lda, const void* B, int b_kind
  * The input-gradient GEMM of dfxp:305 / :460 with a gradient quantiser wider than 8 bits (BASELINE config 5, 16-bit G): both
  * halves are staged per K block beside ONE copy of B, two s32 accumulators per tile live in tensor memory and the epilogue
  * combines them in 64-bit integers before the single rounding — no int64 accumulator in HBM, no second pass over B.
- * K <= 65536; N tiles of at most 128 columns (two accumulator pairs fill the 512 tensor-memory columns).
+ * K <= 65536, or 32768 when B is unsigned (A_lo x B is then u8 x u8); N tiles of at most 128 columns (two accumulator pairs
+ * fill the 512 tensor-memory columns).
  */
 int lbt_gemm_i8_dual(const int8_t* A_hi, const uint8_t* A_lo, size_t lda, const void* B, int b_kind, size_t ldb, size_t M,
                      size_t N, size_t K, const int32_t* ibA, const int32_t* ibB, int exp_const, float* out_f32, size_t ldc,
@@ -222,7 +225,8 @@ int lbt_im2col_i8(const void* src, int src_kind, int N, int H, int W, int C, int
  *   resident in shared memory (the TMA engine retires only one pixel row per ~3 clocks per SM).
  *   src[N,H,W,C] s8|u8, C in {16, 32, 64} or a multiple of 128;  wp[Cout, kh*kw*C] packed K-major
  *   (k = (r*kw + s)*C + c, row pitch ldw bytes);  out[N*OH*OW, Cout] fp32 (row pitch ldc floats):
- *   out = fp32(acc) * 2^(exp_const + *ib_src + *ib_w) (+ bias[co]).  kh*kw*C <= 65536.
+ *   out = fp32(acc) * 2^(exp_const + *ib_src + *ib_w) (+ bias[co]).  kh*kw*C <= 65536, or 32768 when both operands are
+ *   unsigned.
  *   q_out != NULL (Cout % 4 == 0): fused re-quantising epilogue as in lbt_gemm_i8 — k_out[N*OH*OW, Cout] s8,
  *   sums[2*Cout], rows_per_image = OH*OW; `out` may then be NULL.  addend: as in lbt_gemm_i8 (fp32 [M, ldc]).
  */
@@ -240,6 +244,7 @@ int lbt_conv_i8_fprop(const void* src, int src_kind, int N, int H, int W, int C,
  * input gradient tf.gradients(y, X, gradq) (dynamic_fixed_point.py:305).  The TMA halo kernel (two patches per ring slot) where
  * its filter bank fits beside them (C == 64), the im2col-TMA kernel (both planes' blocks per ring slot) for C >= 64 otherwise;
  * LBT_EUNSUPPORTED for narrower sources or Cout < 64: lbt_im2col_i8 + lbt_gemm_i8_dual.  e = exp_const + *ib_src + *ib_w.
+ * kh*kw*C <= 65536, or 32768 with an unsigned filter (lo * W is then u8 x u8).
  */
 int lbt_conv_i8_fprop_dual(const int8_t* src_hi, const uint8_t* src_lo, int N, int H, int W, int C, const void* wp, int w_kind,
                            size_t ldw, int Cout, int kh, int kw, int pad_top, int pad_left, int OH, int OW,
@@ -262,7 +267,8 @@ int lbt_conv_i8_dgrad(const void* g, int g_kind, int N, int OH, int OW, int Cout
  * Implicit-GEMM weight gradient: acc64[(r*kw+s)*C + c, co] += alpha * sum over output pixels m of
  * src[pixel(m) + (r,s), c] * g[m, co] — tf.gradients(y, W, gradq) (dynamic_fixed_point.py:207, 302) in HWIO
  * order, exact.  Both operands are consumed MN-major straight from TMA loads (no transposes); the pixel
- * dimension is split over the SMs (k_splits, 0 = auto; each CTA sums <= 65536 pixels in s32) and reduced
+ * dimension is split over the SMs (k_splits, 0 = auto; each CTA sums <= 65536 pixels in s32, or 32768 when both operands
+ * are unsigned, which may add splits) and reduced
  * with 64-bit atomics.  src[N,H,W,C] and g[N*OH*OW, Cout] are s8|u8 with C, Cout in {16,32,64} or
  * multiples of 128.  Caller zeroes acc64[kh*kw*C, Cout]; finish with lbt_acc64_finalize.
  */
@@ -678,7 +684,8 @@ int lbt_conv_i8_dgrad_bn(const void* g, int g_kind, int N, int H, int W, int C, 
  * with its taps in PARITY-CLASS ORDER (lbt_param_prep with rot180 = 2: taps grouped by (r mod sh, s mod sw), groups in
  * row-major order, reversed (r / sh, s / sw) order inside a group).  Classes no tap reaches get `addend` (or zeros).
  * dX = RN_fp32(exact * 2^(*ib_g + *ib_w + exp_const)) (+ addend), bit-identical to the im2col + GEMM formulation.
- * Cout % 16 == 0 (and a multiple of 128 above 64), Cin % 4 == 0, strides <= 4.
+ * Cout % 16 == 0 (and a multiple of 128 above 64), Cin % 4 == 0, strides <= 4.  Each class sums at most 65536 products per
+ * accumulator (sub-filter taps * Cout), or 32768 when both operands are unsigned.
  */
 int lbt_conv_i8_dgrad_strided(const void* g, int g_kind, int N, int OH, int OW, int Cout, const void* w2, int w_kind, size_t ldw,
                               int Cin, int kh, int kw, int sh, int sw, int pad_top, int pad_left, int H, int W,
@@ -695,7 +702,8 @@ int lbt_conv_i8_dgrad_strided(const void* g, int g_kind, int N, int OH, int OW, 
  * bit-identical to lbt_conv_i8_dgrad_strided on the shortcut followed by lbt_conv_i8_dgrad_strided on the main convolution
  * with that result as addend.  addend (the layout of dX) only without a shortcut.  Null pointers, bad kinds or shapes:
  * LBT_EINVAL; Cin % 4 != 0, strides > 2, Cin neither 64 nor a multiple of 128, Cout (Cout_s) not 32, 64 or a multiple of 128
- * (with the same channel chunk), misalignment, a shortcut lattice that does not match or a shortcut together with addend:
+ * (with the same channel chunk), kh*kw*Cout or Cout_s above 65536 (32768 when both operands of that term are unsigned),
+ * misalignment, a shortcut lattice that does not match or a shortcut together with addend:
  * LBT_EUNSUPPORTED — all before any CUDA call.  Run the two lbt_conv_i8_dgrad_strided calls then.
  */
 int lbt_conv_i8_dgrad_block(const void* g, int g_kind, int N, int OH, int OW, int Cout, const void* w2, int w_kind, size_t ldw,

@@ -78,6 +78,12 @@ inline FastDiv make_fastdiv(uint32_t d) {
   return f;
 }
 
+// Most products one s32 accumulator may sum exactly for operand kinds a, b (LBT_MANT_*): |s8*s8| <= 2^14 and |u8*s8| <= 255*128,
+// so 65536 of them stay below 2^31; |u8*u8| <= 255^2 allows only 32768 (2^15 * 65025 < 2^31 - 1 < 2^16 * 65025).
+inline uint32_t max_products(int a_kind, int b_kind) {
+  return (a_kind == LBT_MANT_U8 && b_kind == LBT_MANT_U8) ? 32768u : 65536u;
+}
+
 #define LBT_REQUIRE_ARCH()                        \
   do {                                            \
     const ::lbt::DeviceInfo& _di = ::lbt::device_info(); \

@@ -125,8 +125,10 @@ extern "C" int lbt_conv_i8_dgrad_block(const void* g, int g_kind, int N, int OH,
   const int cb = Cout >= 128 ? 128 : Cout;
   if (Cin % 4) return LBT_EUNSUPPORTED;
   if (sh > 2 || sw > 2 || (cb != 32 && cb != 64 && cb != 128) || Cout % cb || (Cin != 64 && Cin % 128)) return LBT_EUNSUPPORTED;
-  if (g_short && (Cout_s % cb || Cout_s > 65536 || (Cout_s >= 128 ? 128 : Cout_s) != cb)) return LBT_EUNSUPPORTED;
-  if ((size_t)kh * kw * Cout > 65536 || kh > 255 || kw > 255) return LBT_EUNSUPPORTED;   // exactness bound of one s32 accumulator
+  // exactness bound of one s32 accumulator, for the main term and for the shortcut's
+  if (g_short && (Cout_s % cb || (uint32_t)Cout_s > max_products(gs_kind, ws_kind) || (Cout_s >= 128 ? 128 : Cout_s) != cb))
+    return LBT_EUNSUPPORTED;
+  if ((size_t)kh * kw * Cout > max_products(g_kind, w_kind) || kh > 255 || kw > 255) return LBT_EUNSUPPORTED;
   if ((size_t)N * H * W >= (1ull << 31)) return LBT_EUNSUPPORTED;
   if ((reinterpret_cast<uintptr_t>(g) & 15) || (reinterpret_cast<uintptr_t>(w2) & 15) || (ldw & 15) || (ldc & 3) ||
       (reinterpret_cast<uintptr_t>(dx) & 15) || (addend && (reinterpret_cast<uintptr_t>(addend) & 15)) ||

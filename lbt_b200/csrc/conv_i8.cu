@@ -691,7 +691,8 @@ int lbt::conv_fprop_run(const void* src, int src_kind, int N, int H, int W, int 
                                  exp_const, bias, out, ldc, q_out, k_out, sums, addend, stream, remap, src_lo);
     if (!(dual && rc == LBT_EUNSUPPORTED)) return rc;   // two planes: the filter bank + two patches may not fit; im2col-TMA kernel below
   }
-  if (Ktot > 65536) return LBT_EUNSUPPORTED;  // exactness bound of one s32 accumulator
+  // exactness bound of one s32 accumulator (two planes: the low plane is u8, so a u8 filter makes it u8 x u8)
+  if (Ktot > max_products(dual ? LBT_MANT_U8 : src_kind, w_kind)) return LBT_EUNSUPPORTED;
   if (kh > 255 || kw > 255) return LBT_EUNSUPPORTED;
   LBT_REQUIRE_ARCH();
   const DeviceInfo& di = device_info();
@@ -899,7 +900,9 @@ static int conv_wgrad_run(const void* src, int src_kind, int N, int H, int W, in
   }
   if (splits > p.pix_blocks) splits = p.pix_blocks;
   p.blocks_per_split = (p.pix_blocks + splits - 1) / splits;
-  if (p.blocks_per_split > 65536 / kBlockM) p.blocks_per_split = 65536 / kBlockM;  // s32 exactness bound per CTA
+  // s32 exactness bound per CTA; two planes: the low one is u8, so a u8 source makes it u8 x u8
+  const uint32_t max_blocks = max_products(src_kind, dual ? LBT_MANT_U8 : g_kind) / kBlockM;
+  if (p.blocks_per_split > max_blocks) p.blocks_per_split = max_blocks;
   p.k_splits = (p.pix_blocks + p.blocks_per_split - 1) / p.blocks_per_split;
   p.Kf = (uint32_t)(kh * kw * C);
   p.acc64 = reinterpret_cast<long long*>(acc64);

@@ -908,8 +908,8 @@ int conv_wgrad_ldg_run(const void* src, int src_kind, int N, int H, int W, int C
   const size_t smem = (size_t)nst * p.stage_bytes + 256;
   const uint64_t cap = (uint64_t)di.sm_count * (two ? 2u : 1u);
   unsigned grid = (unsigned)(p.pix_blocks < cap ? p.pix_blocks : cap);
-  // one CTA may sum at most 65536 products per s32 accumulator: 512 pixel blocks
-  if ((p.pix_blocks + grid - 1) / grid > 512) return LBT_EUNSUPPORTED;
+  // one CTA may sum at most max_products(src_kind, g_kind) products per s32 accumulator: 512 pixel blocks, 256 for u8 x u8
+  if ((p.pix_blocks + grid - 1) / grid > max_products(src_kind, g_kind) / kBlockM) return LBT_EUNSUPPORTED;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   switch (p.cpp) {
     case 1: return launch_wgrad_ldg<1>(p, grid, smem, st);

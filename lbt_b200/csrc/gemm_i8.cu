@@ -15,7 +15,7 @@
 // Epilogues:
 //   LBT_EPI_F32   out[m, n] = fp32(acc) * 2^e (+ bias[n])            (fprop / dgrad / dense)
 //   LBT_EPI_ACC64 acc64[m, n] += alpha * acc   (64-bit atomics)       (wgrad split-K: order-independent,
-//                 bit-reproducible; per-split K <= 65536 keeps the s32 partial exact, SURVEY.md H3)
+//                 bit-reproducible; per-split K <= 65536, or 32768 for u8 x u8, keeps the s32 partial exact, SURVEY.md H3)
 #include <cuda.h>
 
 #include "qsite.cuh"
@@ -832,8 +832,8 @@ extern "C" int lbt_gemm_i8(const void* A, int a_kind, size_t lda, const void* B,
   if (epilogue == LBT_EPI_F32) splits = 1;
   if (splits > p.k_blocks) splits = p.k_blocks;
   p.k_blocks_per_split = (p.k_blocks + splits - 1) / splits;
-  // s32 accumulator: |u8*s8| <= 255*128, so one CTA may sum at most 65536 products exactly
-  const uint32_t max_kb = 65536 / kBlockK;
+  // s32 accumulator: one CTA may sum at most max_products(a_kind, b_kind) products exactly (32768 for u8 x u8)
+  const uint32_t max_kb = max_products(a_kind, b_kind) / kBlockK;
   if (p.k_blocks_per_split > max_kb) {
     if (epilogue == LBT_EPI_F32) return LBT_EUNSUPPORTED;  // caller must use the split-K epilogue
     p.k_blocks_per_split = max_kb;
@@ -918,7 +918,8 @@ extern "C" int lbt_gemm_i8_dual(const int8_t* A_hi, const uint8_t* A_lo, size_t 
   p.k_blocks = (uint32_t)((K + kBlockK - 1) / kBlockK);
   p.k_blocks_per_split = p.k_blocks;
   p.k_splits = 1;
-  if (p.k_blocks > 65536 / kBlockK) return LBT_EUNSUPPORTED;   // each s32 accumulator sums at most 65536 products
+  // each s32 accumulator sums at most 65536 products, 32768 for the low plane (u8) x a u8 B
+  if (p.k_blocks > max_products(LBT_MANT_U8, b_kind) / kBlockK) return LBT_EUNSUPPORTED;
   p.epilogue = LBT_EPI_F32;
   p.ibA = ibA;
   p.ibB = ibB;
