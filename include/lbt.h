@@ -519,6 +519,32 @@ int lbt_bn_bwd_apply(const void* kg1, const int8_t* k1, size_t n_outer, size_t n
                      uint8_t* g_mant_lo, void* stream);
 
 /*
+ * The backward pass of a batch-norm with FROZEN statistics — training mode that normalises with the running averages
+ * (dfxp:616 with mean = run_mean, var = run_var as constants) and never updates them — in ONE pass.  With constant mean
+ * and variance the normalisation's VJP is elementwise, so no batch sums over kg1 and no k1 are needed:
+ *   mask  = relu: 0 none, 1 (k2 * 2^-f2 * gamma_q + beta_q > 0), 2 (out > 0); d_add = g * mask (if d_add != NULL)
+ *   kg2   = Q_g2(g * mask)                               (dfxp:687)   sums[0..C)  = sum kg2      (dbeta, :690)
+ *                                                                     sums[C..2C) = sum kg2 * k2 (dgamma, :689)
+ *   kg1   = Q_g1(RN(kg2 * 2^-fg2 * gamma_q))             (dfxp:691, :621)
+ *   den   = RN(sqrt(RN(run_var + eps)))
+ *   dx    = RN(RN(kg1 * 2^-fg1) / den)                   (correctly rounded)
+ * q_grad != NULL: dx is quantised on the spot with the producing convolution's gradient quantiser (dfxp:300) into g_mant,
+ * and `dx` may be NULL.  grad_kind: LBT_MANT_S8 (every gradient quantiser <= 8 bits, g_mant s8) or LBT_MANT_S16 (up to 16
+ * bits, 64-bit partial sums; a q_grad wider than 8 bits writes the byte planes g_mant = hi (s8), g_mant_lo = lo (u8),
+ * k = 256 * hi + lo, as lbt_bn_bwd_apply does).  `sums` (2*C int64) must be zeroed by the caller; the two sums are exact.
+ * The overflow counters of the two (three) gradient quantisers count as in training.  NULL g / k2 / ib2 / gamma_q / beta_q /
+ * run_var / ib_g2 / ib_g1 / sums, relu == 2 without `out`, neither dx nor q_grad, C % 4 != 0, or a bit width out of range
+ * (bits2 2..8, gradients 2..8 or 2..16 by grad_kind): LBT_EINVAL before any CUDA call.
+ */
+int lbt_bn_bwd_running(const float* g, const float* out, int relu, const int8_t* k2, size_t n_outer, size_t n_inner, int C,
+                       int bits2, const int32_t* ib2, const float* gamma_q, const float* beta_q, const float* run_var, float eps,
+                       int bits_g2, const int32_t* ib_g2, const float* noise_g2, uint64_t offset_g2, uint64_t* counters_g2,
+                       int bits_g1, const int32_t* ib_g1, const float* noise_g1, uint64_t offset_g1, uint64_t* counters_g1,
+                       uint64_t seed, const uint64_t* dev_step, float* d_add, int64_t* sums, float* dx,
+                       const lbt_qsite* q_grad, int8_t* g_mant, uint8_t* g_mant_lo, int stats_minmax, int grad_kind,
+                       void* stream);
+
+/*
  * lbt_bn_bwd_quant_stats + lbt_bn_bwd_apply in ONE launch, for tensors small enough that the whole tensor is one wave of
  * resident CTAs (<= 16 batch rows per CTA): the mantissas the second pass needs stay in shared memory and the CTAs meet
  * at a grid-wide barrier (`barrier`: one zeroed uint64 on the device).  Same arithmetic, bit-identical results.  Returns

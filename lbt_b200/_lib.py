@@ -101,6 +101,13 @@ SIGNATURES = {
                                               c_void_p, c_int, c_int, c_void_p]),
     'lbt_bn_bwd_apply': (c_int, [c_void_p, c_void_p, c_size_t, c_size_t, c_int, c_int, c_void_p, c_void_p, c_float,
                                  c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    # g, out, relu, k2, n_outer, n_inner, C, bits2, ib2, gamma_q, beta_q, run_var, eps, bits_g2, ib_g2, noise_g2, offset_g2,
+    # counters_g2, bits_g1, ib_g1, noise_g1, offset_g1, counters_g1, seed, dev_step, d_add, sums, dx, q_grad, g_mant, g_mant_lo,
+    # stats_minmax, grad_kind, stream
+    'lbt_bn_bwd_running': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_size_t, c_int, c_int, c_void_p, c_void_p,
+                                   c_void_p, c_void_p, c_float, c_int, c_void_p, c_void_p, c_u64, c_void_p, c_int, c_void_p,
+                                   c_void_p, c_u64, c_void_p, c_u64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                   c_void_p, c_int, c_int, c_void_p]),
     'lbt_conv_i8_dgrad_strided_dual': (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_int, c_size_t] + [c_int] * 9 +
                                        [c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p, c_void_p]),
     'lbt_conv_i8_dgrad_strided': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_size_t, c_int, c_int, c_int,

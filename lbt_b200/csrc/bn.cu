@@ -1323,6 +1323,166 @@ __global__ void __launch_bounds__(kThreads, 2) bn_bwd_fused_kernel(const BwdFuse
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// bwd with frozen statistics: training with the running averages (dfxp:616 with mean and var constants).  The
+// normalisation's VJP is then elementwise, dx = gq1 / den, so ONE pass does what bwd 1 + bwd 2 do in training: no sums
+// over kg1, no k1.  Per element: ReLU mask -> kg2 = Q(g) (dfxp:687) with the dgamma / dbeta sums -> kg1 = Q(gq2 * gamma_q)
+// (dfxp:691, :621) -> dx = RN(kg1 * 2^-fg1) / sqrt(run_var + eps), correctly rounded -> fp32 dx and / or the producing
+// convolution's gradient quantiser (dfxp:300).
+// ------------------------------------------------------------------------------------------------
+struct BwdRunParams {
+  Tiling t;
+  const float* g;          // gradient w.r.t. the module output
+  const float* out;        // module output (RELU == 2)
+  const int8_t* k2;
+  int bits2;
+  const int32_t* ib2;
+  const float* gq;
+  const float* bq;
+  const float* run_var;    // [C] read only
+  float eps;
+  QSite qg2;               // Rescale_q's gradient quantiser (dfxp:687)
+  QSite qg1;               // Normalization_q's gradient quantiser (dfxp:621)
+  float* d_add;            // optional: gradient w.r.t. the fused shortcut input (= masked g)
+  long long* sums;         // [2*C]: sum kg2, sum kg2*k2
+  float* dx;               // may be NULL when qg is on
+  QSite qg;                // optional: the producing convolution's gradient quantiser (bits == 0: off)
+  int8_t* g_mant;          // its mantissas: s8, or the HIGH byte plane when qg.bits > 8 (WIDE only) ...
+  uint8_t* g_mant_lo;      // ... with the low byte plane here (k = 256 * hi + lo)
+};
+
+// WIDE: gradient quantisers of 9..16 bits (BASELINE config 5) — 64-bit partial sums, and a convolution gradient wider than 8 bits
+// leaves as the two byte planes its tensor-core kernels consume.  MM: min/max statistics for every site of the launch.
+// RELU: 0 none, 1 mask recomputed from k2, 2 mask from `out`.
+template <bool WIDE, bool MM, int RELU>
+__global__ void __launch_bounds__(kThreads, LBT_BN_BWD1_CTAS) bn_bwd_running_kernel(const BwdRunParams p) {
+  extern __shared__ unsigned long long s_acc[];
+  __shared__ uint32_t s_red[16];
+  pdl_trigger();
+  pdl_wait();
+  const int C = p.t.C;
+  const QC c2 = make_qc(p.bits2, __ldg(p.ib2));
+  const QC cg2 = make_qc(p.qg2.bits, __ldg(p.qg2.ib));
+  const QC cg1 = make_qc(p.qg1.bits, __ldg(p.qg1.ib));
+  const uint64_t off2 = site_offset(p.qg2), off1 = site_offset(p.qg1);
+  const bool gq_on = p.qg.bits != 0;
+  QC cq = cg1;
+  uint64_t offq = 0;
+  if (gq_on) {
+    cq = make_qc(p.qg.bits, __ldg(p.qg.ib));
+    offq = site_offset(p.qg);
+  }
+  const bool q16 = WIDE && gq_on && p.qg.bits > 8;
+  uint32_t a1 = 0, a2 = 0, b1 = 0, b2 = 0, n1 = 0, n2 = 0;
+  float amx = -INFINITY, amn = INFINITY, bmx = -INFINITY, bmn = INFINITY, qmx = -INFINITY, qmn = INFINITY;
+  using AccT = typename std::conditional<WIDE, long long, int>::type;
+  Acc<2, AccT> acc;
+  acc.zero();
+  const float gscale = cg2.inv_m * cg1.m;   // kg2 -> dx2 (x 2^-fg2) -> scaled for the second quantiser (x 2^fg1): exact
+  const bool has_dadd = p.d_add != nullptr, has_dx = p.dx != nullptr;
+  for (uint64_t tile = blockIdx.x; tile < p.t.total_tiles; tile += gridDim.x) {
+    const uint32_t rg = (uint32_t)(tile / p.t.chunks), chk = (uint32_t)(tile % p.t.chunks);
+    const uint32_t v = chk * kThreads + threadIdx.x;
+    if (v < p.t.n_vec) {
+      const int c0 = (int)((4ull * v) % (uint64_t)C);
+      const float4 u2v = site_noise(p.qg2, v, off2), u1v = site_noise(p.qg1, v, off1);
+      const float u2[4] = {u2v.x, u2v.y, u2v.z, u2v.w}, u1[4] = {u1v.x, u1v.y, u1v.z, u1v.w};
+      float uq[4] = {0.f, 0.f, 0.f, 0.f};
+      if (gq_on) {
+        const float4 t = site_noise(p.qg, v, offq);
+        uq[0] = t.x; uq[1] = t.y; uq[2] = t.z; uq[3] = t.w;
+      }
+      float gk[4], b[4], gd[4], den[4], rden[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float gq = __ldg(p.gq + c0 + j);
+        gk[j] = gq * c2.inv_m;     // for the ReLU mask: xq2 * gq = k2 * (gq / m2)
+        gd[j] = gq * gscale;       // dx2 * mg1 = kg2 * (gq * mg1 / mg2)
+        b[j] = __ldg(p.bq + c0 + j);
+        den[j] = __fsqrt_rn(__fadd_rn(__ldg(p.run_var + c0 + j), p.eps));   // (var + eps) ** 0.5, dfxp:616
+        rden[j] = __frcp_rn(den[j]);
+      }
+      const uint32_t r0 = rg * p.t.rows_per_group, r1 = min(r0 + p.t.rows_per_group, (uint32_t)p.t.n_outer);   // rows: 32-bit (make_tiling)
+      for (uint32_t r = r0; r < r1; r += kRows) {
+        float4 gv[kRows], ov[kRows];
+        uint32_t w2[kRows];
+#pragma unroll
+        for (int i = 0; i < kRows; ++i)
+          if (r + i < r1) {
+            const size_t idx = 4 * (size_t)((r + i) * p.t.n_vec + v);   // element / 4 fits 32 bits
+            gv[i] = __ldcs(reinterpret_cast<const float4*>(p.g + idx));
+            w2[i] = __ldcs(reinterpret_cast<const uint32_t*>(p.k2 + idx));
+            if (RELU == 2) ov[i] = __ldcs(reinterpret_cast<const float4*>(p.out + idx));
+          }
+#pragma unroll
+        for (int i = 0; i < kRows; ++i)
+          if (r + kRows + i < r1) {
+            const size_t idx = 4 * (size_t)((r + kRows + i) * p.t.n_vec + v);
+            prefetch_l1(p.g + idx);
+            prefetch_l1(p.k2 + idx);
+            if (RELU == 2) prefetch_l1(p.out + idx);
+          }
+#pragma unroll
+        for (int i = 0; i < kRows; ++i)
+          if (r + i < r1) {
+            const size_t idx = 4 * (size_t)((r + i) * p.t.n_vec + v);
+            int k2[4];
+            unpack4(w2[i], k2);
+            float k2f[4];
+            if (RELU == 1) dec4_f(w2[i], k2f);
+            const float gin[4] = {gv[i].x, gv[i].y, gv[i].z, gv[i].w};
+            const float oin[4] = {ov[i].x, ov[i].y, ov[i].z, ov[i].w};
+            float gm[4], o[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              float gj = gin[j];
+              if (RELU == 1) {
+                const float y2 = __fadd_rn(__fmul_rn(k2f[j], gk[j]), b[j]);
+                if (!(y2 > 0.0f)) gj = 0.0f;
+              } else if (RELU == 2) {
+                if (!(oin[j] > 0.0f)) gj = 0.0f;
+              }
+              gm[j] = gj;
+              const float tg2 = sq_scaled<MM>(__fmul_rn(gj, cg2.m), u2[j], cg2, amx, amn, a1, a2);   // dfxp:687
+              const int kg2i = tm_int(tg2);
+              acc.s[0][j] += kg2i;                                                 // dbeta  (dfxp:690)
+              acc.s[1][j] += (AccT)kg2i * k2[j];                                   // dgamma (dfxp:689)
+              const float t1 = sq_scaled<MM>(__fmul_rn(tm_float(tg2), gd[j]), u1[j], cg1, bmx, bmn, b1, b2);   // dfxp:691, :621
+              // the VJP of (xq - mean) / den with constant mean and den: gq1 / den, correctly rounded
+              o[j] = fdiv_by(__fmul_rn(tm_float(t1), cg1.inv_m), den[j], rden[j]);
+            }
+            if (has_dadd) *reinterpret_cast<float4*>(p.d_add + idx) = make_float4(gm[0], gm[1], gm[2], gm[3]);
+            if (has_dx) *reinterpret_cast<float4*>(p.dx + idx) = make_float4(o[0], o[1], o[2], o[3]);
+            if (gq_on) {                                                        // the convolution's gradq, dfxp:300
+              float tq[4];
+#pragma unroll
+              for (int j = 0; j < 4; ++j) tq[j] = sq_scaled<MM>(__fmul_rn(o[j], cq.m), uq[j], cq, qmx, qmn, n1, n2);
+              if (q16) {
+                uint32_t hi, lo;
+                tm_pack4_hilo(tq, hi, lo);
+                *reinterpret_cast<uint32_t*>(p.g_mant + idx) = hi;
+                *reinterpret_cast<uint32_t*>(p.g_mant_lo + idx) = lo;
+              } else {
+                *reinterpret_cast<uint32_t*>(p.g_mant + idx) = tm_pack4(tq);
+              }
+            }
+          }
+      }
+      if (!p.t.fixed_channels) flush_global(acc, p.sums, C, c0);
+    }
+  }
+  if (p.t.fixed_channels) flush_block(acc, p.sums, C, s_acc);
+  const size_t numel = p.t.n_outer * p.t.n_inner;
+  if (MM) {
+    mm_to_counts(cg2, amx, amn, a1, a2);
+    mm_to_counts(cg1, bmx, bmn, b1, b2);
+    if (gq_on) mm_to_counts(cq, qmx, qmn, n1, n2);
+  }
+  publish_counters(p.qg2.counters, a1, a2, numel, s_red);
+  publish_counters(p.qg1.counters, b1, b2, numel, s_red);
+  if (gq_on) publish_counters(p.qg.counters, n1, n2, numel, s_red);
+}
+
 // ---- host helpers ----------------------------------------------------------------------------
 // Resident CTAs per SM of a kernel with `smem` dynamic bytes (cached per kernel and device).
 template <typename K>
@@ -1852,6 +2012,65 @@ extern "C" int lbt_bn_bwd_fused(const lbt_bn_bwd_args* a, void* stream) {
   launch_pdl(bn_bwd_fused_kernel, grid, kThreads, smem_max, reinterpret_cast<cudaStream_t>(stream), q);
   (void)smem;
   return check_launch("lbt_bn_bwd_fused");
+}
+
+extern "C" int lbt_bn_bwd_running(const float* g, const float* out, int relu, const int8_t* k2, size_t n_outer, size_t n_inner,
+                                  int C, int bits2, const int32_t* ib2, const float* gamma_q, const float* beta_q,
+                                  const float* run_var, float eps, int bits_g2, const int32_t* ib_g2, const float* noise_g2,
+                                  uint64_t offset_g2, uint64_t* counters_g2, int bits_g1, const int32_t* ib_g1,
+                                  const float* noise_g1, uint64_t offset_g1, uint64_t* counters_g1, uint64_t seed,
+                                  const uint64_t* dev_step, float* d_add, int64_t* sums, float* dx, const lbt_qsite* q_grad,
+                                  int8_t* g_mant, uint8_t* g_mant_lo, int stats_minmax, int grad_kind, void* stream) {
+  if (!g || !k2 || !ib2 || !gamma_q || !beta_q || !run_var || !ib_g2 || !ib_g1 || !sums) return LBT_EINVAL;
+  if (C <= 0 || (C & 3)) return LBT_EINVAL;
+  if (relu < 0 || relu > 2 || (relu == 2 && !out)) return LBT_EINVAL;
+  if (!dx && !q_grad) return LBT_EINVAL;
+  if (grad_kind != LBT_MANT_S8 && grad_kind != LBT_MANT_S16) return LBT_EINVAL;
+  const bool wide = grad_kind == LBT_MANT_S16;
+  const int gmax = wide ? 16 : 8;
+  if (bits2 < 2 || bits2 > 8 || bits_g2 < 2 || bits_g2 > gmax || bits_g1 < 2 || bits_g1 > gmax) return LBT_EINVAL;
+  if (q_grad) {
+    if (!g_mant || !q_grad->ib || q_grad->bits < 2 || q_grad->bits > gmax) return LBT_EINVAL;
+    if (q_grad->bits > 8 && !g_mant_lo) return LBT_EINVAL;   // two byte planes: k = 256 * hi + lo
+  }
+  if (n_outer == 0 || n_inner == 0) return LBT_OK;
+  if (!al16(g) || !al4(k2) || (out && !al16(out)) || (d_add && !al16(d_add)) || (dx && !al16(dx)) || (g_mant && !al4(g_mant)) ||
+      (g_mant_lo && !al4(g_mant_lo)) || (noise_g2 && !al16(noise_g2)) || (noise_g1 && !al16(noise_g1)) ||
+      (q_grad && q_grad->noise && !al16(q_grad->noise)))
+    return LBT_EUNSUPPORTED;
+  LBT_REQUIRE_ARCH();
+  // one statistics flavour per launch: min/max only when EVERY site asked for it (exact counts are always valid)
+  const bool mm = stats_minmax && (!q_grad || q_grad->stats_minmax);
+  void (*kern)(const BwdRunParams) = nullptr;
+#define LBT_BWDR(W, M) \
+  (relu == 0 ? bn_bwd_running_kernel<W, M, 0> : (relu == 1 ? bn_bwd_running_kernel<W, M, 1> : bn_bwd_running_kernel<W, M, 2>))
+  kern = wide ? (mm ? LBT_BWDR(true, true) : LBT_BWDR(true, false)) : (mm ? LBT_BWDR(false, true) : LBT_BWDR(false, false));
+#undef LBT_BWDR
+  BwdRunParams p{};
+  unsigned grid;
+  const size_t smem = (size_t)2 * C * 8;
+  int rc = make_tiling(p.t, n_outer, n_inner, C, grid, ctas_per_sm(kern, smem));
+  if (rc) return rc;
+  p.g = g;
+  p.out = out;
+  p.k2 = k2;
+  p.bits2 = bits2;
+  p.ib2 = ib2;
+  p.gq = gamma_q;
+  p.bq = beta_q;
+  p.run_var = run_var;
+  p.eps = eps;
+  p.qg2 = make_site(bits_g2, ib_g2, noise_g2, seed, offset_g2, dev_step, counters_g2, stats_minmax);
+  p.qg1 = make_site(bits_g1, ib_g1, noise_g1, seed, offset_g1, dev_step, counters_g1, stats_minmax);
+  p.d_add = d_add;
+  p.sums = reinterpret_cast<long long*>(sums);
+  p.dx = dx;
+  p.qg = site_from_abi(q_grad);
+  p.g_mant = g_mant;
+  p.g_mant_lo = g_mant_lo;
+  if ((rc = set_smem(kern, smem))) return rc;
+  launch_pdl(kern, grid, kThreads, smem, reinterpret_cast<cudaStream_t>(stream), p);
+  return check_launch("lbt_bn_bwd_running");
 }
 
 // Non-zero once the grid barrier of lbt_bn_bwd_fused has timed out (synchronises the device; not in lbt.h).

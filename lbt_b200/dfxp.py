@@ -1265,7 +1265,8 @@ class _WeightDecayGrad(torch.autograd.Function):
 class Normalization_q(nn.Module):
     """dfxp:539-623: quantise, batch moments of the QUANTISED input (biased variance), normalise;
     running statistics with momentum 0.999; backward quantises the gradient then applies the
-    batch-norm VJP."""
+    batch-norm VJP.  ``frozen`` (set by BatchNorm2d_q.freeze_statistics): in training mode too, normalise with the running
+    statistics and leave them alone — the VJP is then g / sqrt(var + eps)."""
 
     def __init__(self, bits, num_features, momentum=0.999, eps=1e-5, *, target_overflow_rate=0.0, input_range=2,
                  grad_range=2, grad_bits=None, name='norm', runtime=None):
@@ -1276,13 +1277,14 @@ class Normalization_q(nn.Module):
         self.register_buffer('X_var_running', torch.ones(num_features))
         self.qX = QuantSite(rt, name + '/X', bits, input_range, target_overflow_rate)          # dfxp:584
         self.qG = QuantSite(rt, name + '/grad', grad_bits or bits, grad_range, target_overflow_rate)   # dfxp:621
+        self.frozen = False
 
     def forward(self, x):
         x = _mem_contig(x)
         xq = _QuantSTE.apply(x, self.qX)
         axes = (0, 2, 3) if x.dim() == 4 else (0,)
         shape = (1, -1, 1, 1) if x.dim() == 4 else (1, -1)
-        if self.training:
+        if self.training and not self.frozen:
             mean = xq.mean(dim=axes)                                                           # dfxp:588
             var = ((xq - mean.view(shape)) ** 2).mean(dim=axes)
             with torch.no_grad():                                                              # dfxp:602-612
@@ -1362,17 +1364,17 @@ def _bn_fwd1(bn, xm_):
 
 
 def _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, next_site=None, next_kind=Q.MANT_NONE, want_fp32=True, next2=None,
-             running=False):
+             running=False, want_k2=False):
     """BN forward pass 2 (+ residual add, ReLU, the consumer's input quantiser): (k2, out or None, next mantissas or None,
     relu_mode).  next2 = (site, kind): a second consumer's input quantiser; its mantissas come back as ``next2[2]`` (a list
     cell the caller passes in).  running: eval mode — normalise with the running statistics (``sums`` is not read, the
-    running averages stay, k2 is None)."""
+    running averages stay, k2 is None unless ``want_k2``: frozen statistics save it for lbt_bn_bwd_running)."""
     norm, resc = bn[0], bn[1]
     rt = norm.qX.runtime
     N, C = k1.shape[0], k1.shape[-1]
     n_inner = k1.numel() // N
     dev = k1.device
-    k2 = None if running else torch.empty_like(k1)
+    k2 = torch.empty_like(k1) if (want_k2 or not running) else None
     out = torch.empty(k1.shape, dtype=torch.float32, device=dev) if want_fp32 else None
     nz2, off2 = _site_args(resc.qX, k1)
     relu_mode = 0 if not relu else (2 if add_ is not None else 1)
@@ -1386,7 +1388,7 @@ def _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, next_site=None, next_kind=Q.MANT_
         qn2 = site2.abi(n_inner, dev)
         nm2 = torch.empty(k1.shape, dtype=torch.uint8 if kind2 == Q.MANT_U8 else torch.int8, device=dev)
         next2[2] = nm2
-    nbytes = k1.numel() * ((1 if running else 2) + (4 if want_fp32 else 0) + (4 if add_ is not None else 0) +
+    nbytes = k1.numel() * ((1 if k2 is None else 2) + (4 if want_fp32 else 0) + (4 if add_ is not None else 0) +
                            (1 if nm is not None else 0) + (1 if nm2 is not None else 0))
     head = (_lib.ptr(k1), N, n_inner, C, norm.qX.bits, _lib.ptr(norm.qX.range))
     site = (float(norm.eps), resc.qX.bits, _lib.ptr(resc.qX.range), _lib.ptr(nz2), rt.seed, off2,
@@ -1486,28 +1488,70 @@ def _bn_backward(bn, g_, k1, k2, sums, gq, bq, out_, relu_mode, has_add, grad_si
     return dx, (gm if gm_lo is None else (gm, gm_lo)), dgamma, dbeta, d_add
 
 
+def _bn_backward_frozen(bn, g_, k2, gq, bq, out_, relu_mode, has_add, grad_site=None, want_dx=True):
+    """The BN backward pass of a layer with frozen statistics (BatchNorm2d_q.freeze_statistics), ONE launch
+    (lbt_bn_bwd_running): mean and variance are constants, so dx = gq1 / sqrt(run_var + eps) needs neither k1 nor batch sums
+    over the gradient.  Same results and return value as _bn_backward."""
+    norm, resc = bn[0], bn[1]
+    rt = norm.qX.runtime
+    N, C = k2.shape[0], k2.shape[-1]
+    n_inner = k2.numel() // N
+    dev = k2.device
+    bsums = rt.zeros_i64(2 * C, dev)
+    d_add = torch.empty(k2.shape, dtype=torch.float32, device=dev) if has_add else None
+    dx = torch.empty(k2.shape, dtype=torch.float32, device=dev) if want_dx else None
+    qg = gm = gm_lo = None
+    if grad_site is not None:
+        qg = grad_site.abi(n_inner, dev)
+        gm = torch.empty_like(k2)
+        if grad_site.bits > 8:
+            gm_lo = torch.empty(k2.shape, dtype=torch.uint8, device=dev)
+    # any gradient quantiser wider than 8 bits (config 5: 16-bit G): the wide instantiation (64-bit partial sums, byte planes)
+    wide = max(resc.qG.bits, norm.qG.bits, grad_site.bits if grad_site is not None else 0) > 8
+    nzg2, offg2 = _site_args(resc.qG, g_)
+    nzg1, offg1 = _site_args(norm.qG, g_)
+    nbytes = k2.numel() * (5 + (4 if relu_mode == 2 else 0) + (4 if has_add else 0) + (4 if want_dx else 0) +
+                           (1 if gm is not None else 0) + (1 if gm_lo is not None else 0))
+    _lib.call('lbt_bn_bwd_running', _lib.ptr(g_), _lib.ptr(out_), relu_mode, _lib.ptr(k2), N, n_inner, C, resc.qX.bits,
+              _lib.ptr(resc.qX.range), _lib.ptr(gq), _lib.ptr(bq), _lib.ptr(norm.X_var_running), float(norm.eps), resc.qG.bits,
+              _lib.ptr(resc.qG.range), _lib.ptr(nzg2), offg2, _lib.ptr(resc.qG.counters), norm.qG.bits,
+              _lib.ptr(norm.qG.range), _lib.ptr(nzg1), offg1, _lib.ptr(norm.qG.counters), rt.seed, _lib.ptr(rt.dev_step),
+              _lib.ptr(d_add), _lib.ptr(bsums), _lib.ptr(dx), ctypes.addressof(qg) if qg is not None else None, _lib.ptr(gm),
+              _lib.ptr(gm_lo), int(resc.qG.target == 0 and norm.qG.target == 0), Q.MANT_S16 if wide else Q.MANT_S8,
+              _lib.stream(), meta=dict(bytes=nbytes))
+    # dbeta = sum gq2 (dfxp:690); dgamma = sum gq2 * xq2 + 2*wd*gamma (dfxp:689)
+    dbeta = _emit_grad(rt, resc.beta, bsums[:C], ibA=resc.qG.range, exp_const=-(resc.qG.bits - 1))
+    dgamma = _emit_grad(rt, resc.gamma, bsums[C:2 * C], ibA=resc.qG.range, ibB=resc.qX.range,
+                        exp_const=-(resc.qG.bits - 1) - (resc.qX.bits - 1), add_scale=2 * resc.weight_decay)
+    return dx, (gm if gm_lo is None else (gm, gm_lo)), dgamma, dbeta, d_add
+
+
 class _FusedBNFn(torch.autograd.Function):
     """Normalization_q + Rescale_q (+ residual add, + ReLU) in 2 forward and 2 backward passes over the
     activation (csrc/bn.cu), saving only the two s8 mantissa tensors for backward."""
 
     @staticmethod
-    def forward(ctx, x, gamma, beta, add, bn, relu, running=False):
-        # running: eval mode without an autograd graph (BatchNorm2d_q._running); nothing is saved
+    def forward(ctx, x, gamma, beta, add, bn, relu, running=False, frozen=False):
+        # running: eval mode (or frozen statistics) without an autograd graph (BatchNorm2d_q._running); nothing is saved.
+        # frozen: frozen statistics with a graph — the running-statistics forward, k2 saved for lbt_bn_bwd_running (no k1)
         x_ = _to_mem(x)
         k1, sums = _bn_fwd1(bn, x_)
         gq, bq = _bn_params(bn[1], gamma, beta)
         add_ = _to_mem(add) if add is not None else None
-        k2, out, _, relu_mode = _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, running=running)
+        k2, out, _, relu_mode = _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, running=running or frozen, want_k2=frozen)
         if not running:
-            ctx.bn, ctx.relu_mode, ctx.has_add = bn, relu_mode, add is not None
-            ctx.save_for_backward(k1, k2, sums, gq, bq, out if relu_mode == 2 else None)
+            ctx.bn, ctx.relu_mode, ctx.has_add, ctx.frozen = bn, relu_mode, add is not None, frozen
+            ctx.save_for_backward(None if frozen else k1, k2, None if frozen else sums, gq, bq, out if relu_mode == 2 else None)
         return _from_mem(out)
 
     @staticmethod
     def backward(ctx, g):
         k1, k2, sums, gq, bq, out = ctx.saved_tensors
-        dx, _, dgamma, dbeta, d_add = _bn_backward(ctx.bn, _to_mem(g), k1, k2, sums, gq, bq, out, ctx.relu_mode, ctx.has_add)
-        return _from_mem(dx), dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None), None, None, None
+        if ctx.frozen:
+            dx, _, dgamma, dbeta, d_add = _bn_backward_frozen(ctx.bn, _to_mem(g), k2, gq, bq, out, ctx.relu_mode, ctx.has_add)
+        else:
+            dx, _, dgamma, dbeta, d_add = _bn_backward(ctx.bn, _to_mem(g), k1, k2, sums, gq, bq, out, ctx.relu_mode, ctx.has_add)
+        return _from_mem(dx), dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None), None, None, None, None
 
 
 _link_count = 0        # fused backward links taken (tests)
@@ -1556,9 +1600,10 @@ class _ConvBNFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, weight, gamma, beta, add, conv, bn, relu, next_site, next_kind, want_fp32, alias, link_in, link_out, pool=None,
-                next2=None, running=False, block=None):
-        # running: eval mode without an autograd graph (BatchNorm2d_q._running): the BN kernels normalise with the running
-        # statistics, nothing is saved for backward
+                next2=None, running=False, block=None, frozen=False):
+        # running: eval mode (or frozen statistics) without an autograd graph (BatchNorm2d_q._running): the BN kernels normalise
+        # with the running statistics, nothing is saved for backward.  frozen: frozen statistics while a graph is recorded —
+        # the same kernels, k2 saved (k1 and the batch sums are not), backward through lbt_bn_bwd_running
         geom = _conv_geom(conv, x, weight)
         N, H, W, Cin, Cout, kh, kw, sh, sw, pt, pl, OH, OW = geom
         norm, resc = bn[0], bn[1]
@@ -1593,7 +1638,7 @@ class _ConvBNFn(torch.autograd.Function):
             tail = (pk, ps, ppt, ppl, POH, POW, _lib.ptr(pooled), _lib.ptr(pidx),
                     ctypes.addressof(qn) if qn is not None else None, _lib.ptr(nmp), int(next_kind), _lib.stream())
             meta = dict(bytes=k1.numel() * (1 if running else 2) + pooled.numel() * (5 + (1 if nmp is not None else 0)))
-            if running:
+            if running or frozen:
                 done = _lib.try_call('lbt_bn_fwd_apply_running_pooled', *head, _lib.ptr(norm.X_mean_running),
                                      _lib.ptr(norm.X_var_running), *site, int(resc.qX.target == 0), *tail, meta=meta)
             else:
@@ -1607,9 +1652,10 @@ class _ConvBNFn(torch.autograd.Function):
                 next_site, next_kind = None, Q.MANT_NONE
         if pooled is None:
             k2, out, nm, relu_mode = _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, next_site, next_kind, True if pool is not None else want_fp32,
-                                              next2=next2 if pool is None else None, running=running)
+                                              next2=next2 if pool is None else None, running=running or frozen,
+                                              want_k2=frozen)
         ctx.conv, ctx.bn, ctx.geom, ctx.xkind, ctx.prep = conv, bn, geom, xkind, prep
-        ctx.relu_mode, ctx.has_add = relu_mode, add is not None
+        ctx.relu_mode, ctx.has_add, ctx.frozen = relu_mode, add is not None, frozen
         ctx.link_in, ctx.link_out = link_in, link_out
         # block: the downsampling block's _BlockDgrad; the unit with the alias is the first unit, the other one the shortcut
         ctx.block = None
@@ -1620,7 +1666,7 @@ class _ConvBNFn(torch.autograd.Function):
             elif block.armed:
                 ctx.block = block
         ctx.block_first = bool(alias)
-        if link_out is not None and out is None and not running:     # the next unit may run this BN's backward pass 1 in its dgrad epilogue
+        if link_out is not None and out is None and not running and not frozen:   # the next unit may run this BN's backward pass 1 in its dgrad epilogue
             link_out.offer(bn, k1, k2, gq, bq, relu_mode, add is not None)
         ctx.pool = None
         if pooled is not None:    # lbt_bn_fwd_apply_pooled did both
@@ -1635,7 +1681,8 @@ class _ConvBNFn(torch.autograd.Function):
             ctx.pool = (pk, ps, ppt, ppl, POH, POW)
             out = pooled
         if not running:
-            ctx.save_for_backward(xm, wm, k1, k2, sums, gq, bq, out if relu_mode == 2 else None, pidx)
+            ctx.save_for_backward(xm, wm, None if frozen else k1, k2, None if frozen else sums, gq, bq,
+                                  out if relu_mode == 2 else None, pidx)
         if out is None:       # mantissa-only activation: the fp32 tensor is never materialised (shape carrier only)
             out = torch.empty(1, dtype=torch.float32, device=dev).expand(N, OH, OW, Cout)
         if nm is None:
@@ -1655,19 +1702,23 @@ class _ConvBNFn(torch.autograd.Function):
         lo = ctx.link_out
         pre = (lo.kg1, lo.bsums) if (lo is not None and lo.done) else None     # pass 1 ran in the consumer's dgrad epilogue
         pool = ((pidx,) + ctx.pool) if ctx.pool is not None else None
-        if pool is not None and not FUSE_POOL:
+        if pool is not None and (not FUSE_POOL or ctx.frozen):
             # the pool's backward as its own launch (lbt_maxpool_bwd, 0.82 of the HBM peak), then the plain BN pass 1: faster
             # on B200 than gathering the windows inside pass 1 (FUSE_POOL)
             _, pk, ps, ppt, ppl, POH, POW = pool
             g_ = _to_mem(g)
-            Np, Hp, Wp_, Cp = k1.shape
-            gd = torch.empty(k1.shape, dtype=torch.float32, device=k1.device)
+            Np, Hp, Wp_, Cp = k2.shape        # (k1 is not saved with frozen statistics)
+            gd = torch.empty(k2.shape, dtype=torch.float32, device=k2.device)
             _lib.call('lbt_maxpool_bwd', _lib.ptr(g_), _lib.ptr(pidx), Np, Hp, Wp_, Cp, pk, ps, ppt, ppl, POH, POW, _lib.ptr(gd),
                       _lib.stream(), meta=dict(bytes=gd.numel() * 4 + g_.numel() * 5))
             g, pool = _from_mem(gd), None
-        _, gm, dgamma, dbeta, d_add = _bn_backward(ctx.bn, _to_mem(g) if pre is None else None, k1, k2, sums, gq, bq, out,
-                                                   ctx.relu_mode, ctx.has_add, grad_site=conv.qG, want_dx=False, pre=pre,
-                                                   pool=pool)   # ... dfxp:300
+        if ctx.frozen:
+            _, gm, dgamma, dbeta, d_add = _bn_backward_frozen(ctx.bn, _to_mem(g), k2, gq, bq, out, ctx.relu_mode, ctx.has_add,
+                                                              grad_site=conv.qG, want_dx=False)   # ... dfxp:300
+        else:
+            _, gm, dgamma, dbeta, d_add = _bn_backward(ctx.bn, _to_mem(g) if pre is None else None, k1, k2, sums, gq, bq, out,
+                                                       ctx.relu_mode, ctx.has_add, grad_site=conv.qG, want_dx=False, pre=pre,
+                                                       pool=pool)   # ... dfxp:300
         bd = ctx.block
         if bd is not None and not ctx.block_first:
             ctx.block = None
@@ -1677,7 +1728,7 @@ class _ConvBNFn(torch.autograd.Function):
                 bd.parked = (conv, ctx.geom, ctx.xkind, wm, ctx.prep, gm)
                 N, H, W, Cin = ctx.geom[:4]
                 dx = torch.empty(1, dtype=torch.float32, device=gm.device).expand(N, H, W, Cin)     # shape carrier only
-                return ((_from_mem(dx),) + (dW, dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None)) + (None,) * 13)
+                return ((_from_mem(dx),) + (dW, dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None)) + (None,) * 14)
         parked = bd.take() if (bd is not None and need_dx) else None
         shortcut = None
         if parked is not None:     # g_alias is the shortcut unit's shape carrier
@@ -1697,7 +1748,7 @@ class _ConvBNFn(torch.autograd.Function):
                                        shortcut=shortcut)
         return ((_from_mem(dx) if dx is not None else None), dW, dgamma, dbeta,
                 (_from_mem(d_add) if d_add is not None else None), None, None, None, None, None, None, None, None, None, None, None,
-                None, None)
+                None, None, None)
 
 
 FUSE_POOL = os.environ.get('LBT_FUSE_POOL', '0') == '1'   # module switch: a MaxPool_q right behind a fused unit runs its backward inside the
@@ -1730,6 +1781,7 @@ def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=Tr
     ONLY consumer) skips the fp32 tensor altogether."""
     relu = relu or getattr(bn, 'relu', False)
     running = isinstance(bn, BatchNorm2d_q) and bn._running(x, add, conv.weight)
+    frozen = isinstance(bn, BatchNorm2d_q) and not running and bn._frozen()    # frozen statistics with a backward pass
     if not _unit_fusable(conv, bn, x, running):
         y = bn(conv(x), add=add, relu=relu) if isinstance(bn, BatchNorm2d_q) else bn(conv(x))
         if pool is not None:
@@ -1768,13 +1820,13 @@ def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=Tr
     # measured: folding pays while the dgrad output is narrow (ResNet-18/20 blocks: -1.6 % step time); for the 256..2048-
     # channel block inputs of ResNet-50 the epilogue-bound 1x1 dgrad GEMMs lose more than the coalesced add costs (+3 %)
     # block (a downsampling block's _BlockDgrad): the shortcut's gradient joins inside the first unit's input-gradient launch,
-    # so the alias pays at every width
+    # so the alias pays at every width (frozen statistics keep both: that unit has a backward pass)
     block = block if (FUSE_BLOCK_DGRAD and not running) else None
     use_alias = bool(alias and x.requires_grad and not getattr(x, '_lbt_hollow', False) and
                      (conv.weight.shape[2] <= 128 or (block is not None and tuple(conv.stride) != (1, 1) and conv.qG.bits <= 8)))
     out, nm, xa = _ConvBNFn.apply(x, conv.weight, bn[1].gamma, bn[1].beta, add, conv, bn, relu, next_site, next_kind,
                                   want_fp32, use_alias, link_in if FUSE_BWD_LINK else None, link_out if FUSE_BWD_LINK else None,
-                                  pgeom, next2, running, block)
+                                  pgeom, next2, running, block, frozen)
     if next_site is not None and nm.numel():       # (empty: the pooled one-kernel path declined, the consumer quantises itself)
         out._lbt_q = {id(next_site): (nm, next_kind)}
         if next2 is not None and next2[2] is not None:
@@ -1831,8 +1883,10 @@ class BatchNorm2d_q(nn.Sequential):
     In training mode with <= 8-bit activation quantisers, <= 16-bit gradient quantisers and C % 4 == 0 the pair runs as the fused kernels of
     csrc/bn.cu; ``forward(x, add=None, relu=False)`` can additionally fold the residual sum and the ReLU
     that follow it in the reference's blocks (dfxp:862, 986).  In eval mode the same kernels normalise with the running
-    statistics (dfxp:616) when no autograd graph is recorded (see ``_running``).  Otherwise the two sub-modules run one
-    after the other."""
+    statistics (dfxp:616) when no autograd graph is recorded (see ``_running``).  ``freeze_statistics()``: training mode
+    with the running statistics, which are then never updated (frozen batch-norm for quantisation-aware fine-tuning); the
+    forward pass runs the eval kernels, the backward pass is ONE launch (lbt_bn_bwd_running).  Otherwise the two
+    sub-modules run one after the other (Normalization_q honours ``frozen`` too)."""
 
     def __init__(self, bits, num_features, momentum=0.999, eps=1e-5, *, weight_decay=0.0, target_overflow_rate=0.0,
                  input_range=2, gamma_range=2, beta_range=2, grad_range=2, grad_bits=None, name='bn', runtime=None,
@@ -1847,9 +1901,25 @@ class BatchNorm2d_q(nn.Sequential):
         self.fused = fused
         self.relu = relu            # apply the ReLU that follows this BN in the reference's layer lists
 
+    @property
+    def frozen(self):
+        return self[0].frozen
+
+    def freeze_statistics(self, flag=True):
+        """Frozen statistics (flag=True) or not: in training mode the layer then normalises with the running averages and
+        never updates them; gamma and beta still train, and all four quantisers run as in training.  Eval mode is unaffected.
+        Returns self."""
+        self[0].frozen = bool(flag)
+        return self
+
+    def _frozen(self):
+        """Training mode with frozen statistics."""
+        return self.training and self[0].frozen
+
     def _can_fuse_c(self, C, dim, running=False):
         norm, resc = self[0], self[1]
-        return (self.fused and (self.training or running) and dim in (2, 4) and C % 4 == 0 and
+        # frozen statistics with a backward pass: on the kernels only with FUSE_UNITS on (off: the eager reference path)
+        return (self.fused and (running or (self.training and (FUSE_UNITS or not norm.frozen))) and dim in (2, 4) and C % 4 == 0 and
                 max(norm.qX.bits, resc.qX.bits) <= 8 and max(norm.qG.bits, resc.qG.bits) <= 16 and
                 min(norm.qX.bits, resc.qX.bits, norm.qG.bits, resc.qG.bits) >= 2)
 
@@ -1857,10 +1927,10 @@ class BatchNorm2d_q(nn.Sequential):
         return self._can_fuse_c(x.shape[1], x.dim(), running)
 
     def _running(self, *inputs):
-        """Eval mode on the fused kernels: normalise with the running statistics.  Only where no autograd graph is recorded
-        (a backward pass through running-statistics batch-norm is not built: eval mode with gradients keeps the eager path),
-        and only with FUSE_UNITS on (off, eval mode runs the eager reference arithmetic)."""
-        if self.training or not FUSE_UNITS:
+        """Eval mode (or frozen statistics) on the fused kernels without a backward pass: normalise with the running
+        statistics.  Only where no autograd graph is recorded (eval mode with gradients keeps the eager path; frozen statistics
+        with a graph take the frozen path, see ``_frozen``), and only with FUSE_UNITS on (off, the eager reference arithmetic)."""
+        if (self.training and not self[0].frozen) or not FUSE_UNITS:
             return False
         return not torch.is_grad_enabled() or not any(t is not None and t.requires_grad
                                                       for t in inputs + (self[1].gamma, self[1].beta))
@@ -1869,7 +1939,7 @@ class BatchNorm2d_q(nn.Sequential):
         relu = relu or self.relu
         running = self._running(x, add)
         if self._can_fuse(x, running):
-            return _FusedBNFn.apply(x, self[1].gamma, self[1].beta, add, self, relu, running)
+            return _FusedBNFn.apply(x, self[1].gamma, self[1].beta, add, self, relu, running, not running and self._frozen())
         y = self[1](self[0](x))
         if add is not None:
             y = y + add

@@ -39,6 +39,15 @@ class Model(nn.Module):
     def ranges(self):
         return self.runtime.ranges()
 
+    def freeze_bn_statistics(self, flag=True):
+        """Freeze (flag=True) or unfreeze the statistics of every BatchNorm2d_q: in training mode they then normalise with
+        their running averages and stop updating them, while gamma, beta and the rest of the model keep training — the usual
+        late phase of quantisation-aware training.  Eval mode is unaffected.  Returns self."""
+        for m in self.modules():
+            if isinstance(m, dfxp.BatchNorm2d_q):
+                m.freeze_statistics(flag)
+        return self
+
     def _kw(self, **extra):
         kw = dict(weight_decay=self.weight_decay, grad_bits=self.grad_bits, runtime=self.runtime)
         kw.update(extra)

@@ -213,6 +213,21 @@ class Trainer:
             loss = self.step(X_static, y_static)
         torch.cuda.synchronize(self.device)
         self._graph, self._graph_loss = graph, loss
+        from .dfxp import Normalization_q
+        self._graph_norms = [m for m in self.model.modules() if isinstance(m, Normalization_q)]
+        self._graph_frozen = [m.frozen for m in self._graph_norms]
+        return self
+
+    def _bn_mode_changed(self):
+        """True when a batch-norm was frozen or unfrozen since the step was captured."""
+        return any(m.frozen != f for m, f in zip(self._graph_norms, self._graph_frozen))
+
+    def freeze_bn_statistics(self, flag=True):
+        """``model.freeze_bn_statistics(flag)``; a captured step recorded in the other mode is dropped (the next ``capture``
+        records the new one).  Returns self."""
+        self.model.freeze_bn_statistics(flag)
+        if self.captured and self._bn_mode_changed():
+            self._graph = self._graph_loss = None
         return self
 
     @property
@@ -221,7 +236,14 @@ class Trainer:
 
     def step_graph(self):
         """One training step = one graph launch, on the current contents of the static inputs.  Returns the loss tensor
-        (static: read it, or copy it, before the next replay overwrites it)."""
+        (static: read it, or copy it, before the next replay overwrites it).  A step captured before the batch-norm
+        statistics were frozen or unfrozen on the model raises: the graph replays the kernels of the mode it was captured in."""
+        if not self.captured:
+            raise _lib.LbtError('Trainer.step_graph: no step is captured (never captured, or dropped by '
+                                'Trainer.freeze_bn_statistics); call capture(X_static, y_static) first')
+        if self._bn_mode_changed():
+            raise _lib.LbtError('Trainer.step_graph: the batch-norm statistics were frozen or unfrozen on the model after '
+                                'capture(); use Trainer.freeze_bn_statistics, which drops the graph, and capture again')
         self._graph.replay()
         return self._graph_loss
 
@@ -289,13 +311,16 @@ class Trainer:
 
     # ---- the epoch loop (trainer.py:109-187) ---------------------------------------------------------------------------
     def fit(self, pipeline, n_epoch, batch_size, *, lr_decay_factor=0.1, decay_epochs=(80, 120, 140), test=None, log=None,
-            max_batches=None, graph=False, eval_running_stats=False):
+            max_batches=None, graph=False, eval_running_stats=False, freeze_bn_epoch=None):
         """``pipeline``: lbt_b200.data.Pipeline over the device-resident training set (shuffle + flip / pad-4 / crop on
         the GPU).  The learning rate is multiplied by ``lr_decay_factor`` at epochs 80, 120 and 140 and the optimizer is
         re-created (momentum slots zeroed) exactly there (trainer.py:117-132).  ``test`` = (X, y) evaluated after each
         epoch (``eval_running_stats``: see ``evaluate(running_stats=...)``).  ``graph=True``: full batches run as replays of the captured step (capture() on first use; the pipeline
         writes each batch straight into the static inputs), a short last batch runs eagerly.  With several replicas the
         pipeline must be rank-aware (lbt_b200.data.Pipeline shards every global batch by rank).
+        ``freeze_bn_epoch``: the batch-norm statistics are frozen from the start of that (0-based) epoch on and unfrozen
+        before it (``freeze_bn_statistics``; a captured step is re-captured in the new mode).  The schedule is a function of
+        the epoch, so a resumed run re-derives it.  None: the model's setting is left as it is.
         Returns [(epoch, last_train_loss, test_loss, test_acc)]."""
         history = []
         if self.world > 1 and getattr(pipeline, 'world', 1) != self.world:
@@ -304,6 +329,8 @@ class Trainer:
         for epoch in range(n_epoch):
             if epoch in decay_epochs:
                 self.set_lr(self.lr * lr_decay_factor, reset_momentum=True)
+            if freeze_bn_epoch is not None:
+                self.freeze_bn_statistics(epoch >= freeze_bn_epoch)
             loss = None
             for b, (X, y) in enumerate(pipeline.epoch(batch_size, epoch)):
                 if max_batches is not None and b >= max_batches:
