@@ -39,7 +39,7 @@ WORKLOADS = [
     ('resnet50_224_b128_g16', M.Resnet50, dict(image=224, num_classes=1000, grad_bits=16), 128, 224, 1000),
 ]
 MODES = {'train': (False, True), 'frozen_fused': (True, True), 'frozen_eager': (True, False)}   # (frozen, FUSE_UNITS)
-BN_BWD = ('lbt_bn_bwd_quant_stats', 'lbt_bn_bwd_apply', 'lbt_bn_bwd_fused', 'lbt_bn_bwd_running')
+BN_BWD = ('lbt_bn_bwd_quant_stats', 'lbt_bn_bwd_apply', 'lbt_bn_bwd_running')
 
 
 def set_mode(tr, mode):

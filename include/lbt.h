@@ -56,12 +56,7 @@ enum lbt_mant_kind {
   /* 3-channel signed 9-bit input (the image fed to a first Conv2d_q, bits+1 = 9): every pixel becomes 16
    * s8 bytes {hi0,hi1,hi2, hi0,hi1,hi2, lo0,lo1,lo2, 0 x 7} with k = 2*hi + lo, i.e. a 16-channel s8 NHWC
    * tensor the implicit-GEMM kernels consume against weights packed {W, W, W, 0}.  n_inner % 3 == 0. */
-  LBT_MANT_S9C3 = 4,
-  /* OR-able flag on the FILTER kind of the convolution entry points: the packed filter was written at least two launches
-   * before this call on the same stream (e.g. by lbt_param_prep at the start of the step), so the kernel may start copying
-   * it before it waits for its immediate predecessor (programmatic dependent launch).  Never set it for a filter produced by
-   * the launch right before the call. */
-  LBT_MANT_PREPARED = 0x100
+  LBT_MANT_S9C3 = 4
 };
 
 /* Per-quantiser overflow statistics block: uint64_t[4] on the device. */
@@ -484,28 +479,6 @@ int lbt_bn_bwd_quant_stats(const float* g, const float* out, int relu, const int
                            uint64_t* counters_g1, uint64_t seed, const uint64_t* dev_step, float* d_add,
                            void* kg1, int64_t* sums, int stats_minmax, int kg1_kind, void* stream);
 /*
- * bwd 1 behind a max-pool (the ImageNet stems: conv -> BN -> ReLU -> 3x3/2 max-pool, models.py layer lists with MaxPool_q,
- * dfxp:993-1006): `g_pooled` [n_outer, OH, OW, C] is the gradient w.r.t. the POOLED tensor and `pool->idx` the winning tap
- * lbt_maxpool_fwd recorded for every pooled element; the pool's backward (each pixel collects the gradient of every window
- * it won, windows visited in (oh, ow) order as lbt_maxpool_bwd does) runs in this kernel's load stage, so the dense fp32
- * gradient of the un-pooled tensor (4 B written + 4 B read per element) never exists.  Bit-identical to
- * lbt_maxpool_bwd followed by lbt_bn_bwd_quant_stats.  Windows with k <= 2 * s, C % 4 == 0, relu in {0, 1}.
- * n_inner = pool->H * pool->W * C.
- */
-typedef struct lbt_pool_geom {
-  const uint8_t* idx;                 /* [n_outer, OH, OW, C] winning tap (r * k + s) */
-  int32_t H, W;                       /* un-pooled grid */
-  int32_t k, s, pad_top, pad_left;    /* window, stride, TF 'SAME' padding before */
-  int32_t OH, OW;                     /* pooled grid */
-} lbt_pool_geom;
-int lbt_bn_bwd_quant_stats_pooled(const float* g_pooled, const lbt_pool_geom* pool, int relu, const int8_t* k2,
-                                  const int8_t* k1, size_t n_outer, size_t n_inner, int C, int bits2, const int32_t* ib2,
-                                  const float* gamma_q, const float* beta_q, int bits_g2, const int32_t* ib_g2,
-                                  const float* noise_g2, uint64_t offset_g2, uint64_t* counters_g2, int bits_g1,
-                                  const int32_t* ib_g1, const float* noise_g1, uint64_t offset_g1,
-                                  uint64_t* counters_g1, uint64_t seed, const uint64_t* dev_step, void* kg1,
-                                  int64_t* sums, int stats_minmax, int kg1_kind, void* stream);
-/*
  * bwd 2: dx = (gq1 - mean(gq1) - xhat * mean(gq1 * xhat)) / sqrt(var + eps), the batch-norm VJP that
  * tf.gradients(y, X, gradq) yields for dfxp:616 (dfxp:623), from kg1, k1 and the two sum buffers.
  * q_grad != NULL: dx is quantised on the spot with the PRODUCING convolution's gradient quantiser (`gradq`,
@@ -543,37 +516,6 @@ int lbt_bn_bwd_running(const float* g, const float* out, int relu, const int8_t*
                        uint64_t seed, const uint64_t* dev_step, float* d_add, int64_t* sums, float* dx,
                        const lbt_qsite* q_grad, int8_t* g_mant, uint8_t* g_mant_lo, int stats_minmax, int grad_kind,
                        void* stream);
-
-/*
- * lbt_bn_bwd_quant_stats + lbt_bn_bwd_apply in ONE launch, for tensors small enough that the whole tensor is one wave of
- * resident CTAs (<= 16 batch rows per CTA): the mantissas the second pass needs stay in shared memory and the CTAs meet
- * at a grid-wide barrier (`barrier`: one zeroed uint64 on the device).  Same arithmetic, bit-identical results.  Returns
- * LBT_EUNSUPPORTED when the tensor does not fit that shape — the caller then runs the two passes as separate launches.
- */
-typedef struct lbt_bn_bwd_args {
-  const float* g;          /* gradient w.r.t. the module output [n_outer, n_inner] */
-  const float* out;        /* module output (relu == 2), or NULL */
-  const int8_t* k2;
-  const int8_t* k1;
-  uint64_t n_outer, n_inner;
-  int32_t C, relu;
-  int32_t bits2, bits1;    /* Rescale_q X bits / Normalization_q X bits */
-  const int32_t* ib2;
-  const int32_t* ib1;
-  const float* gamma_q;
-  const float* beta_q;
-  lbt_qsite q_g2, q_g1;    /* Rescale_q / Normalization_q gradient quantisers */
-  float* d_add;            /* optional */
-  int64_t* bwd_sums;       /* [4*C], zeroed */
-  const int64_t* fwd_sums; /* [2*C] */
-  float eps;
-  int32_t has_q_grad;
-  lbt_qsite q_grad;        /* the producing convolution's gradient quantiser (has_q_grad != 0) */
-  float* dx;               /* optional when has_q_grad */
-  int8_t* g_mant;
-  uint64_t* barrier;
-} lbt_bn_bwd_args;
-int lbt_bn_bwd_fused(const lbt_bn_bwd_args* args, void* stream);
 
 /*
  * tf.nn.max_pool on an NHWC fp32 tensor (`MaxPool_q`, dynamic_fixed_point.py:993-1006): 'SAME' padding ignores
@@ -675,31 +617,6 @@ int lbt_augment_batch(const uint8_t* src, const double* mean, const int64_t* ind
 int lbt_quantize_residual(const float* grad, size_t n_grad_rows, float* buffer, size_t n_outer, size_t n_inner, int bits,
                           int32_t* integer_bits, int mode, const float* noise, uint64_t seed, uint64_t offset,
                           const uint64_t* dev_step, float* out, uint64_t* counters, void* stream);
-
-/*
- * Stride-1 input gradient of a convolution whose INPUT was produced by a fused batch-norm unit, with that batch-norm's
- * backward pass 1 (lbt_bn_bwd_quant_stats) run in the epilogue: the fp32 gradient dX = conv(g, rot180(W)) is never written;
- * instead, per element, the ReLU mask is recomputed from k2 (relu = 1) or skipped (0), kg2 = Q_g2(dX) (dfxp:687),
- * dx2 = gq2 * gamma_q (:691), kg1 = Q_g1(dx2) (:621) is stored, and sums[0..C) += kg2, [C..2C) += kg2*k2, [2C..3C) += kg1,
- * [3C..4C) += kg1*k1 (C = Cout of this call = the batch-norm's channels; caller-zeroed).  Same quantiser ids, noise streams,
- * counters and arithmetic as the two separate launches: bit-identical.  g[N,H,W,C] gradient mantissas of the convolution's
- * output; wp: filter packed for the transposed convolution as for lbt_conv_i8_fprop; OH x OW: the convolution's input grid.
- * Narrow-channel shapes only (LBT_EUNSUPPORTED otherwise: run lbt_conv_i8_fprop + lbt_bn_bwd_quant_stats).
- */
-typedef struct lbt_bn_bwd_link {
-  lbt_qsite q_g2, q_g1;      /* Rescale_q / Normalization_q gradient quantisers */
-  int32_t bits2, relu;       /* Rescale_q input quantiser bits; ReLU: 0 none, 1 recomputed from k2 */
-  const int32_t* ib2;
-  const float* gamma_q;      /* [C] fake-quantised gamma / beta (16-byte aligned) */
-  const float* beta_q;
-  const int8_t* k2;          /* [N*OH*OW, C] saved forward mantissas */
-  const int8_t* k1;
-  int8_t* kg1;               /* [N*OH*OW, C] out */
-  int64_t* sums;             /* [4*C] out */
-} lbt_bn_bwd_link;
-int lbt_conv_i8_dgrad_bn(const void* g, int g_kind, int N, int H, int W, int C, const void* wp, int w_kind, size_t ldw, int Cout,
-                         int kh, int kw, int pad_top, int pad_left, int OH, int OW, const int32_t* ib_g, const int32_t* ib_w,
-                         int exp_const, const lbt_bn_bwd_link* link, void* stream);
 
 /*
  * Input gradient of a STRIDED convolution whose gathered tensor (the output gradient g[N,OH,OW,Cout]) is wide

@@ -50,7 +50,6 @@ SIGNATURES = {
     'lbt_split_s16': (c_int, [c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),
     'lbt_transpose_i8': (c_int, [c_void_p, c_size_t, c_size_t, c_size_t, c_void_p, c_size_t, c_void_p]),
     'lbt_colsum_i': (c_int, [c_void_p, c_int, c_size_t, c_size_t, c_void_p, c_void_p]),
-    'lbt_bn_bwd_fused': (c_int, [c_void_p, c_void_p]),
     'lbt_maxpool_fwd': (c_int, [c_void_p] + [c_int] * 10 + [c_void_p, c_void_p, c_void_p]),
     'lbt_maxpool_bwd': (c_int, [c_void_p, c_void_p] + [c_int] * 10 + [c_void_p, c_void_p]),
     'lbt_avgpool_fwd': (c_int, [c_void_p] + [c_int] * 8 + [c_void_p, c_void_p]),
@@ -95,10 +94,6 @@ SIGNATURES = {
                                        c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_u64, c_void_p, c_int,
                                        c_void_p, c_void_p, c_u64, c_void_p, c_u64, c_void_p, c_void_p, c_void_p,
                                        c_void_p, c_int, c_int, c_void_p]),
-    'lbt_bn_bwd_quant_stats_pooled': (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_size_t, c_size_t, c_int, c_int,
-                                              c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_u64, c_void_p, c_int,
-                                              c_void_p, c_void_p, c_u64, c_void_p, c_u64, c_void_p, c_void_p,
-                                              c_void_p, c_int, c_int, c_void_p]),
     'lbt_bn_bwd_apply': (c_int, [c_void_p, c_void_p, c_size_t, c_size_t, c_int, c_int, c_void_p, c_void_p, c_float,
                                  c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     # g, out, relu, k2, n_outer, n_inner, C, bits2, ib2, gamma_q, beta_q, run_var, eps, bits_g2, ib_g2, noise_g2, offset_g2,
@@ -121,8 +116,6 @@ SIGNATURES = {
     'lbt_dp_export': (c_int, [c_void_p, c_void_p, c_void_p]),
     'lbt_dp_open': (c_int, [c_void_p, c_void_p]),
     'lbt_dp_close': (c_int, [c_void_p]),
-    'lbt_conv_i8_dgrad_bn': (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_int, c_size_t] + [c_int] * 7 +
-                             [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     'lbt_quantize_residual': (c_int, [c_void_p, c_size_t, c_void_p, c_size_t, c_size_t, c_int, c_void_p, c_int, c_void_p, c_u64,
                                       c_u64, c_void_p, c_void_p, c_void_p, c_void_p]),
     'lbt_augment_batch': (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_u64, c_u64,
@@ -148,7 +141,6 @@ _INTERNAL = {
     'lbt_dp_emulate_scratch_bytes': (c_size_t, [c_int]),
     'lbt_dp_step_emulate': (c_int, [c_int, c_void_p, c_void_p, c_size_t, c_float, c_void_p, c_float, c_int, c_void_p, c_void_p,
                                     c_void_p, c_size_t, c_void_p, c_void_p, c_void_p]),
-    'lbt_bn_debug_error': (c_int, []),
 }
 
 
@@ -166,28 +158,6 @@ class QSiteStruct(ctypes.Structure):
     """lbt_qsite (include/lbt.h): one quantiser call site as the fused kernels see it."""
     _fields_ = [('bits', ctypes.c_int32), ('stats_minmax', ctypes.c_int32), ('ib', c_void_p), ('noise', c_void_p),
                 ('seed', c_u64), ('offset', c_u64), ('dev_step', c_void_p), ('counters', c_void_p)]
-
-
-class PoolGeom(ctypes.Structure):
-    """lbt_pool_geom (include/lbt.h): a max-pool whose backward runs inside lbt_bn_bwd_quant_stats_pooled."""
-    _fields_ = [('idx', c_void_p), ('H', ctypes.c_int32), ('W', ctypes.c_int32), ('k', ctypes.c_int32), ('s', ctypes.c_int32),
-                ('pad_top', ctypes.c_int32), ('pad_left', ctypes.c_int32), ('OH', ctypes.c_int32), ('OW', ctypes.c_int32)]
-
-
-class BnBwdLink(ctypes.Structure):
-    """lbt_bn_bwd_link (include/lbt.h)."""
-    _fields_ = [('q_g2', QSiteStruct), ('q_g1', QSiteStruct), ('bits2', ctypes.c_int32), ('relu', ctypes.c_int32), ('ib2', c_void_p),
-                ('gamma_q', c_void_p), ('beta_q', c_void_p), ('k2', c_void_p), ('k1', c_void_p), ('kg1', c_void_p), ('sums', c_void_p)]
-
-
-class BnBwdArgs(ctypes.Structure):
-    """lbt_bn_bwd_args (include/lbt.h)."""
-    _fields_ = [('g', c_void_p), ('out', c_void_p), ('k2', c_void_p), ('k1', c_void_p), ('n_outer', c_u64), ('n_inner', c_u64),
-                ('C', ctypes.c_int32), ('relu', ctypes.c_int32), ('bits2', ctypes.c_int32), ('bits1', ctypes.c_int32),
-                ('ib2', c_void_p), ('ib1', c_void_p), ('gamma_q', c_void_p), ('beta_q', c_void_p), ('q_g2', QSiteStruct),
-                ('q_g1', QSiteStruct), ('d_add', c_void_p), ('bwd_sums', c_void_p), ('fwd_sums', c_void_p), ('eps', c_float),
-                ('has_q_grad', ctypes.c_int32), ('q_grad', QSiteStruct), ('dx', c_void_p), ('g_mant', c_void_p),
-                ('barrier', c_void_p)]
 
 
 DP_MAX_WORLD, DP_PAD_WORDS, DP_PAD_ERROR, DP_HANDLE_BYTES = 8, 32, 18, 64

@@ -767,18 +767,13 @@ struct Bwd1Params {
   float* d_add;         // optional: gradient w.r.t. the fused shortcut input (= masked g)
   void* kg1;            // s8, or s16 in the WIDE instantiation
   long long* sums;      // [4*C]: sum kg2, sum kg2*k2, sum kg1, sum kg1*k1
-  // POOL instantiation: `g` is the gradient of a max-pool of the module output, [n_outer, pOH, pOW, C]; the pool's backward
-  // (a gather over the <= 2 x 2 windows that cover a pixel, lbt_maxpool_bwd) runs in this kernel's load stage
-  const uint8_t* pidx;  // winning tap of every pooled element
-  int pW, pk, ps, ppt, ppl, pOH, pOW;
-  FastDiv d_c4, d_pW, d_ps;
 };
 
 // WIDE: a gradient quantiser wider than 8 bits — kg1 is stored as s16 and the per-thread partial sums are 64-bit
 // (a 16-bit mantissa times an 8-bit one, summed down 4096 rows, does not fit 32).  MM: min/max statistics for both sites.
 // RELU: 0 none, 1 mask recomputed from k2, 2 mask from `out`.  ~31 full-rate instructions per element, no conversions;
 // folded constants (exact, powers of two):  RN(xq2 * g) = RN(k2 * (g / m2));  dx2 * mg1 = RN(kg2 * (g * mg1 / mg2)).
-template <bool WIDE, bool MM, int RELU, bool POOL = false>
+template <bool WIDE, bool MM, int RELU>
 __global__ void __launch_bounds__(kThreads, LBT_BN_BWD1_CTAS) bn_bwd1_kernel(const Bwd1Params p) {
   extern __shared__ unsigned long long s_acc[];
   __shared__ uint32_t s_red[16];
@@ -812,30 +807,6 @@ __global__ void __launch_bounds__(kThreads, LBT_BN_BWD1_CTAS) bn_bwd1_kernel(con
         b[j] = __ldg(p.bq + c0 + j);
       }
       const uint32_t r0 = rg * p.t.rows_per_group, r1 = min(r0 + p.t.rows_per_group, (uint32_t)p.t.n_outer);   // rows: 32-bit (make_tiling)
-      // POOL: the <= 2 x 2 pooling windows over this thread's pixel — the same for every batch row (tf.nn.max_pool's
-      // gradient, dfxp:993-1006: a pixel receives the gradient of each window it won; lbt_maxpool_bwd's gather and order)
-      uint32_t poff[4] = {0u, 0u, 0u, 0u};
-      uint32_t ptap[4] = {0u, 0u, 0u, 0u};
-      bool pok[4] = {false, false, false, false};
-      size_t pimg = 0;
-      if (POOL) {
-        const uint32_t pix = fastdiv(v, p.d_c4), cg = v - pix * p.d_c4.d;
-        const uint32_t ih = fastdiv(pix, p.d_pW), iw = pix - ih * (uint32_t)p.pW;
-        const int th = (int)ih + p.ppt, tw = (int)iw + p.ppl;
-        const int oh_lo = th - p.pk + 1 <= 0 ? 0 : (int)fastdiv((uint32_t)(th - p.pk + p.ps), p.d_ps);
-        const int ow_lo = tw - p.pk + 1 <= 0 ? 0 : (int)fastdiv((uint32_t)(tw - p.pk + p.ps), p.d_ps);
-        const int oh_hi = min(p.pOH - 1, (int)fastdiv((uint32_t)th, p.d_ps)), ow_hi = min(p.pOW - 1, (int)fastdiv((uint32_t)tw, p.d_ps));
-#pragma unroll
-        for (int a = 0; a < 2; ++a)
-#pragma unroll
-          for (int b2 = 0; b2 < 2; ++b2) {
-            const int oh = oh_lo + a, ow = ow_lo + b2;
-            pok[2 * a + b2] = oh <= oh_hi && ow <= ow_hi;
-            ptap[2 * a + b2] = (uint32_t)((th - oh * p.ps) * p.pk + (tw - ow * p.ps)) & 0xffu;
-            poff[2 * a + b2] = pok[2 * a + b2] ? ((uint32_t)(oh * p.pOW + ow) * (uint32_t)C + 4u * cg) : 0u;
-          }
-        pimg = (size_t)p.pOH * p.pOW * C;
-      }
       for (uint32_t r = r0; r < r1; r += kRows) {
         float4 gv[kRows], ov[kRows];
         uint32_t w2[kRows], w1[kRows];
@@ -843,29 +814,7 @@ __global__ void __launch_bounds__(kThreads, LBT_BN_BWD1_CTAS) bn_bwd1_kernel(con
         for (int i = 0; i < kRows; ++i)
           if (r + i < r1) {
             const size_t idx = 4 * (size_t)((r + i) * p.t.n_vec + v);   // element / 4 fits 32 bits
-            if (POOL) {
-              const size_t base = (size_t)(r + i) * pimg;
-              float4 gw[4];
-              uint32_t iw4[4];
-#pragma unroll
-              for (int q = 0; q < 4; ++q)
-                if (pok[q]) {
-                  gw[q] = __ldg(reinterpret_cast<const float4*>(p.g + base + poff[q]));
-                  iw4[q] = __ldg(reinterpret_cast<const uint32_t*>(p.pidx + base + poff[q]));
-                }
-              float4 a4 = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-              for (int q = 0; q < 4; ++q)       // (oh, ow) ascending: lbt_maxpool_bwd's order of additions
-                if (pok[q]) {
-                  if ((iw4[q] & 0xffu) == ptap[q]) a4.x += gw[q].x;
-                  if (((iw4[q] >> 8) & 0xffu) == ptap[q]) a4.y += gw[q].y;
-                  if (((iw4[q] >> 16) & 0xffu) == ptap[q]) a4.z += gw[q].z;
-                  if ((iw4[q] >> 24) == ptap[q]) a4.w += gw[q].w;
-                }
-              gv[i] = a4;
-            } else {
-              gv[i] = __ldcs(reinterpret_cast<const float4*>(p.g + idx));
-            }
+            gv[i] = __ldcs(reinterpret_cast<const float4*>(p.g + idx));
             w2[i] = __ldcs(reinterpret_cast<const uint32_t*>(p.k2 + idx));
             w1[i] = __ldcs(reinterpret_cast<const uint32_t*>(p.k1 + idx));
             if (RELU == 2) ov[i] = __ldcs(reinterpret_cast<const float4*>(p.out + idx));
@@ -874,17 +823,7 @@ __global__ void __launch_bounds__(kThreads, LBT_BN_BWD1_CTAS) bn_bwd1_kernel(con
         for (int i = 0; i < kRows; ++i)
           if (r + kRows + i < r1) {
             const size_t idx = 4 * (size_t)((r + kRows + i) * p.t.n_vec + v);   // element / 4 fits 32 bits
-            if (POOL) {
-              const size_t base = (size_t)(r + kRows + i) * pimg;
-#pragma unroll
-              for (int q = 0; q < 4; ++q)
-                if (pok[q]) {
-                  prefetch_l1(p.g + base + poff[q]);
-                  prefetch_l1(p.pidx + base + poff[q]);
-                }
-            } else {
-              prefetch_l1(p.g + idx);
-            }
+            prefetch_l1(p.g + idx);
             prefetch_l1(p.k2 + idx);
             prefetch_l1(p.k1 + idx);
             if (RELU == 2) prefetch_l1(p.out + idx);
@@ -1114,213 +1053,6 @@ __global__ void __launch_bounds__(kThreads) bn_bwd2_kernel(const Bwd2Params p) {
     publish_counters(p.qg.counters, n1, n2, p.t.n_outer * p.t.n_inner, s_red);
   }
   bn_stamp(4);
-}
-
-// ------------------------------------------------------------------------------------------------
-// bwd 1 + bwd 2 in ONE launch for tensors that fit one wave of resident CTAs (every tensor of a CIFAR-size step):
-// pass 1 as above, but the mantissas the second pass needs (kg1, k1) stay in shared memory; the CTAs then meet at a
-// grid-wide barrier (one int64 word from the step's zeroed arena: all CTAs are co-resident by construction) and run
-// pass 2 from shared memory.  Saves a launch + dependent-launch gap, the kg1 round trip through HBM and a prologue.
-// ------------------------------------------------------------------------------------------------
-constexpr int kMaxSavedRows = 16;
-
-struct BwdFusedParams {
-  Bwd1Params a;
-  Bwd2Params b;               // b.kg1 / b.k1 unused (shared memory)
-  unsigned long long* bar;    // grid barrier word, zero at launch
-};
-
-__device__ int g_bn_error = 0;
-
-__global__ void __launch_bounds__(kThreads, 2) bn_bwd_fused_kernel(const BwdFusedParams q) {
-  extern __shared__ unsigned long long s_dyn[];
-  __shared__ uint32_t s_red[16];
-  const Bwd1Params& p = q.a;
-  const Bwd2Params& p2 = q.b;
-  const int C = p.t.C;
-  unsigned long long* s_acc = s_dyn;                                    // [4*C] (pass 1), then float s_par[4*C]
-  uint2* s_save = reinterpret_cast<uint2*>(s_dyn + 4 * C);              // [rows_per_group][kThreads]: {kg1 word, k1 word}
-  pdl_trigger();
-  pdl_wait();
-  const QC c2 = make_qc(p.bits2, __ldg(p.ib2));
-  const QC cg2 = make_qc(p.qg2.bits, __ldg(p.qg2.ib));
-  const QC cg1 = make_qc(p.qg1.bits, __ldg(p.qg1.ib));
-  const QC c1 = make_qc(p2.bits1, __ldg(p2.ib1));
-  const bool gq_on = p2.qg.bits != 0;
-  QC cq = cg1;
-  uint64_t offq = 0;
-  if (gq_on) {
-    cq = make_qc(p2.qg.bits, __ldg(p2.qg.ib));
-    offq = site_offset(p2.qg);
-  }
-  const uint64_t off2 = site_offset(p.qg2), off1 = site_offset(p.qg1);
-  uint32_t a1 = 0, a2 = 0, b1 = 0, b2 = 0;
-  float amx = -INFINITY, amn = INFINITY, bmx = -INFINITY, bmn = INFINITY;
-  const bool mm2 = p.qg2.minmax != 0, mm1 = p.qg1.minmax != 0;
-  Acc<4> acc;
-  acc.zero();
-  const uint64_t tile = blockIdx.x;   // exactly one tile per CTA
-  const uint32_t rg = (uint32_t)(tile / p.t.chunks), chk = (uint32_t)(tile % p.t.chunks);
-  const uint32_t v = chk * kThreads + threadIdx.x;
-  const bool active = v < p.t.n_vec;
-  const int c0 = active ? (int)((4ull * v) % (uint64_t)C) : 0;
-  const uint32_t r0 = rg * p.t.rows_per_group, r1 = min(r0 + p.t.rows_per_group, (uint32_t)p.t.n_outer);   // rows: 32-bit (make_tiling)
-  if (active) {
-    const float4 u2v = site_noise(p.qg2, v, off2), u1v = site_noise(p.qg1, v, off1);
-    const float u2[4] = {u2v.x, u2v.y, u2v.z, u2v.w}, u1[4] = {u1v.x, u1v.y, u1v.z, u1v.w};
-    float g[4], b[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      g[j] = __ldg(p.gq + c0 + j);
-      b[j] = __ldg(p.bq + c0 + j);
-    }
-    for (uint32_t r = r0; r < r1; r += kRows) {
-      float4 gv[kRows], ov[kRows];
-      uint32_t w2[kRows], w1[kRows];
-#pragma unroll
-      for (int i = 0; i < kRows; ++i)
-        if (r + i < r1) {
-          const size_t idx = 4 * (size_t)((r + i) * p.t.n_vec + v);   // element / 4 fits 32 bits
-          gv[i] = __ldcs(reinterpret_cast<const float4*>(p.g + idx));
-          w2[i] = __ldcs(reinterpret_cast<const uint32_t*>(p.k2 + idx));
-          w1[i] = __ldcs(reinterpret_cast<const uint32_t*>(p.k1 + idx));
-          if (p.relu == 2) ov[i] = __ldcs(reinterpret_cast<const float4*>(p.out + idx));
-        }
-#pragma unroll
-      for (int i = 0; i < kRows; ++i)
-        if (r + kRows + i < r1) {
-          const size_t idx = 4 * (size_t)((r + kRows + i) * p.t.n_vec + v);   // element / 4 fits 32 bits
-          prefetch_l1(p.g + idx);
-          prefetch_l1(p.k2 + idx);
-          prefetch_l1(p.k1 + idx);
-          if (p.relu == 2) prefetch_l1(p.out + idx);
-        }
-#pragma unroll
-      for (int i = 0; i < kRows; ++i)
-        if (r + i < r1) {
-          const size_t idx = 4 * (size_t)((r + i) * p.t.n_vec + v);   // element / 4 fits 32 bits
-          int k2[4], k1[4];
-          unpack4(w2[i], k2);
-          unpack4(w1[i], k1);
-          const float gin[4] = {gv[i].x, gv[i].y, gv[i].z, gv[i].w};
-          const float oin[4] = {ov[i].x, ov[i].y, ov[i].z, ov[i].w};
-          float gm[4], kq1[4];
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            float gj = gin[j];
-            if (p.relu == 1) {
-              const float y2 = __fadd_rn(__fmul_rn(__int2float_rn(k2[j]) * c2.inv_m, g[j]), b[j]);
-              if (!(y2 > 0.0f)) gj = 0.0f;
-            } else if (p.relu == 2) {
-              if (!(oin[j] > 0.0f)) gj = 0.0f;
-            }
-            gm[j] = gj;
-            const float kg2 = mm2 ? squant_mm(gj, u2[j], cg2, amx, amn) : squant(gj, u2[j], cg2, a1, a2);   // dfxp:687
-            const int kg2i = __float2int_rn(kg2);
-            acc.s[0][j] += kg2i;
-            acc.s[1][j] += kg2i * k2[j];
-            const float dx2 = __fmul_rn(kg2 * cg2.inv_m, g[j]);                  // dfxp:691
-            kq1[j] = mm1 ? squant_mm(dx2, u1[j], cg1, bmx, bmn) : squant(dx2, u1[j], cg1, b1, b2);         // dfxp:621
-            const int kg1i = __float2int_rn(kq1[j]);
-            acc.s[2][j] += kg1i;
-            acc.s[3][j] += kg1i * k1[j];
-          }
-          if (p.d_add) *reinterpret_cast<float4*>(p.d_add + idx) = make_float4(gm[0], gm[1], gm[2], gm[3]);
-          s_save[(r + i - r0) * kThreads + threadIdx.x] = make_uint2(pack4(kq1), w1[i]);
-        }
-    }
-  }
-  flush_block(acc, p.sums, C, s_acc);
-  const size_t numel = p.t.n_outer * p.t.n_inner;
-  if (mm2) mm_to_counts(cg2, amx, amn, a1, a2);
-  if (mm1) mm_to_counts(cg1, bmx, bmn, b1, b2);
-  publish_counters(p.qg2.counters, a1, a2, numel, s_red);
-  publish_counters(p.qg1.counters, b1, b2, numel, s_red);
-
-  // ---- grid-wide barrier: every CTA's sums are in global memory before anyone reads them ----
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    __threadfence();
-    atomicAdd(q.bar, 1ull);
-    long long t0 = 0;
-    uint32_t spins = 0;
-    while (*reinterpret_cast<volatile unsigned long long*>(q.bar) < (unsigned long long)gridDim.x) {
-      if ((++spins & 0xff) == 0) {
-        const long long now = clock64();
-        if (t0 == 0) t0 = now;
-        if (now - t0 > 4000000000ll) {  // ~2 s: never hang the GPU on a protocol bug
-          atomicExch(&g_bn_error, 1);
-          break;
-        }
-      }
-    }
-    __threadfence();
-  }
-  __syncthreads();
-
-  // ---- pass 2 from shared memory ----
-  float* s_par = reinterpret_cast<float*>(s_dyn);
-  const DivN n = make_divn((unsigned long long)(p.t.n_outer * (p.t.n_inner / C)));
-  for (int ch = threadIdx.x; ch < C; ch += kThreads) {
-    float mean, var;
-    moments(p2.fsums, C, ch, n, c1.inv_m, mean, var);
-    const float den = __fsqrt_rn(__fadd_rn(var, p2.eps));
-    const double sg = (double)__ldcg(p.sums + 2 * C + ch) * (double)cg1.inv_m;
-    const double sgx = (double)__ldcg(p.sums + 3 * C + ch) * (double)cg1.inv_m * (double)c1.inv_m;
-    const double mg = div_n(sg, n);
-    const double mgx = div_n(__ddiv_rn(__dsub_rn(sgx, __dmul_rn((double)mean, sg)), (double)den), n);
-    s_par[ch] = mean;
-    s_par[C + ch] = den;
-    s_par[2 * C + ch] = (float)mg;
-    s_par[3 * C + ch] = (float)mgx;
-  }
-  __syncthreads();
-  uint32_t n1 = 0, n2 = 0;
-  float mx = -INFINITY, mn = INFINITY;
-  const bool mmq = p2.qg.minmax != 0;
-  if (active) {
-    float mean[4], den[4], mg[4], mgx[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      mean[j] = s_par[c0 + j];
-      den[j] = s_par[C + c0 + j];
-      mg[j] = s_par[2 * C + c0 + j];
-      mgx[j] = s_par[3 * C + c0 + j];
-    }
-    float rden[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) rden[j] = __frcp_rn(den[j]);
-    float uq[4] = {0.f, 0.f, 0.f, 0.f};
-    if (gq_on) {
-      const float4 t = site_noise(p2.qg, v, offq);
-      uq[0] = t.x; uq[1] = t.y; uq[2] = t.z; uq[3] = t.w;
-    }
-    for (size_t r = r0; r < r1; ++r) {
-      const size_t idx = r * p.t.n_inner + 4 * (size_t)v;
-      const uint2 sv = s_save[(r - r0) * kThreads + threadIdx.x];
-      int kg[4], k1[4];
-      unpack4(sv.x, kg);
-      unpack4(sv.y, k1);
-      float o[4];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float gqv = __int2float_rn(kg[j]) * cg1.inv_m;
-        const float xhat = fdiv_by(__fsub_rn(__int2float_rn(k1[j]) * c1.inv_m, mean[j]), den[j], rden[j]);
-        o[j] = fdiv_by(__fsub_rn(__fsub_rn(gqv, mg[j]), __fmul_rn(xhat, mgx[j])), den[j], rden[j]);
-      }
-      if (p2.dx) *reinterpret_cast<float4*>(p2.dx + idx) = make_float4(o[0], o[1], o[2], o[3]);
-      if (gq_on) {
-        float kq[4];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) kq[j] = mmq ? squant_mm(o[j], uq[j], cq, mx, mn) : squant(o[j], uq[j], cq, n1, n2);
-        *reinterpret_cast<uint32_t*>(p2.g_mant + idx) = pack4(kq);
-      }
-    }
-  }
-  if (gq_on) {
-    if (mmq) mm_to_counts(cq, mx, mn, n1, n2);
-    publish_counters(p2.qg.counters, n1, n2, numel, s_red);
-  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1814,23 +1546,14 @@ extern "C" int lbt_bn_fwd_apply_running_pooled(const int8_t* k1, size_t n_outer,
                                  stream, true);
 }
 
-static int bn_bwd1_run(const float* g, const float* out, int relu, const int8_t* k2, const int8_t* k1,
-                       size_t n_outer, size_t n_inner, int C, int bits2, const int32_t* ib2,
-                       const float* gamma_q, const float* beta_q, int bits_g2, const int32_t* ib_g2,
-                       const float* noise_g2, uint64_t offset_g2, uint64_t* counters_g2, int bits_g1,
-                       const int32_t* ib_g1, const float* noise_g1, uint64_t offset_g1,
-                       uint64_t* counters_g1, uint64_t seed, const uint64_t* dev_step, float* d_add,
-                       void* kg1, int64_t* sums, int stats_minmax, int kg1_kind, const lbt_pool_geom* pool, void* stream) {
+extern "C" int lbt_bn_bwd_quant_stats(const float* g, const float* out, int relu, const int8_t* k2, const int8_t* k1,
+                                      size_t n_outer, size_t n_inner, int C, int bits2, const int32_t* ib2,
+                                      const float* gamma_q, const float* beta_q, int bits_g2, const int32_t* ib_g2,
+                                      const float* noise_g2, uint64_t offset_g2, uint64_t* counters_g2, int bits_g1,
+                                      const int32_t* ib_g1, const float* noise_g1, uint64_t offset_g1,
+                                      uint64_t* counters_g1, uint64_t seed, const uint64_t* dev_step, float* d_add,
+                                      void* kg1, int64_t* sums, int stats_minmax, int kg1_kind, void* stream) {
   if (!g || !k2 || !k1 || !ib2 || !gamma_q || !beta_q || !ib_g2 || !ib_g1 || !kg1 || !sums) return LBT_EINVAL;
-  if (pool) {
-    if (!pool->idx || pool->H <= 0 || pool->W <= 0 || pool->k <= 0 || pool->s <= 0 || pool->OH <= 0 || pool->OW <= 0 ||
-        pool->pad_top < 0 || pool->pad_left < 0)
-      return LBT_EINVAL;
-    // <= 2 x 2 windows per pixel, 4 channels per thread, no shortcut sum / saved-output mask in front of the pool
-    if (pool->k > 2 * pool->s || pool->k > 15 || (C & 3) || relu == 2 || d_add) return LBT_EUNSUPPORTED;
-    if (n_inner != (size_t)pool->H * pool->W * C) return LBT_EINVAL;
-    if ((size_t)pool->OH * pool->OW * C >= (1ull << 31) || (reinterpret_cast<uintptr_t>(pool->idx) & 3)) return LBT_EUNSUPPORTED;
-  }
   if (relu < 0 || relu > 2 || (relu == 2 && !out)) return LBT_EINVAL;
   if (kg1_kind != LBT_MANT_S8 && kg1_kind != LBT_MANT_S16) return LBT_EINVAL;
   const bool wide = kg1_kind == LBT_MANT_S16;
@@ -1849,11 +1572,8 @@ static int bn_bwd1_run(const float* g, const float* out, int relu, const int8_t*
     const bool mm = stats_minmax != 0;
 #define LBT_BWD1(W, M)                                                                                     \
   (relu == 0 ? bn_bwd1_kernel<W, M, 0> : (relu == 1 ? bn_bwd1_kernel<W, M, 1> : bn_bwd1_kernel<W, M, 2>))
-#define LBT_BWD1P(W, M) (relu == 0 ? bn_bwd1_kernel<W, M, 0, true> : bn_bwd1_kernel<W, M, 1, true>)
-    if (pool) kern = wide ? (mm ? LBT_BWD1P(true, true) : LBT_BWD1P(true, false)) : (mm ? LBT_BWD1P(false, true) : LBT_BWD1P(false, false));
-    else kern = wide ? (mm ? LBT_BWD1(true, true) : LBT_BWD1(true, false)) : (mm ? LBT_BWD1(false, true) : LBT_BWD1(false, false));
+    kern = wide ? (mm ? LBT_BWD1(true, true) : LBT_BWD1(true, false)) : (mm ? LBT_BWD1(false, true) : LBT_BWD1(false, false));
 #undef LBT_BWD1
-#undef LBT_BWD1P
   }
   int rc = make_tiling(p.t, n_outer, n_inner, C, grid, ctas_per_sm(kern, (size_t)4 * C * 8));
   if (rc) return rc;
@@ -1871,48 +1591,10 @@ static int bn_bwd1_run(const float* g, const float* out, int relu, const int8_t*
   p.d_add = d_add;
   p.kg1 = kg1;
   p.sums = reinterpret_cast<long long*>(sums);
-  if (pool) {
-    p.pidx = pool->idx;
-    p.pW = pool->W;
-    p.pk = pool->k;
-    p.ps = pool->s;
-    p.ppt = pool->pad_top;
-    p.ppl = pool->pad_left;
-    p.pOH = pool->OH;
-    p.pOW = pool->OW;
-    p.d_c4 = make_fastdiv((uint32_t)C / 4);
-    p.d_pW = make_fastdiv((uint32_t)pool->W);
-    p.d_ps = make_fastdiv((uint32_t)pool->s);
-  }
   const size_t smem = (size_t)4 * C * 8;
   if ((rc = set_smem(kern, smem))) return rc;
   launch_pdl(kern, grid, kThreads, smem, reinterpret_cast<cudaStream_t>(stream), p);
   return check_launch("lbt_bn_bwd_quant_stats");
-}
-
-extern "C" int lbt_bn_bwd_quant_stats(const float* g, const float* out, int relu, const int8_t* k2, const int8_t* k1,
-                                      size_t n_outer, size_t n_inner, int C, int bits2, const int32_t* ib2,
-                                      const float* gamma_q, const float* beta_q, int bits_g2, const int32_t* ib_g2,
-                                      const float* noise_g2, uint64_t offset_g2, uint64_t* counters_g2, int bits_g1,
-                                      const int32_t* ib_g1, const float* noise_g1, uint64_t offset_g1,
-                                      uint64_t* counters_g1, uint64_t seed, const uint64_t* dev_step, float* d_add,
-                                      void* kg1, int64_t* sums, int stats_minmax, int kg1_kind, void* stream) {
-  return bn_bwd1_run(g, out, relu, k2, k1, n_outer, n_inner, C, bits2, ib2, gamma_q, beta_q, bits_g2, ib_g2, noise_g2, offset_g2,
-                     counters_g2, bits_g1, ib_g1, noise_g1, offset_g1, counters_g1, seed, dev_step, d_add, kg1, sums, stats_minmax,
-                     kg1_kind, nullptr, stream);
-}
-
-extern "C" int lbt_bn_bwd_quant_stats_pooled(const float* g_pooled, const lbt_pool_geom* pool, int relu, const int8_t* k2,
-                                             const int8_t* k1, size_t n_outer, size_t n_inner, int C, int bits2, const int32_t* ib2,
-                                             const float* gamma_q, const float* beta_q, int bits_g2, const int32_t* ib_g2,
-                                             const float* noise_g2, uint64_t offset_g2, uint64_t* counters_g2, int bits_g1,
-                                             const int32_t* ib_g1, const float* noise_g1, uint64_t offset_g1,
-                                             uint64_t* counters_g1, uint64_t seed, const uint64_t* dev_step, void* kg1,
-                                             int64_t* sums, int stats_minmax, int kg1_kind, void* stream) {
-  if (!pool) return LBT_EINVAL;
-  return bn_bwd1_run(g_pooled, nullptr, relu, k2, k1, n_outer, n_inner, C, bits2, ib2, gamma_q, beta_q, bits_g2, ib_g2, noise_g2,
-                     offset_g2, counters_g2, bits_g1, ib_g1, noise_g1, offset_g1, counters_g1, seed, dev_step, nullptr, kg1, sums,
-                     stats_minmax, kg1_kind, pool, stream);
 }
 
 extern "C" int lbt_bn_bwd_apply(const void* kg1, const int8_t* k1, size_t n_outer, size_t n_inner, int C, int bits1,
@@ -1956,62 +1638,6 @@ extern "C" int lbt_bn_bwd_apply(const void* kg1, const int8_t* k1, size_t n_oute
   if ((rc = set_smem(kern, smem))) return rc;
   launch_pdl(kern, grid, kThreads, smem, reinterpret_cast<cudaStream_t>(stream), p);
   return check_launch("lbt_bn_bwd_apply");
-}
-
-extern "C" int lbt_bn_bwd_fused(const lbt_bn_bwd_args* a, void* stream) {
-  if (!a || !a->g || !a->k2 || !a->k1 || !a->ib2 || !a->gamma_q || !a->beta_q || !a->q_g2.ib || !a->q_g1.ib || !a->bwd_sums ||
-      !a->ib1 || !a->fwd_sums || !a->barrier)
-    return LBT_EINVAL;
-  if (a->relu < 0 || a->relu > 2 || (a->relu == 2 && !a->out)) return LBT_EINVAL;
-  if (!a->dx && !a->has_q_grad) return LBT_EINVAL;
-  if (a->has_q_grad && (!a->g_mant || !a->q_grad.ib || a->q_grad.bits < 2 || a->q_grad.bits > 8)) return LBT_EINVAL;
-  for (int b : {a->bits2, a->q_g2.bits, a->q_g1.bits, a->bits1})
-    if (b < 2 || b > 8) return LBT_EUNSUPPORTED;
-  if (a->n_outer == 0 || a->n_inner == 0) return LBT_OK;
-  if (!al16(a->g) || !al4(a->k2) || !al4(a->k1) || (a->out && !al16(a->out)) || (a->d_add && !al16(a->d_add)) ||
-      (a->dx && !al16(a->dx)) || (a->g_mant && !al4(a->g_mant)))
-    return LBT_EUNSUPPORTED;
-  LBT_REQUIRE_ARCH();
-  const int C = a->C;
-  BwdFusedParams q{};
-  // occupancy with the largest row buffer; the tiling must then be ONE tile per resident CTA with <= kMaxSavedRows rows
-  const size_t smem_max = (size_t)4 * C * 8 + (size_t)kMaxSavedRows * kThreads * sizeof(uint2);
-  int rc = set_smem(bn_bwd_fused_kernel, smem_max);
-  if (rc) return rc;
-  unsigned grid;
-  rc = make_tiling(q.a.t, a->n_outer, a->n_inner, C, grid, ctas_per_sm(bn_bwd_fused_kernel, smem_max));
-  if (rc) return rc;
-  if (!q.a.t.fixed_channels || q.a.t.total_tiles != grid || q.a.t.rows_per_group > (uint32_t)kMaxSavedRows) return LBT_EUNSUPPORTED;
-  q.b.t = q.a.t;
-  q.a.g = a->g;
-  q.a.out = a->out;
-  q.a.relu = a->relu;
-  q.a.k2 = a->k2;
-  q.a.k1 = a->k1;
-  q.a.bits2 = a->bits2;
-  q.a.ib2 = a->ib2;
-  q.a.gq = a->gamma_q;
-  q.a.bq = a->beta_q;
-  q.a.qg2 = site_from_abi(&a->q_g2);
-  q.a.qg1 = site_from_abi(&a->q_g1);
-  q.a.d_add = a->d_add;
-  q.a.kg1 = nullptr;
-  q.a.sums = reinterpret_cast<long long*>(a->bwd_sums);
-  q.b.bits1 = a->bits1;
-  q.b.ib1 = a->ib1;
-  q.b.fsums = reinterpret_cast<const long long*>(a->fwd_sums);
-  q.b.eps = a->eps;
-  q.b.bitsg1 = a->q_g1.bits;
-  q.b.ibg1 = a->q_g1.ib;
-  q.b.bsums = reinterpret_cast<const long long*>(a->bwd_sums);
-  q.b.dx = a->dx;
-  q.b.qg = site_from_abi(a->has_q_grad ? &a->q_grad : nullptr);
-  q.b.g_mant = a->g_mant;
-  q.bar = reinterpret_cast<unsigned long long*>(a->barrier);
-  const size_t smem = (size_t)4 * C * 8 + (size_t)q.a.t.rows_per_group * kThreads * sizeof(uint2);
-  launch_pdl(bn_bwd_fused_kernel, grid, kThreads, smem_max, reinterpret_cast<cudaStream_t>(stream), q);
-  (void)smem;
-  return check_launch("lbt_bn_bwd_fused");
 }
 
 extern "C" int lbt_bn_bwd_running(const float* g, const float* out, int relu, const int8_t* k2, size_t n_outer, size_t n_inner,
@@ -2071,16 +1697,6 @@ extern "C" int lbt_bn_bwd_running(const float* g, const float* out, int relu, co
   if ((rc = set_smem(kern, smem))) return rc;
   launch_pdl(kern, grid, kThreads, smem, reinterpret_cast<cudaStream_t>(stream), p);
   return check_launch("lbt_bn_bwd_running");
-}
-
-// Non-zero once the grid barrier of lbt_bn_bwd_fused has timed out (synchronises the device; not in lbt.h).
-extern "C" int lbt_bn_debug_error() {
-  int v = 0;
-  if (cudaMemcpyFromSymbol(&v, lbt::g_bn_error, sizeof(v)) != cudaSuccess) {
-    (void)cudaGetLastError();
-    return 0;
-  }
-  return v;
 }
 
 extern "C" int lbt_bn_set_debug(void* dev_u64) {

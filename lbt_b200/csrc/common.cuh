@@ -102,7 +102,7 @@ __device__ __forceinline__ uint32_t fastdiv(uint32_t n, const FastDiv& f) { retu
 #endif
 // LBT_PDL_TRIGGER_AFTER_WAIT = 1: a kernel lets its successor start only once its OWN wait has returned, i.e. once its
 // predecessor has completed.  By induction everything older than the immediate predecessor is then complete when a kernel
-// starts, so data produced two or more launches earlier (the packed weights of lbt_param_prep) may be read BEFORE the wait.
+// starts.
 __device__ __forceinline__ void pdl_wait() {
   asm volatile("griddepcontrol.wait;" ::: "memory");
 #if LBT_PDL_TRIGGER_AFTER_WAIT

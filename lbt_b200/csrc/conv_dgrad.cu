@@ -107,8 +107,6 @@ extern "C" int lbt_conv_i8_dgrad_block(const void* g, int g_kind, int N, int OH,
                                        int OHs, int OWs, int Cout_s, const void* w_short, int ws_kind, size_t ldws,
                                        const int32_t* ib_gs, const int32_t* ib_ws, int exp_short, float* dx, size_t ldc,
                                        const float* addend, void* stream) {
-  w_kind &= ~LBT_MANT_PREPARED;
-  ws_kind &= ~LBT_MANT_PREPARED;
   if (!g || !w2 || !dx || !ib_g || !ib_w) return LBT_EINVAL;
   if ((g_kind != LBT_MANT_S8 && g_kind != LBT_MANT_U8) || (w_kind != LBT_MANT_S8 && w_kind != LBT_MANT_U8)) return LBT_EINVAL;
   if (N <= 0 || H <= 0 || W <= 0 || Cin <= 0 || Cout <= 0 || kh <= 0 || kw <= 0 || sh <= 0 || sw <= 0 || OH <= 0 || OW <= 0)

@@ -652,8 +652,6 @@ int lbt::conv_fprop_run(const void* src, int src_kind, int N, int H, int W, int 
                         int kh, int kw, int sh, int sw, int pad_top, int pad_left, int OH, int OW, const int32_t* ib_src,
                         const int32_t* ib_w, int exp_const, const float* bias, float* out, size_t ldc, const lbt_qsite* q_out,
                         int8_t* k_out, int64_t* sums, const float* addend, void* stream, const OutRemap* remap, const void* src_lo) {
-  const bool w_prepared = (w_kind & LBT_MANT_PREPARED) != 0;
-  w_kind &= ~LBT_MANT_PREPARED;
   const bool dual = src_lo != nullptr;   // src = high byte plane (s8), src_lo = low byte plane (u8) of a 16-bit source
   if (!src || !wp) return LBT_EINVAL;
   if (dual && (q_out || bias || !out || src_kind != LBT_MANT_S8 || (reinterpret_cast<uintptr_t>(src_lo) & 15))) return LBT_EUNSUPPORTED;
@@ -675,7 +673,7 @@ int lbt::conv_fprop_run(const void* src, int src_kind, int N, int H, int W, int 
       !(reinterpret_cast<uintptr_t>(wp) & 15) && !(ldw & 15) && ldw >= (size_t)kh * kw * C && (q_out || ldc >= (size_t)Cout)) {
     LBT_REQUIRE_ARCH();   // narrow channels: the cp.async-gather kernel (conv_ldg.cu)
     return conv_ldg_run(src, src_kind, N, H, W, C, wp, w_kind, ldw, Cout, kh, kw, sh, sw, pad_top, pad_left, OH, OW, 0, ib_src,
-                        ib_w, exp_const, bias, out, ldc, q_out, k_out, sums, addend, stream, nullptr, w_prepared);
+                        ib_w, exp_const, bias, out, ldc, q_out, k_out, sums, addend, stream);
   }
   const uint32_t cb = C >= 128 ? 128u : (uint32_t)C;
   if (cb != 16 && cb != 32 && cb != 64 && cb != 128) return LBT_EUNSUPPORTED;

@@ -23,8 +23,7 @@ int conv_ldg_c64_halo();   // 1: 64-channel inputs take the gather kernel when i
 int conv_ldg_run(const void* src, int src_kind, int N, int SH, int SW, int C, const void* wp, int w_kind, size_t ldw, int Cout,
                  int kh, int kw, int sh, int sw, int pt, int pl, int OH, int OW, int gather, const int32_t* ibA,
                  const int32_t* ibB, int exp_const, const float* bias, float* out, size_t ldc, const lbt_qsite* q_out,
-                 int8_t* k_out, int64_t* sums, const float* addend, void* stream, const lbt_bn_bwd_link* link = nullptr,
-                 bool w_prepared = false);
+                 int8_t* k_out, int64_t* sums, const float* addend, void* stream);
 
 // conv_halo.cu: stride-1 convolutions of 64- / 128-channel inputs, halo patches through the TMA engine, resident filter bank
 bool conv_halo_applies(int N, int OH, int OW, int C, int Cout, int kh, int kw, int sh, int sw);

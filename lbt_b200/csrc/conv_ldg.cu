@@ -59,7 +59,6 @@ struct LdgParams {
   uint32_t nstages;              // ring depth
   uint32_t m_tiles;
   int gather;                    // 0 fprop, 1 transposed (dgrad)
-  int w_prepared;                // LBT_MANT_PREPARED: the filter may be read before the programmatic-dependency wait
   const int32_t* ibA;
   const int32_t* ibB;
   int exp_const;
@@ -69,7 +68,6 @@ struct LdgParams {
   size_t ldc;
   uint32_t idesc;
   BnqParams bnq;
-  GqParams gq;                   // fused "BN backward pass 1" epilogue (gq.g2.bits == 0: off); excludes bnq
   unsigned long long* dbg;       // optional timeline of CTA 0 (globaltimer ns), see lbt_conv_ldg_set_debug
   // halo mode (stride-1 gather 0): an M tile is an 8-wide x 16-high patch of output pixels of ONE image
   uint32_t OH, n_img;
@@ -120,7 +118,7 @@ __device__ __forceinline__ uint64_t make_desc_k16(uint32_t smem_addr, uint32_t l
 // 8-row groups are halo rows (stride halo_w * 16 B), and a filter tap is just a different start address.
 // EPI epilogue warps: 8 with two CTAs per SM, or 16 in ONE CTA per SM when the resident filter bank is too big for two CTAs
 // (the 7x7 ImageNet stem: 8 epilogue warps alone on an SM cannot keep up with the fused epilogue).
-template <int BN, int CPP, bool HALO, bool GQ, int EPI = 8>   // CPP = C / 16: 16-byte chunks per pixel; GQ: the fused BN-backward epilogue
+template <int BN, int CPP, bool HALO, int EPI = 8>   // CPP = C / 16: 16-byte chunks per pixel
 __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 1) conv_ldg_kernel(const LdgParams p) {
   constexpr int kEpiWarps = EPI;
   constexpr int kThreads = 32 * (kLoaderWarps + 1 + EPI);
@@ -135,7 +133,7 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
   __shared__ __align__(8) uint64_t b_bar;   // the resident filter bank has landed
   __shared__ uint32_t tmem_slot;
   __shared__ int s_abort;
-  constexpr int kStats = GQ ? 4 : 2;             // per-channel sums of the fused epilogue: bnq 2, gq 4
+  constexpr int kStats = 2;                      // per-channel sums of the fused epilogue
   __shared__ int s_stat[kEpiWarps][kStats * BN];
   __shared__ unsigned long long s_tot[kStats * BN];   // CTA totals of the fused statistics
   __shared__ int2 s_tab[kMaxKC + 8];       // tap slot: {byte offset from the row's base pixel, tap code}
@@ -206,20 +204,7 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
   fence_before();
   __syncthreads();
   fence_after();
-  // everything above touched only shared / tensor memory and kernel parameters.  With LBT_PDL_TRIGGER_AFTER_WAIT the packed
-  // filter bank (written by lbt_param_prep, at least two launches ago) is already final when this kernel starts, so the
-  // epilogue warps start copying it BEFORE waiting for the predecessor (which produced the activations / gradients).
-#if LBT_PDL_TRIGGER_AFTER_WAIT
-  if (p.w_prepared && warp > kLoaderWarps) {
-    for (uint32_t i = threadIdx.x - 32 * (kLoaderWarps + 1); i < p.KCp * BN; i += 32 * kEpiWarps) {
-      const uint32_t kp = i / BN, n = i % BN;
-      const int kc = HALO ? (int)s_kmap[kp] : (kp < p.KC ? (int)kp : -1);
-      const bool v = kc >= 0 && n < p.N;
-      cp_async16(smem_u32(sB + (size_t)i * 16), v ? p.wp + (size_t)n * p.ldw + (size_t)kc * 16 : p.wp, v ? 16u : 0u);
-    }
-    cp_async_arrive_noinc(&b_bar);
-  }
-#endif
+  // everything above touched only shared / tensor memory and kernel parameters
   pdl_wait();
   const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(&tmem_slot);
   volatile int* abort_flag = &s_abort;
@@ -392,10 +377,6 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
   } else {
     // ===== epilogue warps; first they fetch the resident filter bank (the loaders are already gathering tile 0):
     // chunk kc, output channel n -> 16 bytes (zeros beyond Cout / KC), all copies in flight at once =====
-#if LBT_PDL_TRIGGER_AFTER_WAIT
-    if (!p.w_prepared)
-#endif
-    {
     for (uint32_t i = threadIdx.x - 32 * (kLoaderWarps + 1); i < p.KCp * BN; i += 32 * kEpiWarps) {
       const uint32_t kp = i / BN, n = i % BN;
       const int kc = HALO ? (int)s_kmap[kp] : (kp < p.KC ? (int)kp : -1);
@@ -403,7 +384,6 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
       cp_async16(smem_u32(sB + (size_t)i * 16), v ? p.wp + (size_t)n * p.ldw + (size_t)kc * 16 : p.wp, v ? 16u : 0u);
     }
     cp_async_arrive_noinc(&b_bar);
-    }
     // TMEM lane quadrant = warp % 4
     const uint32_t quad = warp & 3;
     const uint32_t half = (uint32_t)(warp - (kLoaderWarps + 1)) >> 2;  // which of the quadrant's kSub warps
@@ -411,15 +391,12 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
     if (p.ibA) e += *p.ibA;
     if (p.ibB) e += *p.ibB;
     const float scale = exp2i(e);
-    const bool fused = !GQ && p.bnq.q.bits != 0;
-    const bool fusedg = GQ;
+    const bool fused = p.bnq.q.bits != 0;
     int* my_stat = s_stat[warp - (kLoaderWarps + 1)];
     BnqState bst;
-    GqState gst;
     bst.tiles = 0;
-    if (fused) bst.init(p.bnq);
-    if (fusedg) gst.init(p.gq);
-    if (fused || fusedg) {
+    if (fused) {
+      bst.init(p.bnq);
       for (int i = lane; i < kStats * BN; i += 32) my_stat[i] = 0;
       __syncwarp();
     }
@@ -446,21 +423,11 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
         row = img * p.OHW + pix;
       } else {
         row = tile * kBlockM + quad * 32 + lane;
-        pix = (fused || fusedg) ? row - fast_div(row, p.OHW, p.ohw_mul, p.ohw_shr) * p.OHW : 0u;   // row % (OH*OW)
+        pix = fused ? row - fast_div(row, p.OHW, p.ohw_mul, p.ohw_shr) * p.OHW : 0u;   // row % (OH*OW)
         rvalid = row < p.M;
       }
       constexpr int G = BN >= 64 ? 16 : (BN < 32 ? BN : 32);  // columns fetched from tensor memory per wait (wide tiles: 16, register budget)
       constexpr bool kSplit = BN > G;       // wide tiles: both warps of a quadrant alternate the G-column groups
-      // fused BN-backward epilogue: the saved mantissas of this warp's FIRST column group are fetched before the wait
-      uint32_t pw2[GQ ? G / 16 : 1][4], pw1[GQ ? G / 16 : 1][4];
-      if constexpr (GQ) {
-        const int cf = kSplit ? G * (int)half : 0;
-#pragma unroll
-        for (int q = 0; q < G / 16; ++q) {
-          const uint32_t c = (uint32_t)(cf + 16 * q);
-          gq_load_k(p.gq, row, rvalid && c < p.N, c, c < p.N ? min(16u, p.N - c) : 0u, p.N, pw2[q], pw1[q]);
-        }
-      }
       if (fused) {   // this warp's noise lines of the tile: into L1 while the accumulator is still being computed
 #pragma unroll 1
         for (int c0 = kSplit ? G * (int)half : 0; c0 < BN; c0 += kSplit ? kSub * G : G)
@@ -477,16 +444,9 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
         bnq_flush(p.bnq, my_stat, 0, BN, p.N, lane);
         bst.tiles = 0;
       }
-      if constexpr (GQ) if (bst.tiles >= (uint32_t)kBnqFlushTiles) {
-        gq_flush(p.gq, my_stat, 0, BN, p.N, lane);
-        bst.tiles = 0;
-      }
       ++bst.tiles;
-      bool first_group = true;
 #pragma unroll 1
       for (int c0 = kSplit ? G * (int)half : 0; c0 < BN; c0 += kSplit ? kSub * G : G) {
-        const bool fg = first_group;   // this group's mantissas were fetched before the wait
-        first_group = false;
         uint32_t vv[G / 16][16];
 #pragma unroll
         for (int q = 0; q < G / 16; ++q) tmem_ld16(taddr + c0 + 16 * q, vv[q]);
@@ -509,12 +469,7 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
             for (int j = 0; j < 16; ++j)
               if (j < (int)ncol) f[j] = __fadd_rn(f[j], __ldg(p.bias + c + j));
           }
-          if (GQ) {
-            if constexpr (GQ) {
-              if (!fg) gq_load_k(p.gq, row, rvalid, (uint32_t)c, ncol, p.N, pw2[q], pw1[q]);
-              gq_chunk(p.gq, gst, f, pw2[q], pw1[q], row, pix, rvalid, (uint32_t)c, ncol, p.N, my_stat, BN, (uint32_t)c, lane);
-            }
-          } else if (rvalid) {
+          if (rvalid) {
             float* o = p.out + (size_t)row * p.ldc + c;
             if (p.addend) {   // + an fp32 tensor of the output's shape (the other branch of a gradient sum)
             const float* ad = p.addend + (o - p.out);
@@ -560,10 +515,6 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
       bnq_flush_cta(p.bnq, my_stat, s_tot, 0, BN, p.N, lane, threadIdx.x - 32 * (kLoaderWarps + 1), 32 * kEpiWarps, 1);
       bnq_finish(p.bnq, bst, (unsigned long long)p.M * p.N, warp == kLoaderWarps + 1, lane);
     }
-    if constexpr (GQ) if (ok) {
-      gq_flush_cta(p.gq, my_stat, s_tot, 0, BN, p.N, lane, threadIdx.x - 32 * (kLoaderWarps + 1), 32 * kEpiWarps, 1);
-      gq_finish(p.gq, gst, (unsigned long long)p.M * p.N, warp == kLoaderWarps + 1, lane);
-    }
   }
 
   fence_before();
@@ -574,47 +525,43 @@ __global__ void __launch_bounds__(32 * (kLoaderWarps + 1 + EPI), EPI == 8 ? 2 : 
   if (threadIdx.x == 32 * kLoaderWarps) dbg_stamp(p, 18);
 }
 
-template <int BN, int CPP, bool HALO, bool GQ, int EPI>
+template <int BN, int CPP, bool HALO, int EPI>
 int launch_ldg3(const LdgParams& p, unsigned grid, size_t smem, cudaStream_t st) {
   static size_t attr_smem[16] = {};
   const int dev = device_info().device;
   if (attr_smem[dev] < smem) {
-    cudaError_t e = cudaFuncSetAttribute(conv_ldg_kernel<BN, CPP, HALO, GQ, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(conv_ldg_kernel<BN, CPP, HALO, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) {
       set_cuda_error(e, "cudaFuncSetAttribute(conv_ldg_kernel)");
       return LBT_ECUDA;
     }
     attr_smem[dev] = smem;
   }
-  launch_pdl(conv_ldg_kernel<BN, CPP, HALO, GQ, EPI>, grid, 32 * (kLoaderWarps + 1 + EPI), smem, st, p);
+  launch_pdl(conv_ldg_kernel<BN, CPP, HALO, EPI>, grid, 32 * (kLoaderWarps + 1 + EPI), smem, st, p);
   return check_launch("lbt_conv_i8 (cp.async gather)");
 }
 
 // p.epi16: one CTA per SM (big filter bank) with a halo loader and a wide tile -> the 16-epilogue-warp instantiation
-template <int BN, int CPP, bool HALO, bool GQ>
+template <int BN, int CPP, bool HALO>
 int launch_ldg2(const LdgParams& p, unsigned grid, size_t smem, cudaStream_t st) {
-  if constexpr (HALO && !GQ && BN >= 64) {
-    if (p.epi16) return launch_ldg3<BN, CPP, HALO, GQ, 16>(p, grid, smem, st);
+  if constexpr (HALO && BN >= 64) {
+    if (p.epi16) return launch_ldg3<BN, CPP, HALO, 16>(p, grid, smem, st);
   }
-  return launch_ldg3<BN, CPP, HALO, GQ, 8>(p, grid, smem, st);
+  return launch_ldg3<BN, CPP, HALO, 8>(p, grid, smem, st);
 }
 
-template <int BN, bool HALO, bool GQ>
+template <int BN, bool HALO>
 int launch_ldg1(const LdgParams& p, unsigned grid, size_t smem, cudaStream_t st) {
   switch (p.cpp) {
-    case 1: return launch_ldg2<BN, 1, HALO, GQ>(p, grid, smem, st);
-    case 2: return launch_ldg2<BN, 2, HALO, GQ>(p, grid, smem, st);
-    default: return launch_ldg2<BN, 4, HALO, GQ>(p, grid, smem, st);
+    case 1: return launch_ldg2<BN, 1, HALO>(p, grid, smem, st);
+    case 2: return launch_ldg2<BN, 2, HALO>(p, grid, smem, st);
+    default: return launch_ldg2<BN, 4, HALO>(p, grid, smem, st);
   }
 }
 
 template <int BN>
 int launch_ldg(const LdgParams& p, unsigned grid, size_t smem, cudaStream_t st, bool halo) {
-  if (p.gq.g2.bits != 0) {   // fused BN-backward epilogue: stride-1 input gradients (halo loader where the image allows)
-    if constexpr (BN <= 64) return halo ? launch_ldg1<BN, true, true>(p, grid, smem, st) : launch_ldg1<BN, false, true>(p, grid, smem, st);
-    else return LBT_EUNSUPPORTED;
-  }
-  return halo ? launch_ldg1<BN, true, false>(p, grid, smem, st) : launch_ldg1<BN, false, false>(p, grid, smem, st);
+  return halo ? launch_ldg1<BN, true>(p, grid, smem, st) : launch_ldg1<BN, false>(p, grid, smem, st);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -923,7 +870,7 @@ int conv_wgrad_ldg_run(const void* src, int src_kind, int N, int H, int W, int C
 int conv_ldg_run(const void* src, int src_kind, int N, int SH, int SW, int C, const void* wp, int w_kind, size_t ldw, int Cout,
                  int kh, int kw, int sh, int sw, int pt, int pl, int OH, int OW, int gather, const int32_t* ibA,
                  const int32_t* ibB, int exp_const, const float* bias, float* out, size_t ldc, const lbt_qsite* q_out,
-                 int8_t* k_out, int64_t* sums, const float* addend, void* stream, const lbt_bn_bwd_link* link, bool w_prepared) {
+                 int8_t* k_out, int64_t* sums, const float* addend, void* stream) {
   const DeviceInfo& di = device_info();
   const int bn = Cout <= 16 ? 16 : (Cout <= 32 ? 32 : (Cout <= 64 ? 64 : 128));
   if ((size_t)N * OH * OW >= (1ull << 31)) return LBT_EUNSUPPORTED;
@@ -976,7 +923,6 @@ int conv_ldg_run(const void* src, int src_kind, int N, int SH, int SW, int C, co
   p.stages_per_tile = (p.KCp + kChunksPerStage - 1) / kChunksPerStage;
   p.m_tiles = (p.M + kBlockM - 1) / kBlockM;
   p.gather = gather;
-  p.w_prepared = w_prepared ? 1 : 0;
   p.ibA = ibA;
   p.ibB = ibB;
   p.exp_const = exp_const;
@@ -989,20 +935,6 @@ int conv_ldg_run(const void* src, int src_kind, int N, int SH, int SW, int C, co
   p.bnq.k = k_out;
   p.bnq.sums = reinterpret_cast<long long*>(sums);
   p.bnq.rows_per_image = (uint32_t)(OH * OW);
-  if (link) {
-    p.gq.g2 = site_from_abi(&link->q_g2);
-    p.gq.g1 = site_from_abi(&link->q_g1);
-    p.gq.bits2 = link->bits2;
-    p.gq.ib2 = link->ib2;
-    p.gq.gamma_q = link->gamma_q;
-    p.gq.beta_q = link->beta_q;
-    p.gq.k2 = link->k2;
-    p.gq.k1 = link->k1;
-    p.gq.relu = link->relu;
-    p.gq.kg1 = link->kg1;
-    p.gq.sums = reinterpret_cast<long long*>(link->sums);
-    p.gq.rows_per_image = (uint32_t)(OH * OW);
-  }
   p.dbg = g_dbg.load(std::memory_order_relaxed);
   // halo mode: every input pixel is copied to shared memory ~1.4 times instead of kh * kw times
   p.OH = (uint32_t)OH;
@@ -1044,7 +976,7 @@ int conv_ldg_run(const void* src, int src_kind, int N, int SH, int SW, int C, co
   p.nstages = nst;
   size_t smem = b_bytes + (size_t)nst * p.stage_bytes + 256;
   const unsigned ctas_per_sm = two ? 2u : 1u;
-  p.epi16 = (!two && halo && bn >= 64 && !link) ? 1 : 0;
+  p.epi16 = (!two && halo && bn >= 64) ? 1 : 0;
   if (p.epi16 && smem < 120 * 1024) smem = 120 * 1024;   // that instantiation owns up to all 512 TMEM columns: never two per SM
   const uint64_t cap = (uint64_t)di.sm_count * ctas_per_sm;
   const unsigned grid = (unsigned)(p.m_tiles < cap ? p.m_tiles : cap);
@@ -1065,8 +997,6 @@ extern "C" int lbt_conv_i8_dgrad(const void* g, int g_kind, int N, int OH, int O
                                  int Cin, int kh, int kw, int sh, int sw, int pad_top, int pad_left, int H, int W,
                                  const int32_t* ib_g, const int32_t* ib_w, int exp_const, float* dx, size_t ldc, const float* addend,
                                  void* stream) {
-  const bool w_prepared = (w_kind & LBT_MANT_PREPARED) != 0;
-  w_kind &= ~LBT_MANT_PREPARED;
   if (!g || !wp || !dx) return LBT_EINVAL;
   if ((g_kind != LBT_MANT_S8 && g_kind != LBT_MANT_U8) || (w_kind != LBT_MANT_S8 && w_kind != LBT_MANT_U8)) return LBT_EINVAL;
   if (N <= 0 || H <= 0 || W <= 0 || Cin <= 0 || Cout <= 0 || kh <= 0 || kw <= 0 || sh <= 0 || sw <= 0 || OH <= 0 || OW <= 0)
@@ -1077,29 +1007,7 @@ extern "C" int lbt_conv_i8_dgrad(const void* g, int g_kind, int N, int OH, int O
   LBT_REQUIRE_ARCH();
   // rows = input pixels (n, h, w); gathered tensor = g[N, OH, OW, Cout]; output channels = Cin
   return conv_ldg_run(g, g_kind, N, OH, OW, Cout, wp, w_kind, ldw, Cin, kh, kw, sh, sw, pad_top, pad_left, H, W, 1, ib_g, ib_w,
-                      exp_const, nullptr, dx, ldc, nullptr, nullptr, nullptr, addend, stream, nullptr, w_prepared);
-}
-
-extern "C" int lbt_conv_i8_dgrad_bn(const void* g, int g_kind, int N, int H, int W, int C, const void* wp, int w_kind, size_t ldw,
-                                    int Cout, int kh, int kw, int pad_top, int pad_left, int OH, int OW, const int32_t* ib_g,
-                                    const int32_t* ib_w, int exp_const, const lbt_bn_bwd_link* link, void* stream) {
-  const bool w_prepared = (w_kind & LBT_MANT_PREPARED) != 0;
-  w_kind &= ~LBT_MANT_PREPARED;
-  if (!g || !wp || !link) return LBT_EINVAL;
-  if ((g_kind != LBT_MANT_S8 && g_kind != LBT_MANT_U8) || (w_kind != LBT_MANT_S8 && w_kind != LBT_MANT_U8)) return LBT_EINVAL;
-  if (N <= 0 || H <= 0 || W <= 0 || C <= 0 || Cout <= 0 || kh <= 0 || kw <= 0 || OH <= 0 || OW <= 0) return LBT_EINVAL;
-  if (!link->k2 || !link->k1 || !link->kg1 || !link->sums || !link->gamma_q || !link->beta_q || !link->ib2 || !link->q_g2.ib ||
-      !link->q_g1.ib)
-    return LBT_EINVAL;
-  if (link->relu != 0 && link->relu != 1) return LBT_EUNSUPPORTED;
-  if (link->q_g2.bits < 2 || link->q_g2.bits > 8 || link->q_g1.bits < 2 || link->q_g1.bits > 8 || (Cout & 3)) return LBT_EUNSUPPORTED;
-  if ((reinterpret_cast<uintptr_t>(g) & 15) || (reinterpret_cast<uintptr_t>(wp) & 15) || (ldw & 15) || ldw < (size_t)kh * kw * C)
-    return LBT_EUNSUPPORTED;
-  if ((reinterpret_cast<uintptr_t>(link->gamma_q) | reinterpret_cast<uintptr_t>(link->beta_q)) & 15) return LBT_EUNSUPPORTED;
-  if (!conv_ldg_enabled() || !conv_ldg_ok(C, Cout, kh, kw)) return LBT_EUNSUPPORTED;
-  LBT_REQUIRE_ARCH();
-  return conv_ldg_run(g, g_kind, N, H, W, C, wp, w_kind, ldw, Cout, kh, kw, 1, 1, pad_top, pad_left, OH, OW, 0, ib_g, ib_w, exp_const,
-                      nullptr, nullptr, (size_t)Cout, nullptr, nullptr, nullptr, nullptr, stream, link, w_prepared);
+                      exp_const, nullptr, dx, ldc, nullptr, nullptr, nullptr, addend, stream);
 }
 
 // Test / bench knob (not in lbt.h): 0 routes every convolution through the TMA-im2col kernel, 1 (default) lets the

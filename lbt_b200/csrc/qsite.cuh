@@ -58,19 +58,6 @@ __device__ __forceinline__ void mm_to_counts(const QC& c, float mx, float mn, ui
 // tm = RD(t + 1.5 * 2^23) is ONE full-rate FADD.RM; floor(t) as an integer is bits(tm) - 0x4B400000, as a float tm - 1.5 * 2^23,
 // and the low byte(s) of bits(tm) are the two's-complement mantissa byte(s).
 constexpr float kFloorMagicF = 12582912.0f;
-constexpr int kFloorMagicI = 0x4B400000;
-__device__ __forceinline__ int squant_i(float x, float u, const QC& c, uint32_t& n1, uint32_t& n2) {
-  const float y = __fmul_rn(x, c.m);
-  n1 += (uint32_t)(y >= c.L) + (uint32_t)(y < -c.L);
-  n2 += (uint32_t)(y >= c.half) + (uint32_t)(y < -c.half);
-  return __float_as_int(__fadd_rd(fminf(fmaxf(__fadd_rn(y, u), -c.L), c.hi), kFloorMagicF)) - kFloorMagicI;
-}
-__device__ __forceinline__ int squant_mm_i(float x, float u, const QC& c, float& mx, float& mn) {
-  const float y = __fmul_rn(x, c.m);
-  mx = fmaxf(mx, y);
-  mn = fminf(mn, y);
-  return __float_as_int(__fadd_rd(fminf(fmaxf(__fadd_rn(y, u), -c.L), c.hi), kFloorMagicF)) - kFloorMagicI;
-}
 
 // a / b, correctly rounded (== __fdiv_rn), for MANY numerators over ONE denominator: r = frcp_rn(b) is computed once
 // (per channel) and each quotient costs five FMA-class instructions instead of the ~12 + special-case branch of the
@@ -126,36 +113,6 @@ struct BnqState {
     tiles = 0;
   }
 };
-
-// Sum 16 per-lane values over the 32 lanes of a warp with a reduce-scatter butterfly (16 shuffles):
-// afterwards lanes 2c and 2c+1 both hold the warp total of v[c], c = (lane >> 1) & 15.
-__device__ __forceinline__ int warp_colsum16(const int (&v)[16], int lane) {
-  int w8[8], w4[4], w2[2];
-  const bool b4 = lane & 16, b3 = lane & 8, b2 = lane & 4, b1 = lane & 2;
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const int send = b4 ? v[j] : v[j + 8];
-    const int recv = __shfl_xor_sync(0xffffffffu, send, 16);
-    w8[j] = (b4 ? v[j + 8] : v[j]) + recv;
-  }
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const int send = b3 ? w8[j] : w8[j + 4];
-    const int recv = __shfl_xor_sync(0xffffffffu, send, 8);
-    w4[j] = (b3 ? w8[j + 4] : w8[j]) + recv;
-  }
-#pragma unroll
-  for (int j = 0; j < 2; ++j) {
-    const int send = b2 ? w4[j] : w4[j + 2];
-    const int recv = __shfl_xor_sync(0xffffffffu, send, 4);
-    w2[j] = (b2 ? w4[j + 2] : w4[j]) + recv;
-  }
-  const int send = b1 ? w2[0] : w2[1];
-  const int recv = __shfl_xor_sync(0xffffffffu, send, 2);
-  int w1 = (b1 ? w2[1] : w2[0]) + recv;
-  w1 += __shfl_xor_sync(0xffffffffu, w1, 1);
-  return w1;
-}
 
 // Per-channel sum k and sum k^2 of a warp's 32 rows x 16 channels from the PACKED mantissas (w[i] = channels 4i .. 4i+3 of
 // this lane's row, two's-complement bytes), ~58 instructions instead of the ~140 of two 16-value butterflies:
@@ -214,7 +171,7 @@ __device__ __forceinline__ void bnq_prefetch(const BnqParams& b, uint32_t pix, u
 //     element becomes the value 0, which quantises to mantissa 0 (u < 1), leaves min / max and the counts alone and adds nothing;
 //   * without a bias the two power-of-two scalings fold into one multiply (exact while the exponents stay far from the
 //     subnormal range — checked on the host side of the branch);
-//   * the mantissa byte is the low byte of the magic-biased floor (squant_i), packed with three PRMT per four elements;
+//   * the mantissa byte is the low byte of the magic-biased floor, packed with three PRMT per four elements;
 //   * statistics from the packed bytes (warp_colstats_packed).
 __device__ __forceinline__ uint32_t pack4_low_bytes(float t0, float t1, float t2, float t3) {
   const uint32_t p01 = __byte_perm(__float_as_uint(t0), __float_as_uint(t1), 0x0040);
@@ -378,168 +335,6 @@ __device__ __forceinline__ void bnq_finish(const BnqParams& b, BnqState& st, uns
     if (n1) atomicAdd(b.q.counters + LBT_CNT_OVER, (unsigned long long)n1);
     if (n2) atomicAdd(b.q.counters + LBT_CNT_OVER_HALF, (unsigned long long)n2);
     if (ticket && blockIdx.x == 0) atomicAdd(b.q.counters + LBT_CNT_NUMEL, numel);   // fire-and-forget, no ticket
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Fused "BN backward pass 1" epilogue of an input-gradient GEMM: the fp32 gradient dX a convolution's dgrad would
-// write is the `g` of the batch-norm that PRECEDES that convolution in the network, so lbt_bn_bwd_quant_stats'
-// arithmetic (ReLU mask recomputed from k2, kg2 = Q(g) dfxp:687, dbeta / dgamma sums :689-690, dx2 = gq2 * gamma_q :691,
-// kg1 = Q(dx2) :621, the two batch-norm VJP sums) runs on the accumulators while they are in registers: no fp32
-// gradient tensor in HBM (4 B written + 4 B read per element) and one launch less per unit.
-// ------------------------------------------------------------------------------------------------
-struct GqParams {
-  QSite g2, g1;             // Rescale_q / Normalization_q gradient quantisers (g2.bits == 0: disabled)
-  int bits2;                // Rescale_q input quantiser (k2 mantissas): bits, range
-  const int32_t* ib2;
-  const float* gamma_q;     // [N] fake-quantised gamma, beta
-  const float* beta_q;
-  const int8_t* k2;         // [M, N] saved mantissas of the forward pass
-  const int8_t* k1;
-  int relu;                 // 0: none, 1: mask recomputed from k2 (dfxp:986)
-  int8_t* kg1;              // [M, N] out
-  long long* sums;          // [4*N] out (caller-zeroed): sum kg2, sum kg2*k2, sum kg1, sum kg1*k1
-  uint32_t rows_per_image;
-};
-
-struct GqState {
-  QC c2, cg2, cg1;
-  uint64_t off2, off1;
-  uint32_t a1, a2, b1, b2;
-  float amx, amn, bmx, bmn;
-  uint32_t tiles;
-  __device__ __forceinline__ void init(const GqParams& g) {
-    c2 = make_qc(g.bits2, __ldg(g.ib2));
-    cg2 = make_qc(g.g2.bits, __ldg(g.g2.ib));
-    cg1 = make_qc(g.g1.bits, __ldg(g.g1.ib));
-    off2 = site_offset(g.g2);
-    off1 = site_offset(g.g1);
-    a1 = a2 = b1 = b2 = 0;
-    amx = bmx = -INFINITY;
-    amn = bmn = INFINITY;
-    tiles = 0;
-  }
-};
-
-// One 16-channel chunk of one row; f = the fp32 gradient the unfused dgrad would have written.
-// s_stat: this warp's private [4][bn] int32 partial sums.  The chunk is processed in four groups of four channels so that
-// only 16 statistics values (4 sums x 4 channels) are live at a time; one reduce-scatter butterfly per group.
-// The saved mantissas k2 / k1 of one 16-channel chunk of one row, as four words each.  Called BEFORE the epilogue waits for
-// the accumulator, so the global-memory latency overlaps the MMA instead of sitting between tcgen05.ld and the store.
-__device__ __forceinline__ void gq_load_k(const GqParams& b, uint32_t row, bool row_ok, uint32_t col, uint32_t ncol, uint32_t N,
-                                          uint32_t (&w2)[4], uint32_t (&w1)[4]) {
-  const int8_t* p2 = b.k2 + (size_t)row * N + col;
-  const int8_t* p1 = b.k1 + (size_t)row * N + col;
-#pragma unroll
-  for (int g = 0; g < 4; ++g) w2[g] = w1[g] = 0u;
-  if (row_ok) {   // N % 4 == 0 and col % 16 == 0: every group of four channels is a whole, 4-byte aligned word
-    if (ncol == 16 && (((reinterpret_cast<uintptr_t>(p2) | reinterpret_cast<uintptr_t>(p1)) & 15u) == 0)) {
-      const uint4 a2 = __ldcs(reinterpret_cast<const uint4*>(p2)), a1 = __ldcs(reinterpret_cast<const uint4*>(p1));
-      w2[0] = a2.x; w2[1] = a2.y; w2[2] = a2.z; w2[3] = a2.w;
-      w1[0] = a1.x; w1[1] = a1.y; w1[2] = a1.z; w1[3] = a1.w;
-    } else {
-#pragma unroll
-      for (int g = 0; g < 4; ++g)
-        if (4u * g < ncol) {
-          w2[g] = __ldcs(reinterpret_cast<const uint32_t*>(p2) + g);
-          w1[g] = __ldcs(reinterpret_cast<const uint32_t*>(p1) + g);
-        }
-    }
-    const uint64_t inner = (uint64_t)(b.rows_per_image ? row % b.rows_per_image : 0u) * N + col;
-    if (b.g2.noise) asm volatile("prefetch.global.L1 [%0];" ::"l"(b.g2.noise + inner));
-    if (b.g1.noise) asm volatile("prefetch.global.L1 [%0];" ::"l"(b.g1.noise + inner));
-  }
-}
-
-__device__ __forceinline__ void gq_chunk(const GqParams& b, GqState& st, const float (&f)[16], const uint32_t (&w2)[4],
-                                         const uint32_t (&w1)[4], uint32_t row, uint32_t pix, bool row_ok, uint32_t col, uint32_t ncol,
-                                         uint32_t N, int* s_stat, uint32_t bn, uint32_t tcol, int lane) {
-  const uint64_t inner = (uint64_t)pix * N + col;   // multiple of 4
-  int8_t* o = b.kg1 + (size_t)row * N + col;
-#pragma unroll
-  for (int g = 0; g < 4; ++g) {
-    float4 u2, u1;
-    const bool ok = row_ok && 4u * g < ncol;    // ncol % 4 == 0
-    if (b.g2.noise) u2 = ok ? __ldg(reinterpret_cast<const float4*>(b.g2.noise + inner) + g) : make_float4(0.f, 0.f, 0.f, 0.f);
-    else u2 = philox_noise4((inner >> 2) + g, b.g2.seed, st.off2);
-    if (b.g1.noise) u1 = ok ? __ldg(reinterpret_cast<const float4*>(b.g1.noise + inner) + g) : make_float4(0.f, 0.f, 0.f, 0.f);
-    else u1 = philox_noise4((inner >> 2) + g, b.g1.seed, st.off1);
-    const float un2[4] = {u2.x, u2.y, u2.z, u2.w}, un1[4] = {u1.x, u1.y, u1.z, u1.w};
-    const uint32_t cg = min(col + 4u * g, N - 4u);   // a masked group reads in-range parameters
-    const float4 ga = __ldg(reinterpret_cast<const float4*>(b.gamma_q + cg)), be = __ldg(reinterpret_cast<const float4*>(b.beta_q + cg));
-    const float gam[4] = {ga.x, ga.y, ga.z, ga.w}, bet[4] = {be.x, be.y, be.z, be.w};
-    int v[16];
-    uint32_t packed = 0;
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const int k2 = (int)(int8_t)((w2[g] >> (8 * t)) & 0xff), k1 = (int)(int8_t)((w1[g] >> (8 * t)) & 0xff);
-      float gj = ok ? f[4 * g + t] : 0.0f;
-      if (b.relu == 1) {
-        const float y2 = __fadd_rn(__fmul_rn(__int2float_rn(k2) * st.c2.inv_m, gam[t]), bet[t]);
-        if (!(y2 > 0.0f)) gj = 0.0f;
-      }
-      const int kg2r = b.g2.minmax ? squant_mm_i(gj, un2[t], st.cg2, st.amx, st.amn) : squant_i(gj, un2[t], st.cg2, st.a1, st.a2);
-      const int kg2i = ok ? kg2r : 0;
-      const float kg2 = __fsub_rn(__int_as_float(kg2r + kFloorMagicI), kFloorMagicF);   // the mantissa as a float, no I2F
-      const float dx2 = ok ? __fmul_rn(kg2 * st.cg2.inv_m, gam[t]) : 0.0f;
-      const int kg1r = b.g1.minmax ? squant_mm_i(dx2, un1[t], st.cg1, st.bmx, st.bmn) : squant_i(dx2, un1[t], st.cg1, st.b1, st.b2);
-      const int kg1i = ok ? kg1r : 0;
-      v[t] = kg2i;
-      v[4 + t] = kg2i * k2;
-      v[8 + t] = kg1i;
-      v[12 + t] = kg1i * k1;
-      packed |= (uint32_t)(kg1i & 0xff) << (8 * t);
-    }
-    if (ok) *(reinterpret_cast<uint32_t*>(o) + g) = packed;
-    const int tot = warp_colsum16(v, lane);
-    if ((lane & 1) == 0) {
-      const int c = (lane >> 1) & 15;          // c = 4 * statistic + channel of the group
-      s_stat[(c >> 2) * bn + tcol + 4 * g + (c & 3)] += tot;
-    }
-  }
-}
-
-// Per-warp flush of the [4][bn] partials for tile columns [col0, col0 + bn) (int32 headroom), and the CTA-level final flush.
-__device__ __forceinline__ void gq_flush(const GqParams& b, int* s_stat, uint32_t col0, uint32_t bn, uint32_t N, int lane) {
-  __syncwarp();
-  for (uint32_t i = lane; i < 4 * bn; i += 32) {
-    const uint32_t k = i / bn, c = i - k * bn;
-    const int v = s_stat[i];
-    if (v && col0 + c < N) atomicAdd(reinterpret_cast<unsigned long long*>(b.sums) + (size_t)k * N + col0 + c, (unsigned long long)(long long)v);
-    s_stat[i] = 0;
-  }
-  __syncwarp();
-}
-__device__ __forceinline__ void gq_flush_cta(const GqParams& b, int* s_stat, unsigned long long* s_tot, uint32_t col0, uint32_t bn, uint32_t N,
-                                             int lane, uint32_t tid, uint32_t nthreads, int bar_id) {
-  __syncwarp();
-  for (uint32_t i = lane; i < 4 * bn; i += 32) {
-    const int v = s_stat[i];
-    if (v) atomicAdd(s_tot + i, (unsigned long long)(long long)v);
-    s_stat[i] = 0;
-  }
-  asm volatile("bar.sync %0, %1;" ::"r"(bar_id), "r"(nthreads) : "memory");
-  for (uint32_t i = tid; i < 4 * bn; i += nthreads) {
-    const uint32_t k = i / bn, c = i - k * bn;
-    const unsigned long long v = s_tot[i];
-    if (v && col0 + c < N) atomicAdd(reinterpret_cast<unsigned long long*>(b.sums) + (size_t)k * N + col0 + c, v);
-  }
-}
-__device__ __forceinline__ void gq_finish(const GqParams& b, GqState& st, unsigned long long numel, bool ticket, int lane) {
-  if (b.g2.minmax) mm_to_counts(st.cg2, st.amx, st.amn, st.a1, st.a2);
-  if (b.g1.minmax) mm_to_counts(st.cg1, st.bmx, st.bmn, st.b1, st.b2);
-  const uint32_t a1 = warp_sum(st.a1), a2 = warp_sum(st.a2), b1 = warp_sum(st.b1), b2 = warp_sum(st.b2);
-  if (lane == 0) {
-    if (b.g2.counters) {
-      if (a1) atomicAdd(b.g2.counters + LBT_CNT_OVER, (unsigned long long)a1);
-      if (a2) atomicAdd(b.g2.counters + LBT_CNT_OVER_HALF, (unsigned long long)a2);
-      if (ticket && blockIdx.x == 0) atomicAdd(b.g2.counters + LBT_CNT_NUMEL, numel);
-    }
-    if (b.g1.counters) {
-      if (b1) atomicAdd(b.g1.counters + LBT_CNT_OVER, (unsigned long long)b1);
-      if (b2) atomicAdd(b.g1.counters + LBT_CNT_OVER_HALF, (unsigned long long)b2);
-      if (ticket && blockIdx.x == 0) atomicAdd(b.g1.counters + LBT_CNT_NUMEL, numel);
-    }
   }
 }
 

@@ -534,21 +534,13 @@ FUSE_POOL_FWD = os.environ.get('LBT_FUSE_POOL_FWD', '1') != '0'
 # First-layer weight gradient through lbt_conv_i8_wgrad_c3 (LBT_STEM_WGRAD=0: the general kernel on the 16-byte pixels).
 STEM_WGRAD = os.environ.get('LBT_STEM_WGRAD', '1') != '0'
 
-# LBT_MANT_PREPARED (include/lbt.h): let the convolution kernels copy a filter packed by lbt_param_prep before they wait for their
-# predecessor.  Measured on B200: the kernels' own time drops 3 % but the step does not move (same-box A/B 1.4347 vs 1.4345 ms),
-# so it is off unless LBT_W_PREFETCH=1.
-_W_PREPARED = 0x100 if os.environ.get('LBT_W_PREFETCH', '0') == '1' else 0
-
-
 def _conv_implicit(src_nhwc, src_kind, wp, Cout, kh, kw, sh, sw, pt, pl, OH, OW, ib_src, ib_w, exp_const, bias, out2d,
-                   bnq=None, addend=None, w_prepared=False):
+                   bnq=None, addend=None):
     """lbt_conv_i8_fprop: out2d[N*OH*OW, Cout] = conv(src, wp) * 2^(exp_const + ib_src + ib_w) (+ bias), or with
     ``bnq = (QSiteStruct, k_out, sums)`` the fused re-quantising epilogue (s8 mantissas + batch statistics)."""
     N, H, W, C = src_nhwc.shape
     qs, k_out, sums = bnq if bnq is not None else (None, None, None)
-    # w_prepared: the filter comes from lbt_param_prep (start of the step): LBT_MANT_PREPARED lets the kernel fetch it early
-    _lib.call('lbt_conv_i8_fprop', _lib.ptr(src_nhwc), src_kind, N, H, W, C, _lib.ptr(wp), Q.MANT_S8 | (_W_PREPARED if w_prepared else 0),
-              wp.stride(0), Cout,
+    _lib.call('lbt_conv_i8_fprop', _lib.ptr(src_nhwc), src_kind, N, H, W, C, _lib.ptr(wp), Q.MANT_S8, wp.stride(0), Cout,
               kh, kw, sh, sw, pt, pl, OH, OW, _lib.ptr(ib_src), _lib.ptr(ib_w), int(exp_const), _lib.ptr(bias),
               _lib.ptr(out2d), out2d.stride(0) if out2d is not None else Cout,
               ctypes.addressof(qs) if qs is not None else None, _lib.ptr(k_out), _lib.ptr(sums), _lib.ptr(addend), _lib.stream(),
@@ -692,7 +684,7 @@ def _conv_fprop(layer, geom, xm, xkind, prep, wm, bq, out2d, bnq=None):
             w3 = wm.view(kh * kw, 3, Cout)
             w16 = torch.cat([w3, w3, w3, torch.zeros(kh * kw, 7, Cout, dtype=torch.int8, device=xm.device)], dim=1)
             wt = _transpose_bytes(w16.view(kh * kw * 16, Cout))
-        _conv_implicit(xm, Q.MANT_S8, wt, Cout, kh, kw, sh, sw, pt, pl, OH, OW, ibx, ibw, e, bq, out2d, bnq, w_prepared=prep is not None)
+        _conv_implicit(xm, Q.MANT_S8, wt, Cout, kh, kw, sh, sw, pt, pl, OH, OW, ibx, ibw, e, bq, out2d, bnq)
         return
     segs = 3 if xkind == Q.MANT_S16 else 1
     wt = prep['wt'] if prep is not None else _transpose_bytes(wm.view(Kf, Cout))     # B operand [Cout, Kf]
@@ -702,14 +694,13 @@ def _conv_fprop(layer, geom, xm, xkind, prep, wm, bq, out2d, bnq=None):
     if kh == 1 and kw == 1 and sh == 1 and sw == 1 and segs == 1 and Cin % 16 == 0 and pt == 0 and pl == 0:
         G.gemm_i8(xm.reshape(N * H * W, Cin), wt, ibA=ibx, ibB=ibw, exp_const=e, bias=bq, out=out2d, bnq=gbnq)   # 1x1
     elif layer.implicit and segs == 1 and _implicit_ok(Cin, kh, kw):
-        _conv_implicit(xm, xkind, wt, Cout, kh, kw, sh, sw, pt, pl, OH, OW, ibx, ibw, e, bq, out2d, bnq,
-                       w_prepared=prep is not None)                                                               # dfxp:291
+        _conv_implicit(xm, xkind, wt, Cout, kh, kw, sh, sw, pt, pl, OH, OW, ibx, ibw, e, bq, out2d, bnq)     # dfxp:291
     else:
         A = _im2col(xm, xkind, OH, OW, kh, kw, sh, sw, pt, pl, False)
         G.gemm_i8(A, wt, ibA=ibx, ibB=ibw, exp_const=e, bias=bq, out=out2d, bnq=gbnq)
 
 
-def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_db, addend=None, link=None, shortcut=None):
+def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_db, addend=None, shortcut=None):
     """dfxp:302-305 from the quantised gradient mantissas gm [N, OH, OW, Cout] (s8): (dX NHWC fp32, dW, db).
     ``addend`` (NHWC fp32, the shape of dX): the gradient reaching the same input along another branch (residual
     shortcut), added in the dgrad epilogue instead of by a separate pass over the tensor.  ``shortcut``: a strided block's
@@ -781,27 +772,7 @@ def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_
     if need_db:
         db = _emit_grad(rt, layer.bias, _colsum(g2, Q.MANT_S8, rt), ibA=layer.qG.range, exp_const=-(gb - 1))      # dfxp:304
     # ---- dgrad: dX[NHW, Cin] = im2colT(G)[NHW, kh*kw*Cout] . Wt[Cin, kh*kw*Cout] ----
-    linked = False
-    if (need_dx and link is not None and link.k1 is not None and addend is None and layer.implicit and sh == 1 and sw == 1 and
-            kh * kw > 1 and _implicit_ok(Cout, kh, kw) and tuple(link.k1.shape) == (N, H, W, Cin)):
-        # the producing unit's BN backward pass 1 in this dgrad's epilogue: no fp32 dX (lbt_conv_i8_dgrad_bn)
-        K2 = kh * kw * Cout
-        pw2 = prep['w2'] if prep is not None else None
-        w2 = pw2 if pw2 is not None else _as_operand(wm.flip(0, 1).permute(2, 0, 1, 3).reshape(Cin, K2))
-        rt = layer.qX.runtime
-        kg1 = torch.empty_like(link.k1)
-        bsums = rt.zeros_i64(4 * Cin + 2, dev)
-        ls = link.struct(H * W * Cin, dev, kg1, bsums)
-        linked = _lib.try_call('lbt_conv_i8_dgrad_bn', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2),
-                               Q.MANT_S8 | (_W_PREPARED if pw2 is not None else 0), w2.stride(0), Cin, kh, kw, kh - 1 - pt, kw - 1 - pl, H, W, _lib.ptr(layer.qG.range),
-                               _lib.ptr(layer.qW.range), int(-(gb - 1) - (wb - 1)), ctypes.addressof(ls), _lib.stream(),
-                               meta=dict(ops=2 * N * H * W * Cin * K2, bytes=N * OH * OW * Cout + Cin * K2 + 3 * N * H * W * Cin))
-        if linked:
-            global _link_count
-            _link_count += 1
-            link.kg1, link.bsums, link.done = kg1, bsums, True
-            dx = torch.empty(1, dtype=torch.float32, device=dev).expand(N, H, W, Cin)      # shape carrier only
-    if need_dx and not linked:
+    if need_dx:
         K2 = kh * kw * Cout
         dx = torch.empty(N, H, W, Cin, dtype=torch.float32, device=dev)
         ad2 = addend.reshape(N * H * W, Cin) if addend is not None else None
@@ -816,12 +787,11 @@ def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_
             # stride 1: dX = conv(G, rot180(W)) with padding (k - 1 - pad): the same implicit-GEMM kernel
             w2 = pw2 if pw2 is not None else _as_operand(wm.flip(0, 1).permute(2, 0, 1, 3).reshape(Cin, K2))
             _conv_implicit(gm, Q.MANT_S8, w2, Cin, kh, kw, 1, 1, kh - 1 - pt, kw - 1 - pl, H, W, layer.qG.range,
-                           layer.qW.range, e, None, dx.view(N * H * W, Cin), addend=ad2, w_prepared=pw2 is not None)   # dfxp:305
+                           layer.qW.range, e, None, dx.view(N * H * W, Cin), addend=ad2)   # dfxp:305
         elif layer.implicit and _gather_ok(Cout, Cin, kh, kw) and sh <= 4 and sw <= 4:
             # any stride: the transposed gather runs in the kernel's loader warps (lbt_conv_i8_dgrad), no im2col matrix
             w2 = pw2 if pw2 is not None else _as_operand(wm.view(kh * kw, Cin, Cout).permute(1, 0, 2).reshape(Cin, K2))
-            _lib.call('lbt_conv_i8_dgrad', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2),
-                      Q.MANT_S8 | (_W_PREPARED if pw2 is not None else 0), w2.stride(0),
+            _lib.call('lbt_conv_i8_dgrad', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2), Q.MANT_S8, w2.stride(0),
                       Cin, kh, kw, sh, sw, pt, pl, H, W, _lib.ptr(layer.qG.range), _lib.ptr(layer.qW.range), int(e),
                       _lib.ptr(dx), Cin, _lib.ptr(ad2), _lib.stream(),
                       meta=dict(ops=2 * N * H * W * Cin * K2, bytes=N * OH * OW * Cout + Cin * K2 + N * H * W * Cin * 4))
@@ -832,13 +802,12 @@ def _conv_backward(layer, geom, xm, xkind, wm, prep, gm, need_dx, need_dw, need_
             else:
                 perm = torch.tensor(_class_perm(kh, kw, sh, sw), device=dev)
                 w2 = _as_operand(wm.view(kh * kw, Cin, Cout).index_select(0, perm).permute(1, 0, 2).reshape(Cin, K2))
-            done = shortcut is not None and addend is None and _dgrad_block(layer, geom, gm, w2, pw2 is not None, e, dx, shortcut)
+            done = shortcut is not None and addend is None and _dgrad_block(layer, geom, gm, w2, e, dx, shortcut)
             if not done:
                 if shortcut is not None:      # the kernel declined the shapes: the shortcut's dgrad first, then this one adds it
                     ad2 = _shortcut_dgrad(shortcut).reshape(N * H * W, Cin)
-                _lib.call('lbt_conv_i8_dgrad_strided', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2),
-                          Q.MANT_S8 | (_W_PREPARED if pw2 is not None else 0), w2.stride(0),
-                          Cin, kh, kw, sh, sw, pt, pl, H, W, _lib.ptr(layer.qG.range), _lib.ptr(layer.qW.range), int(e),
+                _lib.call('lbt_conv_i8_dgrad_strided', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2), Q.MANT_S8,
+                          w2.stride(0), Cin, kh, kw, sh, sw, pt, pl, H, W, _lib.ptr(layer.qG.range), _lib.ptr(layer.qW.range), int(e),
                           _lib.ptr(dx), Cin, _lib.ptr(ad2), _lib.stream(),
                           meta=dict(ops=2 * N * OH * OW * Cin * K2,
                                     bytes=N * OH * OW * Cout * min(sh * sw, kh * kw) + Cin * K2 + N * H * W * Cin * 4))
@@ -894,7 +863,7 @@ def _shortcut_dgrad(parked):
     return dx
 
 
-def _dgrad_block(layer, geom, gm, w2, w_prepared, e, dx, shortcut):
+def _dgrad_block(layer, geom, gm, w2, e, dx, shortcut):
     """lbt_conv_i8_dgrad_block: dx = this strided convolution's input gradient + the parked shortcut's, in one launch.
     False when the kernel does not take the shapes (the caller then runs the two launches)."""
     global _block_dgrad_count
@@ -907,10 +876,10 @@ def _dgrad_block(layer, geom, gm, w2, w_prepared, e, dx, shortcut):
     sw2 = spw2 if spw2 is not None else _as_operand(swm.view(Cin, sCout))
     se = -(sl.qG.bits - 1) - (sl.qW.bits - 1)
     K2 = kh * kw * Cout
-    done = _lib.try_call('lbt_conv_i8_dgrad_block', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2),
-                         Q.MANT_S8 | (_W_PREPARED if w_prepared else 0), w2.stride(0), Cin, kh, kw, sh, sw, pt, pl, H, W,
+    done = _lib.try_call('lbt_conv_i8_dgrad_block', _lib.ptr(gm), Q.MANT_S8, N, OH, OW, Cout, _lib.ptr(w2), Q.MANT_S8,
+                         w2.stride(0), Cin, kh, kw, sh, sw, pt, pl, H, W,
                          _lib.ptr(layer.qG.range), _lib.ptr(layer.qW.range), int(e), _lib.ptr(sgm), Q.MANT_S8, sOH, sOW, sCout,
-                         _lib.ptr(sw2), Q.MANT_S8 | (_W_PREPARED if spw2 is not None else 0), sw2.stride(0),
+                         _lib.ptr(sw2), Q.MANT_S8, sw2.stride(0),
                          _lib.ptr(sl.qG.range), _lib.ptr(sl.qW.range), int(se), _lib.ptr(dx), Cin, None, _lib.stream(),
                          meta=dict(ops=2 * N * OH * OW * Cin * K2 + 2 * N * sOH * sOW * Cin * sCout,
                                    bytes=N * OH * OW * Cout + N * sOH * sOW * sCout + Cin * (K2 + sCout) + N * H * W * Cin * 4))
@@ -1409,18 +1378,17 @@ def _bn_fwd2(bn, k1, sums, gq, bq, add_, relu, next_site=None, next_kind=Q.MANT_
     return k2, out, nm, relu_mode
 
 
-def _bn_backward(bn, g_, k1, k2, sums, gq, bq, out_, relu_mode, has_add, grad_site=None, want_dx=True, pre=None, pool=None):
+def _bn_backward(bn, g_, k1, k2, sums, gq, bq, out_, relu_mode, has_add, grad_site=None, want_dx=True):
     """Both BN backward passes on memory-order tensors: (dx fp32 or None, gradient mantissas of `grad_site` or None,
-    dgamma, dbeta, d_add).  ``pre = (kg1, bsums)``: pass 1 already ran in the epilogue of the consuming convolution's
-    input-gradient kernel (lbt_conv_i8_dgrad_bn); ``g_`` is then not read (may be None).
-    ``pool = (idx, k, s, pad_top, pad_left, POH, POW)``: a max-pool sits behind the unit, ``g_`` is the gradient of the POOLED
-    tensor and the pool's backward runs inside pass 1 (lbt_bn_bwd_quant_stats_pooled)."""
+    dgamma, dbeta, d_add)."""
     norm, resc = bn[0], bn[1]
     rt = norm.qX.runtime
     N, C = k1.shape[0], k1.shape[-1]
     n_inner = k1.numel() // N
     dev = k1.device
-    bsums = pre[1] if pre is not None else rt.zeros_i64(4 * C + 2, dev)   # [4C] sums + the grid-barrier word of the fused launch
+    # [4C] sums; the two spare slots keep every later arena slice at the offset the step was tuned with (exactly 4C measured
+    # 1.7 us slower on ResNet-20's 1.351 ms step, B200 at 1000 W)
+    bsums = rt.zeros_i64(4 * C + 2, dev)
     d_add = torch.empty(k1.shape, dtype=torch.float32, device=dev) if has_add else None
     dx = torch.empty(k1.shape, dtype=torch.float32, device=dev) if want_dx else None
     # gradient quantisers wider than 8 bits (config 5: 16-bit G): kg1 travels as s16, and the convolution's gradient
@@ -1433,54 +1401,21 @@ def _bn_backward(bn, g_, k1, k2, sums, gq, bq, out_, relu_mode, has_add, grad_si
         gm = torch.empty_like(k1)
         if grad_site.bits > 8:
             gm_lo = torch.empty(k1.shape, dtype=torch.uint8, device=dev)
-    nbytes = k1.numel() * (6 + (4 if relu_mode == 2 else 0) + (4 if has_add else 0) + (4 if want_dx else 0) +
-                           (1 if gm is not None else 0))
-    # small tensors: both passes in one launch (lbt_bn_bwd_fused); it declines shapes that are not one wave of CTAs
-    fused = False
-    # (its grid barrier needs every CTA co-resident: not while weight-gradient kernels share the SMs on the side stream)
-    if FUSE_BN_BWD and pre is None and pool is None and not wide and gm_lo is None and not getattr(rt, '_side_pending', False):
-        a = _lib.BnBwdArgs(g=_lib.ptr(g_), out=_lib.ptr(out_), k2=_lib.ptr(k2), k1=_lib.ptr(k1), n_outer=N, n_inner=n_inner, C=C,
-                           relu=relu_mode, bits2=resc.qX.bits, bits1=norm.qX.bits, ib2=_lib.ptr(resc.qX.range),
-                           ib1=_lib.ptr(norm.qX.range), gamma_q=_lib.ptr(gq), beta_q=_lib.ptr(bq),
-                           q_g2=resc.qG.abi(n_inner, dev), q_g1=norm.qG.abi(n_inner, dev), d_add=_lib.ptr(d_add),
-                           bwd_sums=_lib.ptr(bsums), fwd_sums=_lib.ptr(sums), eps=float(norm.eps),
-                           has_q_grad=int(qg is not None), dx=_lib.ptr(dx), g_mant=_lib.ptr(gm),
-                           barrier=bsums[4 * C:].data_ptr())
-        if qg is not None:
-            a.q_grad = qg
-        fused = _lib.try_call('lbt_bn_bwd_fused', ctypes.addressof(a), _lib.stream(), meta=dict(bytes=nbytes))
-    if not fused and pre is not None:
-        kg1 = pre[0]
-    elif not fused and pool is not None:
-        kg1 = torch.empty(k1.shape, dtype=torch.int16 if wide else torch.int8, device=dev)
-        nzg2, offg2 = _site_args(resc.qG, k1)
-        nzg1, offg1 = _site_args(norm.qG, k1)
-        pidx, pk, ps, ppt, ppl, POH, POW = pool
-        geo = _lib.PoolGeom(idx=_lib.ptr(pidx), H=k1.shape[1], W=k1.shape[2], k=pk, s=ps, pad_top=ppt, pad_left=ppl, OH=POH, OW=POW)
-        _lib.call('lbt_bn_bwd_quant_stats_pooled', _lib.ptr(g_), ctypes.addressof(geo), relu_mode, _lib.ptr(k2), _lib.ptr(k1), N,
-                  n_inner, C, resc.qX.bits, _lib.ptr(resc.qX.range), _lib.ptr(gq), _lib.ptr(bq), resc.qG.bits,
-                  _lib.ptr(resc.qG.range), _lib.ptr(nzg2), offg2, _lib.ptr(resc.qG.counters), norm.qG.bits,
-                  _lib.ptr(norm.qG.range), _lib.ptr(nzg1), offg1, _lib.ptr(norm.qG.counters), rt.seed,
-                  _lib.ptr(rt.dev_step), _lib.ptr(kg1), _lib.ptr(bsums),
-                  int(resc.qG.target == 0 and norm.qG.target == 0), kg1_kind, _lib.stream(),
-                  meta=dict(bytes=g_.numel() * 5 + k1.numel() * (3 + (1 if wide else 0))))
-    elif not fused:
-        kg1 = torch.empty(k1.shape, dtype=torch.int16 if wide else torch.int8, device=dev)
-        nzg2, offg2 = _site_args(resc.qG, g_)
-        nzg1, offg1 = _site_args(norm.qG, g_)
-        _lib.call('lbt_bn_bwd_quant_stats', _lib.ptr(g_), _lib.ptr(out_), relu_mode, _lib.ptr(k2), _lib.ptr(k1), N, n_inner,
-                  C, resc.qX.bits, _lib.ptr(resc.qX.range), _lib.ptr(gq), _lib.ptr(bq), resc.qG.bits,
-                  _lib.ptr(resc.qG.range), _lib.ptr(nzg2), offg2, _lib.ptr(resc.qG.counters), norm.qG.bits,
-                  _lib.ptr(norm.qG.range), _lib.ptr(nzg1), offg1, _lib.ptr(norm.qG.counters), rt.seed,
-                  _lib.ptr(rt.dev_step), _lib.ptr(d_add), _lib.ptr(kg1), _lib.ptr(bsums),
-                  int(resc.qG.target == 0 and norm.qG.target == 0), kg1_kind, _lib.stream(),
-                  meta=dict(bytes=g_.numel() * (7 + (1 if wide else 0) + (4 if relu_mode == 2 else 0) + (4 if has_add else 0))))
-    if not fused:
-        _lib.call('lbt_bn_bwd_apply', _lib.ptr(kg1), _lib.ptr(k1), N, n_inner, C, norm.qX.bits, _lib.ptr(norm.qX.range),
-                  _lib.ptr(sums), float(norm.eps), norm.qG.bits, _lib.ptr(norm.qG.range), _lib.ptr(bsums), _lib.ptr(dx),
-                  ctypes.addressof(qg) if qg is not None else None, _lib.ptr(gm), kg1_kind, _lib.ptr(gm_lo), _lib.stream(),
-                  meta=dict(bytes=k1.numel() * (2 + (1 if wide else 0) + (4 if want_dx else 0) + (1 if gm is not None else 0) +
-                                                (1 if gm_lo is not None else 0))))
+    kg1 = torch.empty(k1.shape, dtype=torch.int16 if wide else torch.int8, device=dev)
+    nzg2, offg2 = _site_args(resc.qG, g_)
+    nzg1, offg1 = _site_args(norm.qG, g_)
+    _lib.call('lbt_bn_bwd_quant_stats', _lib.ptr(g_), _lib.ptr(out_), relu_mode, _lib.ptr(k2), _lib.ptr(k1), N, n_inner,
+              C, resc.qX.bits, _lib.ptr(resc.qX.range), _lib.ptr(gq), _lib.ptr(bq), resc.qG.bits,
+              _lib.ptr(resc.qG.range), _lib.ptr(nzg2), offg2, _lib.ptr(resc.qG.counters), norm.qG.bits,
+              _lib.ptr(norm.qG.range), _lib.ptr(nzg1), offg1, _lib.ptr(norm.qG.counters), rt.seed,
+              _lib.ptr(rt.dev_step), _lib.ptr(d_add), _lib.ptr(kg1), _lib.ptr(bsums),
+              int(resc.qG.target == 0 and norm.qG.target == 0), kg1_kind, _lib.stream(),
+              meta=dict(bytes=g_.numel() * (7 + (1 if wide else 0) + (4 if relu_mode == 2 else 0) + (4 if has_add else 0))))
+    _lib.call('lbt_bn_bwd_apply', _lib.ptr(kg1), _lib.ptr(k1), N, n_inner, C, norm.qX.bits, _lib.ptr(norm.qX.range),
+              _lib.ptr(sums), float(norm.eps), norm.qG.bits, _lib.ptr(norm.qG.range), _lib.ptr(bsums), _lib.ptr(dx),
+              ctypes.addressof(qg) if qg is not None else None, _lib.ptr(gm), kg1_kind, _lib.ptr(gm_lo), _lib.stream(),
+              meta=dict(bytes=k1.numel() * (2 + (1 if wide else 0) + (4 if want_dx else 0) + (1 if gm is not None else 0) +
+                                            (1 if gm_lo is not None else 0))))
     # dbeta = sum gq2 (dfxp:690); dgamma = sum gq2 * xq2 + 2*wd*gamma (dfxp:689)
     dbeta = _emit_grad(rt, resc.beta, bsums[:C], ibA=resc.qG.range, exp_const=-(resc.qG.bits - 1))
     dgamma = _emit_grad(rt, resc.gamma, bsums[C:2 * C], ibA=resc.qG.range, ibB=resc.qX.range,
@@ -1554,39 +1489,6 @@ class _FusedBNFn(torch.autograd.Function):
         return _from_mem(dx), dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None), None, None, None, None
 
 
-_link_count = 0        # fused backward links taken (tests)
-FUSE_BWD_LINK = os.environ.get('LBT_BWD_LINK', '0') == '1'   # module switch: a unit's BN backward pass 1 runs in the epilogue of the NEXT unit's input-gradient kernel
-                       # (lbt_conv_i8_dgrad_bn).  Bit-identical; measured on B200: the fused launch takes 29 us where dgrad (13-17 us)
-                       # and the BN pass (12-15 us) take the same in two — its epilogue warps wait on the k1 / k2 / noise loads of
-                       # every tile — and ResNet-20's step goes from 1.433 to 1.484 ms, so it is OFF by default.
-
-
-class _BwdLink:
-    """Backward hand-off between two consecutive fused units A -> B whose only connection is A's (mantissa-only) output:
-    B's input-gradient kernel runs A's BN backward pass 1 in its epilogue (lbt_conv_i8_dgrad_bn) and leaves (kg1, sums)
-    here; A's backward then starts at pass 2.  No fp32 gradient tensor exists between the two units."""
-
-    def __init__(self):
-        self.bn = self.k1 = self.k2 = self.gq = self.bq = None
-        self.relu_mode = 0
-        self.kg1 = self.bsums = None
-        self.done = False
-
-    def offer(self, bn, k1, k2, gq, bq, relu_mode, has_add):
-        norm, resc = bn[0], bn[1]
-        if has_add or relu_mode not in (0, 1) or resc.qG.bits > 8 or norm.qG.bits > 8 or k1.shape[-1] % 4:
-            return
-        self.bn, self.k1, self.k2, self.gq, self.bq, self.relu_mode = bn, k1, k2, gq, bq, relu_mode
-
-    def struct(self, n_inner, dev, kg1, bsums):
-        norm, resc = self.bn[0], self.bn[1]
-        # arena=True: the step's pre-generated noise vectors (a GEMM epilogue cannot reuse a Philox draw down the batch the
-        # way the BN kernels do: in-kernel generation costs ~30 instructions per element there)
-        return _lib.BnBwdLink(q_g2=resc.qG.abi(n_inner, dev, arena=True), q_g1=norm.qG.abi(n_inner, dev, arena=True), bits2=resc.qX.bits,
-                              relu=self.relu_mode, ib2=_lib.ptr(resc.qX.range), gamma_q=_lib.ptr(self.gq), beta_q=_lib.ptr(self.bq),
-                              k2=_lib.ptr(self.k2), k1=_lib.ptr(self.k1), kg1=_lib.ptr(kg1), sums=_lib.ptr(bsums))
-
-
 class _ConvBNFn(torch.autograd.Function):
     """One Conv2d_q + BatchNorm2d_q unit (+ residual add, + ReLU) with every hand-off between the two modules kept
     in integer mantissas (north_star (2): the GEMM epilogue re-quantises its output, no fake-quant fp32 round trip):
@@ -1599,8 +1501,8 @@ class _ConvBNFn(torch.autograd.Function):
     the results are bit-identical (tests/test_fused_gpu.py)."""
 
     @staticmethod
-    def forward(ctx, x, weight, gamma, beta, add, conv, bn, relu, next_site, next_kind, want_fp32, alias, link_in, link_out, pool=None,
-                next2=None, running=False, block=None, frozen=False):
+    def forward(ctx, x, weight, gamma, beta, add, conv, bn, relu, next_site, next_kind, want_fp32, alias, pool=None, next2=None,
+                running=False, block=None, frozen=False):
         # running: eval mode (or frozen statistics) without an autograd graph (BatchNorm2d_q._running): the BN kernels normalise
         # with the running statistics, nothing is saved for backward.  frozen: frozen statistics while a graph is recorded —
         # the same kernels, k2 saved (k1 and the batch sums are not), backward through lbt_bn_bwd_running
@@ -1656,7 +1558,6 @@ class _ConvBNFn(torch.autograd.Function):
                                               want_k2=frozen)
         ctx.conv, ctx.bn, ctx.geom, ctx.xkind, ctx.prep = conv, bn, geom, xkind, prep
         ctx.relu_mode, ctx.has_add, ctx.frozen = relu_mode, add is not None, frozen
-        ctx.link_in, ctx.link_out = link_in, link_out
         # block: the downsampling block's _BlockDgrad; the unit with the alias is the first unit, the other one the shortcut
         ctx.block = None
         if block is not None and not running:
@@ -1666,13 +1567,11 @@ class _ConvBNFn(torch.autograd.Function):
             elif block.armed:
                 ctx.block = block
         ctx.block_first = bool(alias)
-        if link_out is not None and out is None and not running and not frozen:   # the next unit may run this BN's backward pass 1 in its dgrad epilogue
-            link_out.offer(bn, k1, k2, gq, bq, relu_mode, add is not None)
         ctx.pool = None
         if pooled is not None:    # lbt_bn_fwd_apply_pooled did both
             ctx.pool = tuple(pool)
             out = pooled
-        elif pool is not None:    # MaxPool_q behind the unit (ImageNet stem): its backward runs inside this unit's BN pass 1
+        elif pool is not None:    # MaxPool_q behind the unit (ImageNet stem)
             pk, ps, ppt, ppl, POH, POW = pool
             pooled = torch.empty(N, POH, POW, Cout, dtype=torch.float32, device=dev)
             pidx = torch.empty(N, POH, POW, Cout, dtype=torch.uint8, device=dev)
@@ -1699,26 +1598,21 @@ class _ConvBNFn(torch.autograd.Function):
         conv = ctx.conv
         xm, wm, k1, k2, sums, gq, bq, out, pidx = ctx.saved_tensors
         need_dx, need_dw = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
-        lo = ctx.link_out
-        pre = (lo.kg1, lo.bsums) if (lo is not None and lo.done) else None     # pass 1 ran in the consumer's dgrad epilogue
-        pool = ((pidx,) + ctx.pool) if ctx.pool is not None else None
-        if pool is not None and (not FUSE_POOL or ctx.frozen):
-            # the pool's backward as its own launch (lbt_maxpool_bwd, 0.82 of the HBM peak), then the plain BN pass 1: faster
-            # on B200 than gathering the windows inside pass 1 (FUSE_POOL)
-            _, pk, ps, ppt, ppl, POH, POW = pool
+        if ctx.pool is not None:
+            # the pool's backward as its own launch (lbt_maxpool_bwd, 0.82 of the HBM peak), then the plain BN pass 1
+            pk, ps, ppt, ppl, POH, POW = ctx.pool
             g_ = _to_mem(g)
             Np, Hp, Wp_, Cp = k2.shape        # (k1 is not saved with frozen statistics)
             gd = torch.empty(k2.shape, dtype=torch.float32, device=k2.device)
             _lib.call('lbt_maxpool_bwd', _lib.ptr(g_), _lib.ptr(pidx), Np, Hp, Wp_, Cp, pk, ps, ppt, ppl, POH, POW, _lib.ptr(gd),
                       _lib.stream(), meta=dict(bytes=gd.numel() * 4 + g_.numel() * 5))
-            g, pool = _from_mem(gd), None
+            g = _from_mem(gd)
         if ctx.frozen:
             _, gm, dgamma, dbeta, d_add = _bn_backward_frozen(ctx.bn, _to_mem(g), k2, gq, bq, out, ctx.relu_mode, ctx.has_add,
                                                               grad_site=conv.qG, want_dx=False)   # ... dfxp:300
         else:
-            _, gm, dgamma, dbeta, d_add = _bn_backward(ctx.bn, _to_mem(g) if pre is None else None, k1, k2, sums, gq, bq, out,
-                                                       ctx.relu_mode, ctx.has_add, grad_site=conv.qG, want_dx=False, pre=pre,
-                                                       pool=pool)   # ... dfxp:300
+            _, gm, dgamma, dbeta, d_add = _bn_backward(ctx.bn, _to_mem(g), k1, k2, sums, gq, bq, out, ctx.relu_mode, ctx.has_add,
+                                                       grad_site=conv.qG, want_dx=False)   # ... dfxp:300
         bd = ctx.block
         if bd is not None and not ctx.block_first:
             ctx.block = None
@@ -1728,7 +1622,7 @@ class _ConvBNFn(torch.autograd.Function):
                 bd.parked = (conv, ctx.geom, ctx.xkind, wm, ctx.prep, gm)
                 N, H, W, Cin = ctx.geom[:4]
                 dx = torch.empty(1, dtype=torch.float32, device=gm.device).expand(N, H, W, Cin)     # shape carrier only
-                return ((_from_mem(dx),) + (dW, dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None)) + (None,) * 14)
+                return ((_from_mem(dx),) + (dW, dgamma, dbeta, (_from_mem(d_add) if d_add is not None else None)) + (None,) * 12)
         parked = bd.take() if (bd is not None and need_dx) else None
         shortcut = None
         if parked is not None:     # g_alias is the shortcut unit's shape carrier
@@ -1740,24 +1634,15 @@ class _ConvBNFn(torch.autograd.Function):
         else:
             addend = _to_mem(g_alias) if (g_alias is not None and need_dx) else None
         ctx.block = None
-        li = ctx.link_in if (addend is None and shortcut is None and FUSE_BWD_LINK) else None
         if isinstance(gm, tuple):        # 9..16-bit gradient: (hi, lo) byte planes
             dx, dW, _ = _conv_backward16(conv, ctx.geom, xm, ctx.xkind, wm, ctx.prep, gm[0], gm[1], need_dx, need_dw, False, addend=addend)
         else:
-            dx, dW, _ = _conv_backward(conv, ctx.geom, xm, ctx.xkind, wm, ctx.prep, gm, need_dx, need_dw, False, addend=addend, link=li,
+            dx, dW, _ = _conv_backward(conv, ctx.geom, xm, ctx.xkind, wm, ctx.prep, gm, need_dx, need_dw, False, addend=addend,
                                        shortcut=shortcut)
         return ((_from_mem(dx) if dx is not None else None), dW, dgamma, dbeta,
-                (_from_mem(d_add) if d_add is not None else None), None, None, None, None, None, None, None, None, None, None, None,
-                None, None, None)
+                (_from_mem(d_add) if d_add is not None else None)) + (None,) * 12
 
 
-FUSE_POOL = os.environ.get('LBT_FUSE_POOL', '0') == '1'   # module switch: a MaxPool_q right behind a fused unit runs its backward inside the
-                      # unit's BN pass 1 (lbt_bn_bwd_quant_stats_pooled).  Bit-identical and 1.6 GB less DRAM traffic on ResNet-18's stem, but
-                      # measured slower on B200 (923 us vs 480 + 320 us for the two launches: 2.25 window gathers per element and 123
-                      # registers per thread leave the pass load-issue bound), so it is OFF by default
-FUSE_BN_BWD = False   # module switch: both BN backward passes in ONE launch (lbt_bn_bwd_fused, grid barrier) where the
-                      # tensor is one wave of CTAs.  Bit-identical; measured no faster on B200 (1.77 vs 1.75 ms ResNet-20
-                      # step: the barrier + second fp64 prologue cost what the saved launch gains), so off by default
 FUSE_UNITS = True     # module switch for the Conv2d_q + BatchNorm2d_q fused units (tests compare both settings); in eval mode it
                       # also selects the running-statistics kernels of a stand-alone BatchNorm2d_q (off: the eager reference path)
 DUAL_WGRAD = os.environ.get('LBT_DUAL_WGRAD', '1') != '0'   # 16-bit gradients: weight gradient of both byte planes in one launch
@@ -1772,8 +1657,7 @@ def _unit_fusable(conv, bn, x, running=False):
             x.is_cuda)
 
 
-def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=True, alias=False, link_in=None, link_out=None,
-                 pool=None, block=None):
+def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=True, alias=False, pool=None, block=None):
     """``bn(conv(x), add=add, relu=relu)`` as ONE fused unit when the shapes allow (else exactly that expression).
 
     next_conv: the Conv2d_q that consumes the result — its input quantiser then runs inside this unit's last kernel
@@ -1790,7 +1674,7 @@ def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=Tr
     pgeom = None
     if pool is not None:      # ``pool``: a MaxPool_q that consumes the unit's output and nothing else does
         if add is not None or alias or not pool_fusable(pool):
-            y = conv_bn_unit(conv, bn, x, add=add, relu=relu, alias=alias, link_in=link_in, link_out=link_out)
+            y = conv_bn_unit(conv, bn, x, add=add, relu=relu, alias=alias)
             return (pool(y[0]), y[1]) if alias else pool(y)
         Hc, Wc = _conv_geom(conv, x, conv.weight)[11:13]
         pgeom = pool.geometry(Hc, Wc)
@@ -1825,8 +1709,7 @@ def conv_bn_unit(conv, bn, x, add=None, relu=False, next_conv=None, want_fp32=Tr
     use_alias = bool(alias and x.requires_grad and not getattr(x, '_lbt_hollow', False) and
                      (conv.weight.shape[2] <= 128 or (block is not None and tuple(conv.stride) != (1, 1) and conv.qG.bits <= 8)))
     out, nm, xa = _ConvBNFn.apply(x, conv.weight, bn[1].gamma, bn[1].beta, add, conv, bn, relu, next_site, next_kind,
-                                  want_fp32, use_alias, link_in if FUSE_BWD_LINK else None, link_out if FUSE_BWD_LINK else None,
-                                  pgeom, next2, running, block, frozen)
+                                  want_fp32, use_alias, pgeom, next2, running, block, frozen)
     if next_site is not None and nm.numel():       # (empty: the pooled one-kernel path declined, the consumer quantises itself)
         out._lbt_q = {id(next_site): (nm, next_kind)}
         if next2 is not None and next2[2] is not None:
@@ -1848,7 +1731,7 @@ def run_layers(layers, x, next_conv=None):
         nxt = layers[i + 1] if i + 1 < len(layers) else None
         if isinstance(m, Conv2d_q) and isinstance(nxt, BatchNorm2d_q):
             after = layers[i + 2] if i + 2 < len(layers) else next_conv
-            if (FUSE_POOL or FUSE_POOL_FWD) and isinstance(after, MaxPool_q) and i + 2 < len(layers):
+            if FUSE_POOL_FWD and isinstance(after, MaxPool_q) and i + 2 < len(layers):
                 after2 = layers[i + 3] if i + 3 < len(layers) else next_conv
                 x = conv_bn_unit(m, nxt, x, pool=after, next_conv=_first_conv(after2))   # conv -> BN -> ReLU -> max-pool (ImageNet stem)
                 i += 3
@@ -2041,7 +1924,7 @@ class MaxPool_q(nn.Module):
 
 
 def pool_fusable(pool):
-    """A MaxPool_q whose backward lbt_bn_bwd_quant_stats_pooled can run: at most 2 x 2 windows over a pixel."""
+    """A MaxPool_q that conv_bn_unit takes into the fused unit (``pool``): at most 2 x 2 windows over a pixel."""
     return isinstance(pool, MaxPool_q) and pool.k <= 2 * pool.s and pool.k <= 15
 
 
@@ -2271,20 +2154,15 @@ class ResidualBlock_q(nn.Module):
         if paired:
             # the first unit hands back an alias of x for the shortcut branch: the shortcut's gradient then returns
             # through that unit's backward and is added in its dgrad epilogue (no separate add over the tensor)
-            # consecutive units of the residual branch are linked: the later unit's input-gradient kernel runs the earlier
-            # unit's BN backward pass 1 in its epilogue (_BwdLink)
-            link = _BwdLink()
             # a strided first unit and a 1x1 shortcut unit: one launch for the block's input gradient (_BlockDgrad)
             bd = _BlockDgrad() if len(sc_layers) == 2 and tuple(res[0].stride) != (1, 1) else None
-            r, xs = conv_bn_unit(res[0], res[1], x, next_conv=res[2], want_fp32=False, alias=True, link_out=link, block=bd)
+            r, xs = conv_bn_unit(res[0], res[1], x, next_conv=res[2], want_fp32=False, alias=True, block=bd)
             if xs is not x and getattr(x, '_lbt_q', None) is not None:
                 xs._lbt_q = x._lbt_q       # mantissas made for the shortcut convolution's quantiser travel with the alias
             for i in range(2, len(res) - 2, 2):
-                nxt = _BwdLink()
-                r = conv_bn_unit(res[i], res[i + 1], r, next_conv=res[i + 2], want_fp32=False, link_in=link, link_out=nxt)
-                link = nxt
+                r = conv_bn_unit(res[i], res[i + 1], r, next_conv=res[i + 2], want_fp32=False)
             sc = conv_bn_unit(sc_layers[0], sc_layers[1], xs, block=bd) if len(sc_layers) == 2 else self.shortcut(xs)
-            return conv_bn_unit(res[-2], res[-1], r, add=sc, relu=True, next_conv=next_conv, link_in=link)
+            return conv_bn_unit(res[-2], res[-1], r, add=sc, relu=True, next_conv=next_conv)
         r = x
         for m in res[:-1]:
             r = m(r)

@@ -256,15 +256,13 @@ class Trainer:
 
     def check(self):
         """Raise if a device-side watchdog fired: a cross-replica wait of lbt_dp_step timed out (the kernel then skips the
-        optimizer and every later step: the error word is sticky), or a grid barrier of the fused BN backward gave up.
-        Synchronises; fit() calls it once per epoch, state_dict() always."""
+        optimizer and every later step: the error word is sticky).  Synchronises when data-parallel; fit() calls it once per
+        epoch, state_dict() always."""
         if self.dp is not None:
             e = self.dp.error()
             if e:
                 raise _lib.LbtError('lbt_dp_step: a cross-replica wait timed out (flag slot %d); the replicas are no longer '
                                     'in step — this run cannot continue' % (e - 1))
-        if _lib.lib().lbt_bn_debug_error():
-            raise _lib.LbtError('lbt_bn_bwd_fused: the grid barrier timed out; gradients of that step are invalid')
 
     # ---- evaluation (trainer.py:164-187) ---------------------------------------------------------------------------
     @torch.no_grad()

@@ -57,8 +57,8 @@ def test_cpu_tensor_is_an_error():
         quantizer.quantize(torch.zeros(4, 4), 8, torch.tensor(2, dtype=torch.int32))
 
 
-def test_new_entry_points_validate_arguments_without_gpu():
-    """lbt_dp_step / lbt_augment_batch / lbt_quantize_residual / lbt_conv_i8_dgrad_bn reject bad arguments before any CUDA call."""
+def test_dp_augment_and_residual_entry_points_validate_arguments_without_gpu():
+    """lbt_dp_step / lbt_augment_batch / lbt_quantize_residual reject bad arguments before any CUDA call."""
     h = _lib.lib()
     buf = (ctypes.c_float * 16)()
     p = ctypes.cast(buf, ctypes.c_void_p)
@@ -80,13 +80,8 @@ def test_new_entry_points_validate_arguments_without_gpu():
     assert h.lbt_quantize_residual(p, 1, p, 2, 4, 0, ib, 0, None, 0, 0, None, p, None, None) == -1
     assert h.lbt_quantize_residual(p, 1, p, 2, 4, 8, ib, 1, None, 0, 0, None, p, None, None) == -1
     assert h.lbt_quantize_residual(p, 0, p, 0, 4, 8, ib, 0, None, 0, 0, None, p, None, None) == 0
-    # fused dgrad + BN backward: the link descriptor is mandatory and must be complete
-    assert h.lbt_conv_i8_dgrad_bn(p, 1, 1, 16, 16, 16, p, 1, 144, 16, 3, 3, 1, 1, 16, 16, ib, ib, 0, None, None) == -1
-    link = _lib.BnBwdLink()
-    assert h.lbt_conv_i8_dgrad_bn(p, 1, 1, 16, 16, 16, p, 1, 144, 16, 3, 3, 1, 1, 16, 16, ib, ib, 0, ctypes.addressof(link), None) == -1
 
 
-def test_struct_mirrors_of_the_new_descriptors():
+def test_dp_struct_mirrors_match_the_header():
     assert ctypes.sizeof(_lib.DpPeers) == 8 + 4 * 8 * 8
-    assert ctypes.sizeof(_lib.BnBwdLink) == 2 * ctypes.sizeof(_lib.QSiteStruct) + 8 + 7 * 8
     assert _lib.DP_PAD_WORDS * 4 <= 256 and _lib.DP_HANDLE_BYTES == 64

@@ -18,8 +18,7 @@ from lbt_b200.trainer import Trainer  # noqa: E402
 SEED = 77
 WD = 2e-4
 BWD = 'lbt_bn_bwd_running'
-TRAINING_BN = ('lbt_bn_bwd_apply', 'lbt_bn_bwd_quant_stats', 'lbt_bn_bwd_quant_stats_pooled', 'lbt_bn_bwd_fused',
-               'lbt_bn_fwd_apply', 'lbt_bn_fwd_apply2', 'lbt_bn_fwd_apply_pooled')
+TRAINING_BN = ('lbt_bn_bwd_apply', 'lbt_bn_bwd_quant_stats', 'lbt_bn_fwd_apply', 'lbt_bn_fwd_apply2', 'lbt_bn_fwd_apply_pooled')
 
 
 def nchw(x_nhwc):
@@ -552,7 +551,7 @@ def test_frozen_step_runs_the_one_pass_backward_and_no_aten_batch_norm_arithmeti
     ops_train, k_train = profile(False)
     ops_frozen, k_frozen = profile(True)
     assert any('bn_bwd_running_kernel' in k for k in k_frozen)
-    assert not any(s in k for k in k_frozen for s in ('bn_bwd1_kernel', 'bn_bwd2_kernel', 'bn_bwd_fused_kernel'))
+    assert not any(s in k for k in k_frozen for s in ('bn_bwd1_kernel', 'bn_bwd2_kernel'))
     assert any('bn_bwd1_kernel' in k for k in k_train)
     assert all(n <= ops_train.get(op, 0) for op, n in ops_frozen.items()), (ops_frozen, ops_train)
     ops_eager, _ = profile(True, fused=False)

@@ -11,12 +11,8 @@ from lbt_b200 import dfxp as D, models as M  # noqa: E402
 from lbt_b200.trainer import Trainer  # noqa: E402
 
 
-def _run(name, fused, steps, batch, image, kw, bn_bwd=False, link=False, pool=False):
+def _run(name, fused, steps, batch, image, kw):
     D.FUSE_UNITS = fused
-    D.FUSE_POOL = pool
-    D.FUSE_BN_BWD = bn_bwd
-    D.FUSE_BWD_LINK = link
-    D._link_count = 0
     try:
         torch.manual_seed(3)
         model = getattr(M, name)(8, weight_decay=2e-4, seed=9, **kw).cuda()
@@ -33,41 +29,6 @@ def _run(name, fused, steps, batch, image, kw, bn_bwd=False, link=False, pool=Fa
                     bn=[b.clone() for n, b in model.named_buffers() if 'running' in n])
     finally:
         D.FUSE_UNITS = True
-        D.FUSE_POOL = False
-        D.FUSE_BN_BWD = False
-        D.FUSE_BWD_LINK = False
-
-
-@pytest.mark.parametrize('name,batch,image,kw', [('Resnet18', 4, 64, dict(image=64, num_classes=10)),
-                                                 ('Resnet18', 3, 60, dict(image=60, num_classes=10)),      # 30 x 30 -> 15 x 15: ragged windows
-                                                 ('Resnet18', 2, 72, dict(image=72, num_classes=10, grad_bits=16)),   # s16 kg1
-                                                 ('Resnet50', 2, 64, dict(image=64, num_classes=10))])
-def test_pool_backward_inside_bn_pass_equals_separate_kernels(name, batch, image, kw):
-    """lbt_bn_bwd_quant_stats_pooled (the stem's max-pool backward gathered in the load stage of the BN backward pass 1: no
-    dense fp32 gradient of the un-pooled tensor) vs lbt_maxpool_bwd + lbt_bn_bwd_quant_stats."""
-    from lbt_b200 import _lib
-    seen = []
-    orig = _lib.call
-
-    def spy(fn, *a, **k):
-        seen.append(fn)
-        return orig(fn, *a, **k)
-
-    _lib.call = spy
-    try:
-        a = _run(name, True, 3, batch, image, kw, pool=True)
-        fused_calls = list(seen)
-        del seen[:]
-        b = _run(name, True, 3, batch, image, kw, pool=False)
-    finally:
-        _lib.call = orig
-    assert fused_calls.count('lbt_bn_bwd_quant_stats_pooled') == 3 and 'lbt_maxpool_bwd' not in fused_calls
-    assert seen.count('lbt_maxpool_bwd') == 3 and 'lbt_bn_bwd_quant_stats_pooled' not in seen
-    assert a['losses'] == b['losses'], (a['losses'], b['losses'])
-    assert torch.equal(a['ranges'], b['ranges'])
-    assert torch.equal(a['counters'], b['counters'])
-    for k in ('g', 'w', 'a'):
-        assert torch.equal(a[k].view(torch.int32), b[k].view(torch.int32)), k
 
 
 @pytest.mark.parametrize('name,batch,image,kw', [
@@ -86,38 +47,6 @@ def test_fused_units_equal_unfused_bit_for_bit(name, batch, image, kw):
         assert torch.equal(a[k].view(torch.int32), b[k].view(torch.int32)), k
     for x, y in zip(a['bn'], b['bn']):
         assert torch.equal(x, y)
-
-
-@pytest.mark.parametrize('name,batch,image,kw', [('CIFAR10_Resnet20', 16, 32, {}), ('CIFAR10_Resnet20', 3, 32, {}),
-                                                 ('Resnet18', 4, 64, dict(image=64, num_classes=10)),
-                                                 ('Resnet50', 2, 64, dict(image=64, num_classes=10))])
-def test_backward_link_equals_separate_bn_pass(name, batch, image, kw):
-    """lbt_conv_i8_dgrad_bn (a unit's BN backward pass 1 in the epilogue of the next unit's input-gradient kernel, no fp32
-    gradient tensor between them) vs lbt_conv_i8_fprop + lbt_bn_bwd_quant_stats."""
-    a = _run(name, True, 3, batch, image, kw, link=True)
-    linked = D._link_count
-    b = _run(name, True, 3, batch, image, kw, link=False)
-    assert D._link_count == 0
-    if name == 'CIFAR10_Resnet20':
-        assert linked == 3 * 9, linked              # every residual block, every step
-    assert a['losses'] == b['losses']
-    assert torch.equal(a['ranges'], b['ranges'])
-    assert torch.equal(a['counters'], b['counters'])
-    for k in ('g', 'w', 'a'):
-        assert torch.equal(a[k].view(torch.int32), b[k].view(torch.int32)), k
-
-
-@pytest.mark.parametrize('name,batch,image,kw', [('CIFAR10_Resnet20', 64, 32, {}), ('CIFAR10_Resnet20', 7, 32, {}),
-                                                 ('Resnet18', 4, 64, dict(image=64, num_classes=10))])
-def test_single_launch_bn_backward_equals_two_passes(name, batch, image, kw):
-    """lbt_bn_bwd_fused (both BN backward passes + grid barrier in one launch) vs the two separate launches."""
-    a = _run(name, True, 3, batch, image, kw, bn_bwd=True)
-    b = _run(name, True, 3, batch, image, kw, bn_bwd=False)
-    assert a['losses'] == b['losses']
-    assert torch.equal(a['ranges'], b['ranges'])
-    assert torch.equal(a['counters'], b['counters'])
-    for k in ('g', 'w', 'a'):
-        assert torch.equal(a[k].view(torch.int32), b[k].view(torch.int32)), k
 
 
 def test_fused_unit_hands_mantissas_to_the_next_conv():
